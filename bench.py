@@ -20,6 +20,8 @@ scaling: the matrix is fixed).
 --config hubbard | heg | sweep run BASELINE.json configs 2, 3 and 5 with the same timing code (one JSON line each).
 --impl reference times the CPU restatement of the reference's own fast_sparse_matrix_multiply_upper_triangular
 (oracle/, threads emulate the MPI rank decomposition of davidson_sparse_mpi2) on a bounded sample of the same workload.
+--dump-outputs DIR writes y of the last timed step (caller row order, float64) as DIR/y.npy with the caller rows it holds
+as DIR/y_rows.npy (a fixed seeded sample of at most 2^21 rows per run), so that two builds can be compared row for row.
 """
 import argparse
 import json
@@ -32,6 +34,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True   # the tree may be read-only; nothing is written into it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 CURVE = os.path.join(ROOT, "data", "C2_v2z_curve")
@@ -151,8 +154,9 @@ def run_reference(args):
         O.matvec_upper_mt(cnt, idx, val, x, cores)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        O.matvec_upper_mt(cnt, idx, val, x, cores)
+        y = O.matvec_upper_mt(cnt, idx, val, x, cores)
     t = (time.perf_counter() - t0) / args.steps
+    dump_outputs(args, "", y)
     v = nnz_full / t
     sample = ("C2 cc-pVDZ r1.24253 time_sym=f, %s (nnz_full=%d); %d threads, rows dealt round-robin, private y + reduction; "
               "obtaining the sample (oracle HCI run incl. its H builds) took %.1f s on one core (untimed)" % (desc, nnz_full, cores, t_space + t_build))
@@ -165,6 +169,21 @@ def run_reference(args):
                              "why_port": "the reference is Fortran 90 + MPI + LAPACK; probe of this host: %s" % json.dumps(tool)},
             "e2e": {"value": v, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
     print(json.dumps(line))
+
+
+DUMP_ROWS = 1 << 21   # --dump-outputs: rows kept per run, shared by its workloads (y + row ids in float64: 33.6 MB in all)
+
+
+def dump_outputs(args, tag, y):
+    """--dump-outputs: y (caller row order) of the last timed step as DIR/<tag>y.npy, or a fixed seeded sample of its rows when
+    it holds more than this workload's share of DUMP_ROWS; the caller rows kept go to DIR/<tag>y_rows.npy (float64, 0-based)"""
+    if not args.dump_outputs:
+        return
+    n, m = len(y), DUMP_ROWS // args.dump_workloads
+    rows = np.arange(n) if n <= m else np.sort(np.random.default_rng(0).choice(n, m, replace=False))
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    np.save(os.path.join(args.dump_outputs, tag + "y.npy"), np.ascontiguousarray(y[rows], dtype=np.float64))
+    np.save(os.path.join(args.dump_outputs, tag + "y_rows.npy"), rows.astype(np.float64))
 
 
 def cpu_baseline(args):
@@ -248,7 +267,8 @@ def bench_owner(up, dn, world):
 
 
 def time_hv(c, H, n, nloc, steps, warmup, x_host, projector=None):
-    """device-resident H.v steps: CUDA events on the launching stream, max over ranks -> (ms per step, per-step list, launches)"""
+    """device-resident H.v steps on x_host (internal row order): CUDA events on the launching stream, max over ranks
+    -> (ms per step, per-step list, launches, y of the last step on the device)"""
     import ctypes as C
     import torch
     from sqmc_b200 import _lib
@@ -367,7 +387,8 @@ def parity_block(system_factory, up, dn, x_host, y_full, nrows=16, scale=1.0, sh
             "how": "y from the e2e call (host vectors); rows recomputed from oracle brute-force full rows; x_dot_y / y_norm2 must agree to 1e-12 relative across GPU counts"}
 
 
-def emit(c, args, H, system_factory, up, dn, workload, config_extra, t_build, t_space, hci_log=None, projector=None, with_cpu=True):
+def emit(c, args, H, system_factory, up, dn, workload, config_extra, t_build, t_space, hci_log=None, projector=None, with_cpu=True,
+         dump_tag=""):
     """time the resident matrix and print the JSON line (rank 0)"""
     import torch.distributed as dist
     from sqmc_b200 import spaces
@@ -378,13 +399,17 @@ def emit(c, args, H, system_factory, up, dn, workload, config_extra, t_build, t_
     bt = H.build_times()
     nnz_max = max_over_ranks(c, float(nnz_loc))
     x_host = spaces.splitmix_vector(n)
+    perm = H.perm()   # internal row p holds caller row perm[p]: the device leg gets the same x (caller order) as the e2e leg
     sampler = ClockSampler(c.local)
     if c.rank == 0:
         sampler.start()
-    ms_step, per, launches, _ = time_hv(c, H, n, nloc, args.steps, args.warmup, x_host)
+    ms_step, per, launches, y = time_hv(c, H, n, nloc, args.steps, args.warmup, x_host[perm])
     clocks = sampler.stop() if c.rank == 0 else None
-    e2e_steps = max(3, min(args.steps, 10))
-    t_e2e, h2d, d2h, y_full, e2e_call = time_e2e(c, H, n, up, dn, x_host, e2e_steps, projector=projector)
+    if args.dump_outputs:   # one rank (main): y holds all n rows
+        y_caller = np.empty(n)
+        y_caller[perm] = y[:n].cpu().numpy()
+        dump_outputs(args, dump_tag, y_caller)
+    t_e2e, h2d, d2h, y_full, e2e_call = time_e2e(c, H, n, up, dn, x_host, args.steps, projector=projector)
     mode = H.exchange_mode()
     if c.rank != 0:
         return
@@ -517,7 +542,8 @@ def run_heg(c, args):
         fac = lambda cutoff=cutoff: O.System.heg(3, 0.5, 14, 7, cutoff)  # noqa: E731
         wl = ("HEG 14 electrons r_s=0.5 cutoff %.1f (%d orbitals), %d determinants: HCI space grown on the GPU to eps_var=%.0e; "
               "step = one H.v" % (cutoff, heg.norb, len(up), log[-1]["eps_var"]))
-        emit(c, args, H, fac, up, dn, wl, {"case": "heg", "cutoff": cutoff, "E_var": e}, t_build, t_space, hci_log=log, with_cpu=False)
+        emit(c, args, H, fac, up, dn, wl, {"case": "heg", "cutoff": cutoff, "E_var": e}, t_build, t_space, hci_log=log, with_cpu=False,
+             dump_tag="cutoff%.1f_" % cutoff)
         H.close()
 
 
@@ -536,7 +562,7 @@ def run_sweep(c, args):
         t_build = timed_build(c, H, up, dn)
         fac = lambda fd=fd, chem=chem: O.System.chem(fd, chem.norb, chem.nelec, chem.nup, chem.orbital_symmetries_fcidump)  # noqa: E731
         wl = "C2 cc-pVDZ r%s (FCIDUMP), time_sym=f, the %d lowest-diagonal-energy A_g determinants of %d; step = one H.v" % (rr, len(up), sector)
-        emit(c, args, H, fac, up, dn, wl, {"case": "sweep", "geometry": rr}, t_build, t_space, with_cpu=False)
+        emit(c, args, H, fac, up, dn, wl, {"case": "sweep", "geometry": rr}, t_build, t_space, with_cpu=False, dump_tag="r%s_" % rr)
         H.close()
 
 
@@ -560,12 +586,19 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--davidson", action="store_true", help="also run a full device Davidson and print it on a second line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write y of the last timed step (caller row order; a fixed seeded sample of rows above 2^21) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
+    args.dump_workloads = {"heg": 2, "sweep": len(args.geometries.split(",")) if args.geometries else len(GEOMETRIES)}.get(args.config, 1)
     if args.impl == "reference":
         return run_reference(args)
     c = setup_dist()
+    if args.dump_outputs and c.world > 1:
+        raise SystemExit("bench.py: --dump-outputs runs on one GPU (the device leg's y is sharded over ranks)")
     {"c2": run_c2, "hubbard": run_hubbard, "heg": run_heg, "sweep": run_sweep}[args.config](c, args)
     if c.world > 1:
         import torch.distributed as dist
