@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""In-process A/B of the H.v kernel variants on ONE resident matrix (same box, same clocks).
-usage: bundle_inproc.py [n_dets] [space: hci|lowest] [R:variant,...]   variant = SQMC_BUNDLE_KERNEL (10*MODE + MINB), R = 0 plain rows"""
+"""In-process A/B of the H.v row layouts on ONE resident matrix (same box, same clocks).
+usage: bundle_inproc.py [n_dets] [space: hci|lowest] [R,...]   R = rows per bundle (2 or 4), 0 = plain rows"""
 import ctypes as C, json, os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -9,8 +9,7 @@ from sqmc_b200 import _lib, spaces
 
 n_dets = int(sys.argv[1]) if len(sys.argv) > 1 else 10_000_000
 space = sys.argv[2] if len(sys.argv) > 2 else "hci"
-order = ([tuple(int(q) for q in a.split(":")) for a in sys.argv[3].split(",")] if len(sys.argv) > 3
-         else [(4, 14), (4, 15), (4, 4), (4, 5), (2, 14), (2, 15), (2, 4), (2, 5), (0, 0), (4, 15), (4, 14)])
+order = [int(a) for a in sys.argv[3].split(",")] if len(sys.argv) > 3 else [4, 2, 0, 4, 2, 0]
 _lib.init(device=0)
 L = _lib.load()
 chem = sq.ChemSystem("data/C2_v2z_curve/r1.24253/FCIDUMP")
@@ -26,8 +25,7 @@ x = torch.from_numpy(spaces.splitmix_vector(n)).cuda(); y = torch.zeros(n, dtype
 sp = C.c_void_p(stream.cuda_stream)
 ref = None
 cur = 4
-for R, var in order:
-    os.environ["SQMC_BUNDLE_KERNEL"] = str(var)
+for R in order:
     t0 = time.perf_counter()
     if R != cur:
         H.set_row_bundle(R); cur = R
@@ -43,5 +41,5 @@ for R, var in order:
     ms = e0.elapsed_time(e1) / 30
     yy = y.cpu().numpy().copy()
     if ref is None: ref = yy
-    print(json.dumps({"n": n, "nnz_full": nnz, "R": R, "kernel": var, "ms": ms, "GBs": (12.0 * nnz + 20.0 * n) / ms / 1e6, "frac_6455.6": (12.0 * nnz + 20.0 * n) / ms / 1e6 / 6455.6,
+    print(json.dumps({"n": n, "nnz_full": nnz, "R": R, "ms": ms, "GBs": (12.0 * nnz + 20.0 * n) / ms / 1e6, "frac_6455.6": (12.0 * nnz + 20.0 * n) / ms / 1e6 / 6455.6,
                       "set_layout_s": t_set, "max_rel_diff_vs_first": float(np.max(np.abs(yy - ref)) / np.max(np.abs(ref)))}), flush=True)

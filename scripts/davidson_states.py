@@ -14,12 +14,10 @@ H.generate_sparse_ham_upper_triangular(up, dn)
 for R in (4, 0):
     H.set_row_bundle(R)
     for ns in (1, 2):
-        for pipe in ((2, 4) if (R and ns == 2) else (2,)):
-            os.environ["SQMC_SPMM_PIPE"] = str(pipe)
-            H.davidson_sparse(n_states=ns, max_vec_per_state=3)  # warm-up
-            H.davidson_sparse(n_states=ns, max_vec_per_state=3)
-            t0 = time.perf_counter()
-            d = H.davidson_sparse(n_states=ns)
-            t = time.perf_counter() - t0
-            print(json.dumps({"rows_per_bundle": R, "n_states": ns, "spmm_pipe": pipe, "seconds": t, "n_matvec": d["n_matvec"],
-                              "ms_per_matvec_all_in": 1e3 * t / d["n_matvec"], "evals": [float(e) for e in d["evals"]]}), flush=True)
+        H.davidson_sparse(n_states=ns, max_vec_per_state=3)  # warm-up
+        H.davidson_sparse(n_states=ns, max_vec_per_state=3)
+        t0 = time.perf_counter()
+        d = H.davidson_sparse(n_states=ns)
+        t = time.perf_counter() - t0
+        print(json.dumps({"rows_per_bundle": R, "n_states": ns, "seconds": t, "n_matvec": d["n_matvec"],
+                          "ms_per_matvec_all_in": 1e3 * t / d["n_matvec"], "evals": [float(e) for e in d["evals"]]}), flush=True)

@@ -1374,8 +1374,7 @@ static int build_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, const
   // probes plus the staging of 2 W words per (tile, group).  HEG spaces have ~10 determinants per alpha string (137 220 / 15 024,
   // 10^6 / 73 111): there the scan is 3-4x faster (build of the 10^6-determinant HEG space: 0.10 s vs 0.47 s), so probes need
   // n >= 64 nA (C2 10^7: 669 per group, C2 10^6 lowest-energy: 96, Hubbard full sector: 804).
-  bool use_bmp = !ts && W <= 8192 && nA * (int64_t)W <= (1ll << 28) && n >= 64 * nA;
-  if (const char *be = getenv("SQMC_CONNECT_BITMAP")) use_bmp = use_bmp && atoi(be) != 0;
+  const bool use_bmp = !ts && W <= 8192 && nA * (int64_t)W <= (1ll << 28) && n >= 64 * nA;
   if (use_bmp) {
     SQ_CHECK(neighbour_lists<NW>(EBb.p, gB_off.p, nB, T.ndn, T.norb, nbrB_off, nbrB, s));
     for (int pass = 0; pass < (old ? 2 : 1); pass++) {
@@ -1391,8 +1390,7 @@ static int build_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, const
   }
   // probe lists staged in shared memory when they are short enough (lmax = ndn (norb - ndn) + 1 ids per string) and the ids fit 16 bits
   const int probe_lmax = T.ndn * (T.norb - T.ndn) + 1;
-  bool stage_ids = use_bmp && nB <= 65535 && 2 * W * 4 + probe_lmax * kConnTile * 2 <= 160 * 1024;
-  if (const char *se = getenv("SQMC_CONNECT_STAGE")) stage_ids = stage_ids && atoi(se) != 0;
+  const bool stage_ids = use_bmp && nB <= 65535 && 2 * W * 4 + probe_lmax * kConnTile * 2 <= 160 * 1024;
   const int bmp_smem = 2 * W * 4 + (stage_ids ? probe_lmax * kConnTile * 2 : 0);
   if (use_bmp && bmp_smem > 24 * 1024) {
     SQ_CUDA(cudaFuncSetAttribute(connect_bitmap_kernel<NW, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bmp_smem));
@@ -1759,10 +1757,10 @@ int build_h(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *det
   // the previous call on this handle.  Then the previous matrix is kept and only pairs with a new determinant are generated
   // and evaluated -- the result is identical to a from-scratch build (an entry depends only on its two determinants).
   // Taken when the previous matrix is resident, unscaled, built (not imported) on one rank, without time-reversal
-  // expansion and by a partial-connection builder (chem / heg); otherwise the matrix is rebuilt.  SQMC_INCREMENTAL=0 disables.
+  // expansion and by a partial-connection builder (chem / heg); otherwise the matrix is rebuilt.  A caller that wants a rebuild
+  // passes ndet_old = 0.
   const ModelTables &T = h->T;
-  const char *ie = getenv("SQMC_INCREMENTAL");
-  bool inc = !(ie && atoi(ie) == 0) && ndet_old > 0 && ndet_old < n && h->d_rowptr && h->d_up && h->n == ndet_old && G.nranks == 1 && h->scale == 1.0 &&
+  bool inc = ndet_old > 0 && ndet_old < n && h->d_rowptr && h->d_up && h->n == ndet_old && G.nranks == 1 && h->scale == 1.0 &&
              !(T.model == MODEL_CHEM && T.time_sym) && T.model != MODEL_HUBBARDK && h->row0 == 0 && h->row1 == h->n;
   OldMatrix old;
   if (inc) {

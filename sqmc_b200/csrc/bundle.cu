@@ -187,23 +187,15 @@ __global__ void __launch_bounds__(256) bundle_decode_kernel(const int64_t *__res
 }
 
 // ------------------------------------------------------------------ H.v on bundles: one warp per bundle, R sums per lane
-// MODE 1: product routed with a 0.0 / 1.0 multiplier built from the one-hot bit (exact: p*1+a and p*0+a round like a+p and a)
-// MODE 0: compare + predicated add (what ptxas turns into DADD + FSEL pairs); kept for A/B measurements
-template <int R, int MODE, int Q>
-__device__ __forceinline__ void badd_one(double (&acc)[R], int32_t word, double p) {
-  if constexpr (Q < R) {
-    if constexpr (MODE == 1) {
-      const int hi = (word & (1 << Q)) * (0x3FF00000 >> Q);  // 0x3FF00000 = high word of 1.0
-      acc[Q] = fma(p, __hiloint2double(hi, 0), acc[Q]);
-    } else {
-      asm("{\n\t.reg .pred q;\n\t.reg .b32 t;\n\tand.b32 t, %2, %3;\n\tsetp.ne.s32 q, t, 0;\n\t@q add.rn.f64 %0, %0, %1;\n\t}" : "+d"(acc[Q]) : "d"(p), "r"(word), "n"(1 << Q));
-    }
-    badd_one<R, MODE, Q + 1>(acc, word, p);
-  }
-}
-template <int R, int MODE>
+// A product is routed to its row sum with a 0.0 / 1.0 multiplier built from the one-hot bit (exact: p*1+a and p*0+a round like
+// a+p and a).
+template <int R, int Q = 0>
 __device__ __forceinline__ void badd(double (&acc)[R], int32_t word, double p) {
-  badd_one<R, MODE, 0>(acc, word, p);
+  if constexpr (Q < R) {
+    const int hi = (word & (1 << Q)) * (0x3FF00000 >> Q);  // 0x3FF00000 = high word of 1.0
+    acc[Q] = fma(p, __hiloint2double(hi, 0), acc[Q]);
+    badd<R, Q + 1>(acc, word, p);
+  }
 }
 
 __device__ __forceinline__ int4 ld_col4(const int32_t *p, const Policies &P) {
@@ -232,21 +224,28 @@ __device__ __forceinline__ void blk_load(Blk &B, const int32_t *cols, const doub
   B.v23 = ld_val2(vals + o + 4 * lane + 2, P);
 }
 
+// XT: the gathers of x go through the texture path (tex1Dfetch on a linear texture over x) instead of LSU loads: the LSU data
+// pipe of L1TEX is the busiest unit of this kernel (90 % under ncu, half of its wavefronts are the gathers) and the texture
+// pipe is idle otherwise.  A linear texture needs a 512-byte aligned base; other vectors are gathered with LSU loads.
+//
 // SCAT (distributed-slice entry points): the kernel does not write y but sends every finished row sum -- plus c*w[row] for the
 // projector, do_walk.f90:2290 -- straight to the rank that owns the determinant (a store into that rank's exchange buffer
 // over NVLink, p2p.cu), and the last CTA publishes the epoch to every peer: H.v and the reduce-scatter of
 // mpi_redscatt_real_dparray (mpi_routines.f90:1592) are one kernel, the transfers overlap the arithmetic bundle by bundle.
-
-// NV = 1: y = H x.  NV = 2: two right-hand sides at once (Davidson with n_states >= 2, SURVEY.md 8(d) "SpMM"): x / y hold the
-// two vectors interleaved (x[2*col + k]), one 16-byte gather serves both and the matrix is streamed once
-// (algorithmic bytes 12*nnz_full + 36*n for two vectors instead of 2*(12*nnz_full + 20*n)).
-// XT: the gathers of x go through the texture path (tex1Dfetch on a linear texture over x) instead of LSU loads: the LSU data
-// pipe of L1TEX is the busiest unit of this kernel (90 % under ncu, half of its wavefronts are the gathers) and the texture
-// pipe is idle otherwise.
-template <int R, int MODE, int NV, int MINB, bool SCAT, bool XT>
-__global__ void __launch_bounds__(256, MINB) bundle_hv_kernel(const int64_t *__restrict__ rowptr, int64_t nloc, int64_t nb, const int32_t *__restrict__ cols,
-                                                              const double *__restrict__ vals, const double *__restrict__ x, double *__restrict__ y,
-                                                              OwnerScatter O, cudaTextureObject_t xtex) {
+//
+// The start of a bundle is ordered for latency.  ncu's stall samples and the shared-bundle / several-bundles-per-warp experiments
+// (profiles/r02_bundle_kernel_ab.txt) showed that the per-bundle prologue -- row pointers -> head / tail entries (up to five scalar
+// load -> gather -> add rounds, one after the other) -> first block -> first gathers -- is a chain of serial memory latencies during
+// which the warp has nothing else in flight.  Here the first block's three 128-bit stream loads are issued FIRST, and the (up to
+// five) scalar load pairs of the head / tail entries are all issued before their gathers, so these latencies overlap: 2 % on the
+// 26-block bundles of the bench matrix, 6 % on 9-block bundles.
+//
+// x is the last parameter: placed in front of O it would move OwnerScatter in parameter space and change how the SCAT
+// instantiations load it.
+template <int R, bool SCAT, bool XT>
+__global__ void __launch_bounds__(256, 4) bundle_hv_kernel(const int64_t *__restrict__ rowptr, int64_t nloc, int64_t nb, const int32_t *__restrict__ cols,
+                                                           const double *__restrict__ vals, double *__restrict__ y, OwnerScatter O,
+                                                           cudaTextureObject_t xtex, const double *__restrict__ x) {
   const Policies P;
   auto gx = [&](int32_t col) -> double {
     if constexpr (XT) {
@@ -255,158 +254,6 @@ __global__ void __launch_bounds__(256, MINB) bundle_hv_kernel(const int64_t *__r
     } else {
       return ld_x(x + col, P);
     }
-  };
-  auto gx2 = [&](int32_t col) -> double2 {
-    if constexpr (XT) {
-      const int4 t = tex1Dfetch<int4>(xtex, col);
-      return make_double2(__hiloint2double(t.y, t.x), __hiloint2double(t.w, t.z));
-    } else {
-      return bld_x2(x + 2 * (int64_t)col, P);
-    }
-  };
-  const int64_t b = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
-  const int lane = threadIdx.x & 31;
-  if (b < nb) {
-  const int64_t r0 = b * R;
-  const int64_t e0 = rowptr[r0], e1 = rowptr[min(r0 + R, nloc)];
-  const Sigma S(e0, e1 - e0);
-  double acc[R], acc2[NV == 2 ? R : 1];
-#pragma unroll
-  for (int r = 0; r < R; r++) acc[r] = 0.0;
-#pragma unroll
-  for (int r = 0; r < (NV == 2 ? R : 1); r++) acc2[r] = 0.0;
-
-  const int64_t o0 = e0 + S.h;
-  auto work = [&](const Blk &B, double (&xa)[4], double (&xb)[4]) {
-    badd<R, MODE>(acc, B.c.x, B.v01.x * xa[0]);
-    badd<R, MODE>(acc, B.c.y, B.v01.y * xa[1]);
-    badd<R, MODE>(acc, B.c.z, B.v23.x * xa[2]);
-    badd<R, MODE>(acc, B.c.w, B.v23.y * xa[3]);
-    if (NV == 2) {
-      badd<(NV == 2 ? R : 1), MODE>(acc2, B.c.x, B.v01.x * xb[0]);
-      badd<(NV == 2 ? R : 1), MODE>(acc2, B.c.y, B.v01.y * xb[1]);
-      badd<(NV == 2 ? R : 1), MODE>(acc2, B.c.z, B.v23.x * xb[2]);
-      badd<(NV == 2 ? R : 1), MODE>(acc2, B.c.w, B.v23.y * xb[3]);
-    }
-  };
-  auto gather = [&](const Blk &B, double (&xa)[4], double (&xb)[4]) {
-    if (NV == 1) {
-      xa[0] = gx(B.c.x >> kBShift);
-      xa[1] = gx(B.c.y >> kBShift);
-      xa[2] = gx(B.c.z >> kBShift);
-      xa[3] = gx(B.c.w >> kBShift);
-    } else {
-      double2 t;
-      t = gx2(B.c.x >> kBShift); xa[0] = t.x; xb[0] = t.y;
-      t = gx2(B.c.y >> kBShift); xa[1] = t.x; xb[1] = t.y;
-      t = gx2(B.c.z >> kBShift); xa[2] = t.x; xb[2] = t.y;
-      t = gx2(B.c.w >> kBShift); xa[3] = t.x; xb[3] = t.y;
-    }
-  };
-  // software pipeline over the full blocks with two named register sets: gathers of the current block, then the next
-  // block's 128-bit stream loads, then the current block's arithmetic (the loads are asm volatile: their order is kept)
-  Blk A, B;
-  double xa[4], xb[4];
-  const int64_t nblk = S.nblk;
-  if (nblk > 0) blk_load(A, cols, vals, o0, lane, P);
-  // entries in front of the first aligned block (<= 3) and behind the last full block (<= 127), merged order, scalar loads -- after the
-  // first block's stream loads are on their way (see bundle_hvk_kernel)
-  if constexpr (NV == 1) {
-    // all load pairs first (slot 0: head, slots 1..4: tail), then all gathers, then the products; absent entries get column word 0 /
-    // value 0.0: a product 0.0 * x[0] that is routed nowhere
-    const int64_t t0 = o0 + (nblk << 7) + lane;
-    int32_t cw[5];
-    double vv[5], xx[5];
-    cw[0] = 0; vv[0] = 0.0;
-    if (lane < S.h) { cw[0] = ld_col(cols + e0 + lane, P); vv[0] = ld_val(vals + e0 + lane, P); }
-#pragma unroll
-    for (int q = 0; q < 4; q++) {
-      cw[q + 1] = 0; vv[q + 1] = 0.0;
-      if (t0 + 32 * q < e1) { cw[q + 1] = ld_col(cols + t0 + 32 * q, P); vv[q + 1] = ld_val(vals + t0 + 32 * q, P); }
-    }
-#pragma unroll
-    for (int q = 0; q < 5; q++) xx[q] = gx(cw[q] >> kBShift);
-#pragma unroll
-    for (int q = 0; q < 5; q++) badd<R, MODE>(acc, cw[q], vv[q] * xx[q]);
-  } else {  // two vectors: 2 R row sums are live, the entries are taken one round at a time
-    auto one = [&](int32_t cw, double v) {
-      const double2 xv = gx2(cw >> kBShift);
-      badd<R, MODE>(acc, cw, v * xv.x);
-      badd<(NV == 2 ? R : 1), MODE>(acc2, cw, v * xv.y);
-    };
-    if (lane < S.h) one(ld_col(cols + e0 + lane, P), ld_val(vals + e0 + lane, P));
-    for (int64_t k = o0 + (nblk << 7) + lane; k < e1; k += 32) one(ld_col(cols + k, P), ld_val(vals + k, P));
-  }
-  int64_t j = 0;
-  for (; j + 2 <= nblk; j += 2) {
-    gather(A, xa, xb);
-    blk_load(B, cols, vals, o0 + ((j + 1) << 7), lane, P);
-    work(A, xa, xb);
-    gather(B, xa, xb);
-    if (j + 2 < nblk) blk_load(A, cols, vals, o0 + ((j + 2) << 7), lane, P);
-    work(B, xa, xb);
-  }
-  if (j < nblk) {
-    gather(A, xa, xb);
-    work(A, xa, xb);
-  }
-
-  double m0 = 0.0, m1 = 0.0;
-#pragma unroll
-  for (int r = 0; r < R; r++) {
-    double a0 = acc[r], a1 = NV == 2 ? acc2[NV == 2 ? r : 0] : 0.0;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-      a0 += __shfl_xor_sync(0xffffffffu, a0, o);
-      if (NV == 2) a1 += __shfl_xor_sync(0xffffffffu, a1, o);
-    }
-    if (lane == r) { m0 = a0; m1 = a1; }
-  }
-  if (lane < R && r0 + lane < nloc) {
-    const int64_t row = r0 + lane;
-    if (SCAT) {
-      double v = m0;
-      if (O.w) v = v + O.c * O.w[row];
-      O.dst[O.owner[row]][O.pos[row]] = v;
-    } else if (NV == 1) {
-      y[row] = m0;
-    } else {
-      y[2 * row] = m0;
-      y[2 * row + 1] = m1;
-    }
-  }
-  }  // b < nb
-  if (SCAT) {  // all rows of this CTA are on their way: the last CTA publishes the epoch to every peer
-    __threadfence_system();
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      const unsigned long long prev = atomicAdd(O.counter, 1ull);
-      if (prev == gridDim.x - 1) {
-        *O.counter = 0ull;
-        __threadfence_system();
-        for (int p = 0; p < O.nranks; p++)
-          if (O.flag[p]) asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(O.flag[p]), "l"(O.epoch) : "memory");
-      }
-    }
-  }
-}
-
-// ------------------------------------------------------------------ the adopted single-vector kernel
-// Same storage format, arithmetic and per-row order as bundle_hv_kernel<R, 1, 1, 4, ., true> (bit-identical results) with the start of a
-// bundle ordered for latency.  ncu's stall samples and the shared-bundle / several-bundles-per-warp experiments (profiles/
-// r02_bundle_kernel_ab.txt) showed that the per-bundle prologue -- row pointers -> head / tail entries (up to five scalar load ->
-// gather -> add rounds, one after the other) -> first block -> first gathers -- is a chain of serial memory latencies during which
-// the warp has nothing else in flight.  Here the first block's three 128-bit stream loads are issued FIRST, and the (up to five)
-// scalar load pairs of the head / tail entries are all issued before their gathers, so these latencies overlap: 2 % on the
-// 26-block bundles of the bench matrix, 6 % on 9-block bundles.
-template <int R, int MINB, bool SCAT>
-__global__ void __launch_bounds__(256, MINB) bundle_hvk_kernel(const int64_t *__restrict__ rowptr, int64_t nloc, int64_t nb, const int32_t *__restrict__ cols,
-                                                               const double *__restrict__ vals, double *__restrict__ y, OwnerScatter O,
-                                                               cudaTextureObject_t xtex) {
-  const Policies P;
-  auto gx = [&](int32_t col) -> double {
-    const int2 t = tex1Dfetch<int2>(xtex, col);
-    return __hiloint2double(t.y, t.x);
   };
   const int lane = threadIdx.x & 31;
   const int64_t b = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
@@ -435,7 +282,7 @@ __global__ void __launch_bounds__(256, MINB) bundle_hvk_kernel(const int64_t *__
 #pragma unroll
       for (int q = 0; q < 5; q++) xx[q] = gx(cw[q] >> kBShift);
 #pragma unroll
-      for (int q = 0; q < 5; q++) badd<R, 1>(acc, cw[q], vv[q] * xx[q]);
+      for (int q = 0; q < 5; q++) badd<R>(acc, cw[q], vv[q] * xx[q]);
     }
     auto gather = [&](const Blk &K) {
       xa[0] = gx(K.c.x >> kBShift);
@@ -444,10 +291,10 @@ __global__ void __launch_bounds__(256, MINB) bundle_hvk_kernel(const int64_t *__
       xa[3] = gx(K.c.w >> kBShift);
     };
     auto work = [&](const Blk &K) {
-      badd<R, 1>(acc, K.c.x, K.v01.x * xa[0]);
-      badd<R, 1>(acc, K.c.y, K.v01.y * xa[1]);
-      badd<R, 1>(acc, K.c.z, K.v23.x * xa[2]);
-      badd<R, 1>(acc, K.c.w, K.v23.y * xa[3]);
+      badd<R>(acc, K.c.x, K.v01.x * xa[0]);
+      badd<R>(acc, K.c.y, K.v01.y * xa[1]);
+      badd<R>(acc, K.c.z, K.v23.x * xa[2]);
+      badd<R>(acc, K.c.w, K.v23.y * xa[3]);
     };
     // software pipeline over the full blocks with two named register sets: gathers of the current block, then the next block's
     // 128-bit stream loads, then the current block's arithmetic (the loads are asm volatile: their order is kept)
@@ -498,6 +345,98 @@ __global__ void __launch_bounds__(256, MINB) bundle_hvk_kernel(const int64_t *__
   }
 }
 
+// Two right-hand sides at once (Davidson with n_states >= 2, SURVEY.md 8(d) "SpMM"): x / y hold the two vectors interleaved
+// (x[2*col + k]), one 16-byte gather serves both and the matrix is streamed once (algorithmic bytes 12*nnz_full + 36*n for two
+// vectors instead of 2*(12*nnz_full + 20*n)).  2 R row sums are live, so the head / tail entries are taken one round at a time.
+template <int R, bool XT>
+__global__ void __launch_bounds__(256, 4) bundle_hv2_kernel(const int64_t *__restrict__ rowptr, int64_t nloc, int64_t nb, const int32_t *__restrict__ cols,
+                                                            const double *__restrict__ vals, const double *__restrict__ x, double *__restrict__ y,
+                                                            cudaTextureObject_t xtex) {
+  const Policies P;
+  auto gx2 = [&](int32_t col) -> double2 {
+    if constexpr (XT) {
+      const int4 t = tex1Dfetch<int4>(xtex, col);
+      return make_double2(__hiloint2double(t.y, t.x), __hiloint2double(t.w, t.z));
+    } else {
+      return bld_x2(x + 2 * (int64_t)col, P);
+    }
+  };
+  const int64_t b = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (b >= nb) return;
+  const int64_t r0 = b * R;
+  const int64_t e0 = rowptr[r0], e1 = rowptr[min(r0 + R, nloc)];
+  const Sigma S(e0, e1 - e0);
+  double acc[R], acc2[R];
+#pragma unroll
+  for (int r = 0; r < R; r++) acc[r] = 0.0;
+#pragma unroll
+  for (int r = 0; r < R; r++) acc2[r] = 0.0;
+
+  const int64_t o0 = e0 + S.h;
+  auto work = [&](const Blk &K, double (&xa)[4], double (&xb)[4]) {
+    badd<R>(acc, K.c.x, K.v01.x * xa[0]);
+    badd<R>(acc, K.c.y, K.v01.y * xa[1]);
+    badd<R>(acc, K.c.z, K.v23.x * xa[2]);
+    badd<R>(acc, K.c.w, K.v23.y * xa[3]);
+    badd<R>(acc2, K.c.x, K.v01.x * xb[0]);
+    badd<R>(acc2, K.c.y, K.v01.y * xb[1]);
+    badd<R>(acc2, K.c.z, K.v23.x * xb[2]);
+    badd<R>(acc2, K.c.w, K.v23.y * xb[3]);
+  };
+  auto gather = [&](const Blk &K, double (&xa)[4], double (&xb)[4]) {
+    double2 t;
+    t = gx2(K.c.x >> kBShift); xa[0] = t.x; xb[0] = t.y;
+    t = gx2(K.c.y >> kBShift); xa[1] = t.x; xb[1] = t.y;
+    t = gx2(K.c.z >> kBShift); xa[2] = t.x; xb[2] = t.y;
+    t = gx2(K.c.w >> kBShift); xa[3] = t.x; xb[3] = t.y;
+  };
+  // software pipeline over the full blocks as in bundle_hv_kernel
+  Blk A, B;
+  double xa[4], xb[4];
+  const int64_t nblk = S.nblk;
+  if (nblk > 0) blk_load(A, cols, vals, o0, lane, P);
+  // entries in front of the first aligned block (<= 3) and behind the last full block (<= 127), merged order, scalar loads -- after the
+  // first block's stream loads are on their way
+  auto one = [&](int32_t cw, double v) {
+    const double2 xv = gx2(cw >> kBShift);
+    badd<R>(acc, cw, v * xv.x);
+    badd<R>(acc2, cw, v * xv.y);
+  };
+  if (lane < S.h) one(ld_col(cols + e0 + lane, P), ld_val(vals + e0 + lane, P));
+  for (int64_t k = o0 + (nblk << 7) + lane; k < e1; k += 32) one(ld_col(cols + k, P), ld_val(vals + k, P));
+  int64_t j = 0;
+  for (; j + 2 <= nblk; j += 2) {
+    gather(A, xa, xb);
+    blk_load(B, cols, vals, o0 + ((j + 1) << 7), lane, P);
+    work(A, xa, xb);
+    gather(B, xa, xb);
+    if (j + 2 < nblk) blk_load(A, cols, vals, o0 + ((j + 2) << 7), lane, P);
+    work(B, xa, xb);
+  }
+  if (j < nblk) {
+    gather(A, xa, xb);
+    work(A, xa, xb);
+  }
+
+  double m0 = 0.0, m1 = 0.0;
+#pragma unroll
+  for (int r = 0; r < R; r++) {
+    double a0 = acc[r], a1 = acc2[r];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      a0 += __shfl_xor_sync(0xffffffffu, a0, o);
+      a1 += __shfl_xor_sync(0xffffffffu, a1, o);
+    }
+    if (lane == r) { m0 = a0; m1 = a1; }
+  }
+  if (lane < R && r0 + lane < nloc) {
+    const int64_t row = r0 + lane;
+    y[2 * row] = m0;
+    y[2 * row + 1] = m1;
+  }
+}
+
 // ------------------------------------------------------------------ host side
 // default: bundles of 4 rows (measured best on B200, profiles/r01_bundle_experiment.txt); SQMC_BUNDLE=0|2|4 overrides.
 // Read per call (a getenv is ~100 ns) so that one process can A/B layouts on one resident matrix.
@@ -506,16 +445,6 @@ static int bundle_want() {
   const int v = e ? atoi(e) : 4;
   return (v == 2 || v == 4) ? v : 0;
 }
-// kernel variant: SQMC_BUNDLE_KERNEL = 10*MODE + MINB (MODE 4 = the adopted kernel: 0/1-multiplier routing, gathers through the
-// texture path; 3 = the same body as a member of the general template (two vectors, A/B), 1 = 3 with LSU gathers, 0 = predicated
-// adds; MINB = CTAs/SM the register allocation is bounded for).  Default 44 (falls back to 14 when the vector is not 512-byte
-// aligned; two interleaved vectors use 34).  All variants start a bundle with the latency-ordered prologue.  A/B results in profiles/r02_bundle_kernel_ab.txt.
-static int bundle_variant() {
-  const char *e = getenv("SQMC_BUNDLE_KERNEL");
-  const int v = e ? atoi(e) : 44;
-  return (v == 4 || v == 5 || v == 14 || v == 15 || v == 34 || v == 35 || v == 44) ? v : 44;
-}
-
 template <int R>
 static int encode_t(sqmc_b200_handle *h, int cap, cudaStream_t s) {
   const int64_t nloc = h->row1 - h->row0, nb = div_up(nloc, (int64_t)R);
@@ -631,66 +560,39 @@ void x_textures_release(sqmc_b200_handle *h) {
   h->xtex.clear();
 }
 
-template <int NV>
-static int launch_hv(sqmc_b200_handle *h, const double *x, double *y, cudaStream_t s) {
-  const int64_t nloc = h->row1 - h->row0;
-  const int R = h->bundle_R;
-  const int64_t nb = div_up(nloc, (int64_t)R);
-  if (nb == 0) return 0;
-  const unsigned grid = (unsigned)div_up(nb * 32, (int64_t)256);
-  const int var = bundle_variant();
-  const OwnerScatter none = {};
-  if (var >= 30 && ((uintptr_t)x & 511) == 0) {  // gathers through the texture path (a linear texture needs a 512-byte aligned base)
-    cudaTextureObject_t tex = 0;
-    SQ_CHECK(x_texture(h, x, NV, &tex));
-#define SQ_BT(RR, MINB) bundle_hv_kernel<RR, 1, NV, MINB, false, true><<<grid, 256, 0, s>>>(h->d_rowptr, nloc, nb, h->d_cols, h->d_vals, x, y, none, tex)
-    if (NV == 1 && var == 44) {
-      if (R == 4) bundle_hvk_kernel<4, 4, false><<<grid, 256, 0, s>>>(h->d_rowptr, nloc, nb, h->d_cols, h->d_vals, y, none, tex);
-      else bundle_hvk_kernel<2, 4, false><<<grid, 256, 0, s>>>(h->d_rowptr, nloc, nb, h->d_cols, h->d_vals, y, none, tex);
-    } else if (R == 4) { if (var == 35) SQ_BT(4, 5); else SQ_BT(4, 4); }
-    else { if (var == 35) SQ_BT(2, 5); else SQ_BT(2, 4); }
-#undef SQ_BT
-    SQ_LAUNCH_CHECK();
-    return 0;
-  }
-  const int var_lsu = var >= 30 ? var - 20 : var;  // unaligned vector: same routing, LSU gathers
-#define SQ_BL(RR, MODE, MINB) bundle_hv_kernel<RR, MODE, NV, MINB, false, false><<<grid, 256, 0, s>>>(h->d_rowptr, nloc, nb, h->d_cols, h->d_vals, x, y, none, 0)
-  if (R == 4) {
-    if (var_lsu == 14) SQ_BL(4, 1, 4); else if (var_lsu == 15) SQ_BL(4, 1, 5); else if (var_lsu == 4) SQ_BL(4, 0, 4); else SQ_BL(4, 0, 5);
-  } else {
-    if (var_lsu == 14) SQ_BL(2, 1, 4); else if (var_lsu == 15) SQ_BL(2, 1, 5); else if (var_lsu == 4) SQ_BL(2, 0, 4); else SQ_BL(2, 0, 5);
-  }
-#undef SQ_BL
-  SQ_LAUNCH_CHECK();
-  return 0;
+template <int R, bool XT>
+static void hv_launch(const sqmc_b200_handle *h, int nv, const OwnerScatter *O, unsigned grid, int64_t nloc, int64_t nb, const double *x, double *y,
+                      cudaTextureObject_t tex, cudaStream_t s) {
+  if (nv == 2) bundle_hv2_kernel<R, XT><<<grid, 256, 0, s>>>(h->d_rowptr, nloc, nb, h->d_cols, h->d_vals, x, y, tex);
+  else if (O) bundle_hv_kernel<R, true, XT><<<grid, 256, 0, s>>>(h->d_rowptr, nloc, nb, h->d_cols, h->d_vals, y, *O, tex, x);
+  else bundle_hv_kernel<R, false, XT><<<grid, 256, 0, s>>>(h->d_rowptr, nloc, nb, h->d_cols, h->d_vals, y, OwnerScatter{}, tex, x);
 }
-int bundle_spmv(sqmc_b200_handle *h, const double *x, double *y, cudaStream_t s) { return launch_hv<1>(h, x, y, s); }
 
-// y = H x (+ c*w) with every row sum sent to its owner from inside the kernel (see OwnerScatter).  The grid always has at
-// least one CTA so that a rank without rows still publishes its epoch.
-int bundle_spmv_scatter(sqmc_b200_handle *h, const double *x, const OwnerScatter &O, cudaStream_t s) {
+// y = H x on bundles for nv (1 or 2) interleaved vectors; with O (one vector) every row sum goes to its owner instead of y.
+// R is the matrix's bundle size; x is gathered through a texture when its base is 512-byte aligned, with LSU loads otherwise.
+static int launch_hv(sqmc_b200_handle *h, int nv, const double *x, double *y, const OwnerScatter *O, cudaStream_t s) {
   const int64_t nloc = h->row1 - h->row0;
   const int R = h->bundle_R;
   const int64_t nb = div_up(nloc, (int64_t)R);
+  if (nb == 0 && !O) return 0;  // the scatter grid keeps one CTA so that a rank without rows still publishes its epoch
   const unsigned grid = (unsigned)std::max<int64_t>(1, div_up(nb * 32, (int64_t)256));
-  if (bundle_variant() >= 30 && ((uintptr_t)x & 511) == 0) {
-    cudaTextureObject_t tex = 0;
-    SQ_CHECK(x_texture(h, x, 1, &tex));
-    if (R == 4) bundle_hvk_kernel<4, 4, true><<<grid, 256, 0, s>>>(h->d_rowptr, nloc, nb, h->d_cols, h->d_vals, nullptr, O, tex);
-    else bundle_hvk_kernel<2, 4, true><<<grid, 256, 0, s>>>(h->d_rowptr, nloc, nb, h->d_cols, h->d_vals, nullptr, O, tex);
-  } else if (R == 4) {
-    bundle_hv_kernel<4, 1, 1, 4, true, false><<<grid, 256, 0, s>>>(h->d_rowptr, nloc, nb, h->d_cols, h->d_vals, x, nullptr, O, 0);
-  } else {
-    bundle_hv_kernel<2, 1, 1, 4, true, false><<<grid, 256, 0, s>>>(h->d_rowptr, nloc, nb, h->d_cols, h->d_vals, x, nullptr, O, 0);
-  }
+  cudaTextureObject_t tex = 0;
+  const bool xt = ((uintptr_t)x & 511) == 0;
+  if (xt) SQ_CHECK(x_texture(h, x, nv, &tex));
+  if (R == 4) (xt ? hv_launch<4, true> : hv_launch<4, false>)(h, nv, O, grid, nloc, nb, x, y, tex, s);
+  else (xt ? hv_launch<2, true> : hv_launch<2, false>)(h, nv, O, grid, nloc, nb, x, y, tex, s);
   SQ_LAUNCH_CHECK();
   return 0;
 }
+int bundle_spmv(sqmc_b200_handle *h, const double *x, double *y, cudaStream_t s) { return launch_hv(h, 1, x, y, nullptr, s); }
+
+// y = H x (+ c*w) with every row sum sent to its owner from inside the kernel (see OwnerScatter)
+int bundle_spmv_scatter(sqmc_b200_handle *h, const double *x, const OwnerScatter &O, cudaStream_t s) { return launch_hv(h, 1, x, nullptr, &O, s); }
 
 // y2 = H x2 for two interleaved vectors; only on bundled matrices (the caller falls back to two H.v otherwise)
 int bundle_spmm2(sqmc_b200_handle *h, const double *x2, double *y2, cudaStream_t s) {
   if (!h->bundle_R) { set_error("bundle_spmm2: matrix is not in row-bundle order"); return 2; }
-  return launch_hv<2>(h, x2, y2, s);
+  return launch_hv(h, 2, x2, y2, nullptr, s);
 }
 
 // one row out of a bundled matrix (get_row): read the bundle's segment and keep the entries tagged with this row

@@ -164,7 +164,7 @@ struct sqmc_b200_handle {
   int64_t bin_off[sqmc::kNumBins + 1] = {0};
   bool bins_ready = false;  // built lazily by the first plain-row H.v
 
-  // ---- row-bundle ordering (csrc/bundle.cu; active when bundle_R > 0: d_cols holds column << 3 | row-in-bundle) ----
+  // ---- row-bundle ordering (csrc/bundle.cu; active when bundle_R > 0: d_cols holds column << 4 | 1 << row-in-bundle) ----
   int bundle_R = 0, bundle_cap = 0;
   double *d_diag = nullptr;        // [nloc] diagonal of the local rows (copied out before the entries are re-ordered)
 
@@ -178,7 +178,7 @@ struct sqmc_b200_handle {
   int32_t *d_dest_pos = nullptr;            // [nloc] its position inside the owner's slice
   int32_t *d_my_internal = nullptr;         // [my_n] internal row of the k-th determinant this rank owns
   struct XTex { const double *ptr; int64_t n; int nv; cudaTextureObject_t tex; };
-  std::vector<XTex> xtex;  // linear textures over gathered vectors (texture-path variant of the H.v kernel)
+  std::vector<XTex> xtex;  // linear textures over gathered vectors (texture-path gathers of the H.v kernels)
   unsigned long long *d_scat_counter = nullptr;  // CTA counter of the fused H.v + owner exchange kernel on a single rank
   // ---- work buffers ----
   double *d_x = nullptr;   // n (global length, internal order)
@@ -260,7 +260,7 @@ int export_upper_device(sqmc_b200_handle *h, int64_t *counts, int64_t *indices, 
 int import_upper_device(sqmc_b200_handle *h, int64_t n, const int64_t *counts, const int64_t *indices, const double *values);
 int extract_diag(sqmc_b200_handle *h, double *diag_dev, cudaStream_t s);  // diagonal of the local rows (spmv.cu)
 // bundle.cu
-int bundle_encode(sqmc_b200_handle *h);  // plain CSR -> row bundles in place (SQMC_BUNDLE=2|4|8), no-op otherwise
+int bundle_encode(sqmc_b200_handle *h);  // plain CSR -> row bundles in place (SQMC_BUNDLE=2|4, default 4), no-op otherwise
 int bundle_encode_r(sqmc_b200_handle *h, int R);  // same with an explicit bundle size
 int bundle_decode(sqmc_b200_handle *h);  // exact inverse
 int bundle_spmv(sqmc_b200_handle *h, const double *x_dev, double *y_dev, cudaStream_t s);

@@ -522,9 +522,7 @@ static int select_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, cons
     SQ_CHECK(gather_strings(NW, dn.p, idx.p, sdn.p, n, s));
   }
   HM.mark("upload + sorted copy of the list");
-  static int want_hb = -1;
-  if (want_hb < 0) { const char *e = getenv("SQMC_SELECT_TABLES"); want_hb = (e && atoi(e) == 0) ? 0 : 1; }
-  const bool use_hb = want_hb && T.model == MODEL_CHEM && NW == 1 && T.norb <= 64;
+  const bool use_hb = T.model == MODEL_CHEM && NW == 1 && T.norb <= 64;
   if (use_hb) SQ_CHECK(hb_build(h));
   int64_t nd = n;  // determinants this rank expands (all of them on one rank)
   SQ_CHECK(shard_round_robin<NW>(up, dn, dc, dm, n, nd, s));

@@ -123,3 +123,43 @@ def test_tiny_spaces_in_every_layout(oracle, heg_space, n):
         assert c[-1] == n and v[-1] == val[-1]        # full row, ascending columns: its last entry is the diagonal of row n
         assert abs(H.davidson_sparse(n_states=1)["evals"][0] - ref["evals"][0]) < 1e-8
         assert abs(H.matrix_lanczos_sparse()["lowest_eigenvalue"] - oracle.lanczos(cnt, idx, val)["lowest"]) < 1e-8
+
+
+@pytest.mark.parametrize("R", [2, 4])
+def test_unaligned_vector_takes_lsu_gathers_with_identical_result(c2_space, R):
+    """A vector whose base is not 512-byte aligned cannot back a linear texture: the bundle kernel gathers it with LSU loads
+    instead.  The same x read from a 512-byte aligned and from an 8-byte offset device address gives the same y, bit for bit,
+    and that y agrees with the plain-row product.  sqmc_b200_matvec_dev works in the library's internal row order."""
+    import ctypes as C
+    import sqmc_b200 as sq
+    from sqmc_b200 import _lib, spaces
+    S, r = c2_space
+    H = sq.SparseHamiltonian(sq.ChemSystem(C2_FCIDUMP, time_sym=False, z=1))
+    H.generate_sparse_ham_upper_triangular(r["up"], r["dn"])
+    n = len(r["up"])
+    L = _lib.load()
+    x = spaces.splitmix_vector(n, seed=11)
+    base, ybuf = C.c_void_p(), C.c_void_p()
+    _lib.check(L.sqmc_b200_device_malloc(C.byref(base), (n + 128) * 8))
+    _lib.check(L.sqmc_b200_device_malloc(C.byref(ybuf), n * 8))
+    try:
+        aligned = (base.value + 511) // 512 * 512
+        assert aligned + 8 + n * 8 <= base.value + (n + 128) * 8
+
+        def product(x_addr):
+            _lib.check(L.sqmc_b200_memcpy_h2d(x_addr, x.ctypes.data, n * 8))
+            _lib.check(L.sqmc_b200_matvec_dev(H._h, x_addr, ybuf, None))
+            y = np.empty(n)
+            _lib.check(L.sqmc_b200_memcpy_d2h(y.ctypes.data, ybuf, n * 8))
+            return y
+
+        H.set_row_bundle(0)
+        y_plain = product(aligned)
+        H.set_row_bundle(R)
+        y_tex = product(aligned)
+        y_lsu = product(aligned + 8)
+        assert np.array_equal(y_tex, y_lsu)
+        assert np.max(np.abs(y_tex - y_plain)) <= 1e-12 * np.max(np.abs(y_plain))
+    finally:
+        L.sqmc_b200_device_free(base)
+        L.sqmc_b200_device_free(ybuf)
