@@ -109,6 +109,20 @@ int sqmc_b200_pt2_alias(sqmc_b200_handle *h, int64_t n, const void *dets_up, con
                         double eps_pt_big, int n_mc, double target_error, int32_t *rannyu_state, int max_samples, double *pt_energy,
                         double *pt_energy_std_dev, int *n_samples, double *e_2pt_samples, int64_t *n_connected);
 
+/* ---- one-particle density matrix (the step before natural orbitals, hci.f90:3198,3400,3554) ----------------
+ * One-particle density matrices of (variational) wavefunctions, spin resolved:
+ *   rdm[s][sigma](p,q) = <Psi_s| a+_{p sigma} a_{q sigma} |Psi_s>,   Psi_s = sum_i wts(i,s) |D_i>,   sigma = 0 (up), 1 (dn)
+ * p,q = 0..norb-1 index the bits of the determinant words (for chem: the reference's reordered orbital numbering).
+ * wts: n x n_states column-major, leading dimension ldw >= n; no normalisation is applied.
+ * rdm: n_states * 2 * norb * norb doubles, matrix (s, sigma) at offset (s*2 + sigma)*norb*norb, element (p,q) at p + norb*q.
+ * time_sym handles: D_i are the representatives, each standing for (|u,d> + z|d,u>)/sqrt2 (u != d) or |u,u>.
+ * The sign of a+_p a_q is permutation_factor's (alpha string first), so sum_pq h_pq gamma_pq is the one-body energy of the
+ * library's Hamiltonian.  The result is exactly symmetric and bit-identical across calls and across permutations of the rows.
+ * Errors: n <= 0, n_states < 1, ldw < n, a determinant listed twice, on time_sym handles a representative whose partner
+ * (d,u) is listed too.  No communication: on a multi-rank handle the call works on this rank's GPU over the list given. */
+int sqmc_b200_one_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states,
+                      const double *wts, int64_t ldw, double *rdm);
+
 /* ---- sparse H build --------------------------------------------------------
  * Replaces generate_sparse_ham_chem_upper_triangular (chemistry.f90:7639),
  * its _mpi twin (:8012), generate_sparse_ham_heg_upper_triangular

@@ -297,6 +297,25 @@ class SparseHamiltonian:
         return dict(lowest_eigenvalue=eig3[0], highest_eigenvalue=eig3[1], second_lowest_eigenvalue=eig3[2], lowest_eigenvector=evec,
                     ritz=ritz[:nlog.value].copy(), n_iter=nit.value)
 
+    def one_rdm(self, dets_up, dets_dn, wts):
+        """One-particle density matrices <Psi_s| a+_{p sigma} a_{q sigma} |Psi_s> of the wavefunctions wts (n,) or (n, n_states)
+        over the determinant list (any order, no built matrix needed; on time_sym systems the representatives).  Orbitals are
+        the bits of the determinant words (chem: the reordered numbering, see natorb.natural_orbitals).  No normalisation.
+        -> float64 array [s, sigma, p, q] of shape (n_states, 2, norb, norb), sigma 0 = up, 1 = dn; (2, norb, norb) for 1-D wts."""
+        up = np.ascontiguousarray(dets_up, dtype=np.uint64).reshape(-1, 2)
+        dn = np.ascontiguousarray(dets_dn, dtype=np.uint64).reshape(-1, 2)
+        w = np.asarray(wts, dtype=np.float64)
+        one = w.ndim == 1
+        w = np.asfortranarray(w.reshape(-1, 1) if one else w)
+        if len(dn) != len(up) or w.shape[0] != len(up):
+            raise ValueError("one_rdm: dets_up, dets_dn and wts must have the same number of rows")
+        norb, ns = self.system.norb, w.shape[1]
+        out = np.zeros((ns, 2, norb, norb))
+        check(self._L.sqmc_b200_one_rdm(self._h, len(up), _p(up), _p(dn), ns, _p(w), max(w.shape[0], 1), _p(out)))
+        # the library stores (p,q) at p + norb*q: the [s, sigma] block read in C order is gamma transposed
+        out = np.ascontiguousarray(out.transpose(0, 1, 3, 2))
+        return out[0] if one else out
+
     def second_order_pt(self, dets_up, dets_dn, wts, var_energy, eps_pt):
         """Deterministic second-order PT with the HCI screened sum (second_order_pt, hci.f90:1100-1182) -> (delta_e_2pt, ndets_connected)."""
         up = np.ascontiguousarray(dets_up, dtype=np.uint64).reshape(-1, 2)

@@ -50,7 +50,7 @@ def build(force=False, verbose=False):
               "--expt-extended-lambda"] + ARCH
     if verbose:
         common += ["-Xptxas", "-v"]
-    units = [("build.cu", ["--fmad=false"]), ("select.cu", ["--fmad=false"]), ("spmv.cu", []), ("convert.cu", []), ("bundle.cu", []), ("p2p.cu", []), ("growbuf.cu", []), ("local.cu", []), ("davidson.cu", []), ("api.cu", [])]
+    units = [("build.cu", ["--fmad=false"]), ("select.cu", ["--fmad=false"]), ("spmv.cu", []), ("convert.cu", []), ("bundle.cu", []), ("p2p.cu", []), ("growbuf.cu", []), ("local.cu", []), ("davidson.cu", []), ("rdm.cu", []), ("api.cu", [])]
     objs = []
     procs = []
     for name, extra in units:

@@ -276,4 +276,6 @@ int davidson_single(sqmc_b200_handle *h, const double *v0, double *evec, double 
                     int ritz_log_cap, int *n_ritz_logged);
 int lanczos(sqmc_b200_handle *h, const double *v0, double *evec, double *eig3, double tol, int max_iter, int *n_iter_out, double *ritz_log,
             int ritz_log_cap, int *n_ritz_logged);
+// rdm.cu
+int one_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw, double *rdm);
 }  // namespace sqmc

@@ -185,3 +185,32 @@ def read_dtm_projector(path, nup, ndn, n_core_orb=0):
     if counts.sum() != nnz:
         raise ValueError("read_dtm_projector: per-row counts sum to %d, header says %d" % (counts.sum(), nnz))
     return dict(up=up, dn=dn, counts=counts, indices=indices, values=values, dtm_energy=energy)
+
+
+# ----------------------------------------------------------------------------- FCIDUMP
+def write_fcidump(path, h, eri, ecore, nelec, ms2=0, orbsym=None, isym=1, tol=1.0e-12):
+    """Write a molecular FCIDUMP: the header (NORB, NELEC, MS2, ORBSYM, ISYM), then the unique entries with |v| > tol in the
+    usual order -- (pq|rs) with p >= q, r >= s, pq >= rs, then h_pq with p >= q as `v p q 0 0`, then the core energy as
+    `v 0 0 0 0`.  h: (norb, norb) symmetric, eri: (norb,)*4 chemists' (pq|rs) with the 8-fold symmetry; orbitals 1-based
+    in the file.  Values are written with 17 significant digits, so a read returns them bit for bit."""
+    norb = h.shape[0]
+    orbsym = [1] * norb if orbsym is None else [int(x) for x in orbsym]
+    lines = [" &FCI NORB=%d,NELEC=%d,MS2=%d," % (norb, nelec, ms2), "  ORBSYM=" + "".join("%d," % x for x in orbsym),
+             "  ISYM=%d," % isym, " &END"]
+    for p in range(norb):
+        for q in range(p + 1):
+            pq = p * (p + 1) // 2 + q
+            for r in range(p + 1):
+                for s in range(r + 1):
+                    if r * (r + 1) // 2 + s > pq:
+                        break
+                    v = eri[p, q, r, s]
+                    if abs(v) > tol:
+                        lines.append("%.17g %d %d %d %d" % (v, p + 1, q + 1, r + 1, s + 1))
+    for p in range(norb):
+        for q in range(p + 1):
+            if abs(h[p, q]) > tol:
+                lines.append("%.17g %d %d 0 0" % (h[p, q], p + 1, q + 1))
+    lines.append("%.17g 0 0 0 0" % ecore)
+    with open(path, "w") as f:
+        f.write("\n".join(lines) + "\n")

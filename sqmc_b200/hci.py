@@ -9,7 +9,8 @@ Loop rules restated from the reference (hci.f90:359-517; do_walk.f90:418-533):
     or after 50 iterations (:89);
   * Davidson starts from the previous vectors padded with zeros, from unit vectors in iteration 1 (:453-485);
   * PT per state: second_order_pt with eps_pt on the final wavefunction (do_pt, :4220-4243).
-Out of scope here: natural orbitals, active spaces, Green's functions, stochastic PT (n_mc > 0, eps_pt_big).
+Out of scope here: active spaces, Green's functions, stochastic PT (n_mc > 0, eps_pt_big).  Natural orbitals of the final
+wavefunction: natorb.py and scripts/natorb.py.
 """
 import re
 
@@ -195,4 +196,5 @@ def run_input(path, fcidump=None, device=0, log=print, wf_dir=None):
     res = perform_hci(H, system, cfg["eps_var"], cfg["eps_var_sched"], n_states=cfg["n_states"], eps_pt=cfg["eps_pt"], log=log,
                       wf_dir=wf_dir, dump_wf_var=cfg["dump_wf_var"])
     res["config"] = cfg
+    res["system"], res["hamiltonian"] = system, H
     return res
