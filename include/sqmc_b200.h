@@ -123,6 +123,20 @@ int sqmc_b200_pt2_alias(sqmc_b200_handle *h, int64_t n, const void *dets_up, con
 int sqmc_b200_one_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states,
                       const double *wts, int64_t ldw, double *rdm);
 
+/* ---- two-particle density matrix ------------------------------------------------------------------------------------
+ * Spin-resolved two-particle density matrices in chemists' order (they pair with (pq|rs)):
+ *   rdm2[s][b](p,q,r,s') = <Psi_s| a+_{p sigma} a+_{r tau} a_{s' tau} a_{q sigma} |Psi_s>,   b = 0 (sigma tau = alpha alpha),
+ *   1 (alpha beta), 2 (beta beta); beta alpha is alpha beta with the index pairs swapped and is not stored.
+ * 1/2 sum_b' sum (pq|rs') Gamma is the two-body energy, with b' running over aa, ab, ba (= ab) and bb.
+ * Arguments, orbital numbering, time_sym handling and errors are those of sqmc_b200_one_rdm; in addition norb must be <= 64.
+ * rdm2: n_states * 3 * norb^4 doubles, element (p,q,r,s') of block b, state s at p + norb*(q + norb*(r + norb*(s' + norb*(b + 3*s)))).
+ * Signs are those of the library's Hamiltonian (alpha string first), so the energy identity holds with its own integrals.
+ * Every element is written from one accumulated representative of its symmetry orbit, so Gamma_{pq,rs} = Gamma_{qp,sr}, and in
+ * the same-spin blocks Gamma_{pq,rs} = Gamma_{rs,pq} = -Gamma_{ps,rq} and Gamma = 0 for p = r or q = s, hold bit for bit.  The
+ * representatives are summed as 128-bit fixed-point integers, so the result is bit-identical across calls and row permutations. */
+int sqmc_b200_two_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states,
+                      const double *wts, int64_t ldw, double *rdm2);
+
 /* ---- sparse H build --------------------------------------------------------
  * Replaces generate_sparse_ham_chem_upper_triangular (chemistry.f90:7639),
  * its _mpi twin (:8012), generate_sparse_ham_heg_upper_triangular

@@ -316,6 +316,26 @@ class SparseHamiltonian:
         out = np.ascontiguousarray(out.transpose(0, 1, 3, 2))
         return out[0] if one else out
 
+    def two_rdm(self, dets_up, dets_dn, wts):
+        """Two-particle density matrices Gamma^{st}_{pq,rs} = <Psi_k| a+_{p s} a+_{r t} a_{s t} a_{q s} |Psi_k> (chemists' order:
+        1/2 sum (pq|rs) Gamma over aa, ab, ba = ab and bb is the two-body energy) of the wavefunctions wts (n,) or (n, n_states),
+        with the determinant list, orbital numbering and normalisation of one_rdm; norb <= 64.
+        -> float64 array [k, b, p, q, r, s] of shape (n_states, 3, norb, norb, norb, norb), b = 0 (alpha alpha), 1 (alpha beta),
+        2 (beta beta); (3, norb, norb, norb, norb) for 1-D wts."""
+        up = np.ascontiguousarray(dets_up, dtype=np.uint64).reshape(-1, 2)
+        dn = np.ascontiguousarray(dets_dn, dtype=np.uint64).reshape(-1, 2)
+        w = np.asarray(wts, dtype=np.float64)
+        one = w.ndim == 1
+        w = np.asfortranarray(w.reshape(-1, 1) if one else w)
+        if len(dn) != len(up) or w.shape[0] != len(up):
+            raise ValueError("two_rdm: dets_up, dets_dn and wts must have the same number of rows")
+        norb, ns = self.system.norb, w.shape[1]
+        out = np.zeros((ns, 3) + (norb,) * 4) if norb <= 64 else np.zeros(1)   # the library rejects norb > 64
+        check(self._L.sqmc_b200_two_rdm(self._h, len(up), _p(up), _p(dn), ns, _p(w), max(w.shape[0], 1), _p(out)))
+        # the library stores (p,q,r,s) at p + norb*(q + norb*(r + norb*s)): the [k, b] block read in C order is [s, r, q, p]
+        out = np.ascontiguousarray(out.transpose(0, 1, 5, 4, 3, 2))
+        return out[0] if one else out
+
     def second_order_pt(self, dets_up, dets_dn, wts, var_energy, eps_pt):
         """Deterministic second-order PT with the HCI screened sum (second_order_pt, hci.f90:1100-1182) -> (delta_e_2pt, ndets_connected)."""
         up = np.ascontiguousarray(dets_up, dtype=np.uint64).reshape(-1, 2)

@@ -451,6 +451,13 @@ int sqmc_b200_one_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const
   return one_rdm(h, n, dets_up, dets_dn, n_states, wts, ldw, rdm);
 }
 
+int sqmc_b200_two_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw,
+                      double *rdm2) {
+  SQ_CHECK(require_init());
+  if (!h || !dets_up || !dets_dn || !wts || !rdm2) { set_error("two_rdm: null argument"); return 2; }
+  return two_rdm(h, n, dets_up, dets_dn, n_states, wts, ldw, rdm2);
+}
+
 int sqmc_b200_pt2(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, const double *wts, double var_energy, double eps_pt,
                   double *delta_e, int64_t *n_connected) {
   SQ_CHECK(require_init());

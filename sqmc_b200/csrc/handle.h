@@ -278,4 +278,5 @@ int lanczos(sqmc_b200_handle *h, const double *v0, double *evec, double *eig3, d
             int ritz_log_cap, int *n_ritz_logged);
 // rdm.cu
 int one_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw, double *rdm);
+int two_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw, double *rdm2);
 }  // namespace sqmc

@@ -1,4 +1,4 @@
-// rdm.cu -- one-particle density matrices of variational wavefunctions (sqmc_b200_one_rdm).
+// rdm.cu -- one- and two-particle density matrices of variational wavefunctions (sqmc_b200_one_rdm, sqmc_b200_two_rdm).
 //
 //   rdm[s][sigma](p,q) = <Psi_s| a+_{p sigma} a_{q sigma} |Psi_s>,   Psi_s = sum_i wts(i,s) |D_i>
 //
@@ -21,6 +21,7 @@
 #include <thrust/iterator/counting_iterator.h>
 
 #include <cub/cub.cuh>
+#include <vector>
 
 #include "handle.h"
 
@@ -246,21 +247,23 @@ static int make_view(int norb, const uint64_t *major, const uint64_t *minor, con
   return 0;
 }
 
+// The part both density matrices share: upload, the time_sym expansion to n2 plain determinants (up, dn, w column-major
+// n2 x S), and view 0 (sorted by (up, dn): idx0, ma0 = up, mi0 = dn, c0 interleaved) with the duplicate and partner check.
 template <int NW>
-static int one_rdm_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int S, const double *wts, int64_t ldw, double *rdm) {
+static int prepare_dets(sqmc_b200_handle *h, const char *who, int64_t n, const void *dets_up, const void *dets_dn, int S, const double *wts,
+                        int64_t ldw, DevBuf<uint64_t> &up, DevBuf<uint64_t> &dn, DevBuf<double> &w, int64_t &n2, DevBuf<int32_t> &idx0,
+                        DevBuf<uint64_t> &ma0, DevBuf<uint64_t> &mi0, DevBuf<double> &c0) {
   cudaStream_t s = G.stream;
   const ModelTables &T = h->T;
   const int norb = T.norb;
   const bool ts = T.model == MODEL_CHEM && T.time_sym;
-  DevBuf<uint64_t> up, dn;
-  DevBuf<double> w;
   SQ_CHECK(up.alloc(n * NW));
   SQ_CHECK(dn.alloc(n * NW));
   SQ_CHECK(upload_dets(NW, norb, dets_up, up.p, n, s));
   SQ_CHECK(upload_dets(NW, norb, dets_dn, dn.p, n, s));
   SQ_CHECK(w.alloc(n * S));
   SQ_CUDA(cudaMemcpy2DAsync(w.p, n * sizeof(double), wts, ldw * sizeof(double), n * sizeof(double), S, cudaMemcpyHostToDevice, s));
-  int64_t n2 = n;
+  n2 = n;
   if (ts) {
     DevBuf<int32_t> flag, sel, nsel;
     SQ_CHECK(flag.alloc(n));
@@ -279,7 +282,7 @@ static int one_rdm_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, con
     SQ_CUDA(cudaMemcpyAsync(&m, nsel.p, sizeof(int), cudaMemcpyDeviceToHost, s));
     SQ_CUDA(cudaStreamSynchronize(s));
     n2 = n + m;
-    if (n2 > INT32_MAX) { set_error("one_rdm: %lld plain determinants after the time-reversal expansion exceed the 32-bit row index", (long long)n2); return 2; }
+    if (n2 > INT32_MAX) { set_error("%s: %lld plain determinants after the time-reversal expansion exceed the 32-bit row index", who, (long long)n2); return 2; }
     DevBuf<uint64_t> eu, ed;
     DevBuf<double> ew;
     SQ_CHECK(eu.alloc(n2 * NW));
@@ -292,25 +295,34 @@ static int one_rdm_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, con
     up.n = dn.n = n2 * NW;
     w.n = n2 * S;
   }
+  SQ_CHECK(make_view<NW>(norb, up.p, dn.p, w.p, n2, S, idx0, ma0, mi0, c0, s));
+  DevBuf<int> flag;
+  SQ_CHECK(flag.alloc(1));
+  SQ_CUDA(cudaMemsetAsync(flag.p, 0, sizeof(int), s));
+  if (n2 > 1) {
+    duplicate_kernel<NW><<<(unsigned)div_up(n2 - 1, 256), 256, 0, s>>>(ma0.p, mi0.p, idx0.p, n2, n, flag.p);
+    SQ_LAUNCH_CHECK();
+  }
+  int hf = 0;
+  SQ_CUDA(cudaMemcpyAsync(&hf, flag.p, sizeof(int), cudaMemcpyDeviceToHost, s));
+  SQ_CUDA(cudaStreamSynchronize(s));
+  if (hf & 1) { set_error("%s: the determinant list holds a determinant twice", who); return 2; }
+  if (hf & 2) { set_error("%s: the list holds both (u,d) and its time-reversed partner (d,u); pass one representative per pair", who); return 2; }
+  return 0;
+}
+
+template <int NW>
+static int one_rdm_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int S, const double *wts, int64_t ldw, double *rdm) {
+  cudaStream_t s = G.stream;
+  const int norb = h->T.norb;
   // view 0: (up, dn) order, beta singles; view 1: (dn, up) order, alpha singles
+  DevBuf<uint64_t> up, dn;
+  DevBuf<double> w;
+  int64_t n2 = 0;
   DevBuf<int32_t> idx0, idx1;
   DevBuf<uint64_t> ma0, mi0, ma1, mi1;
   DevBuf<double> c0, c1;
-  SQ_CHECK(make_view<NW>(norb, up.p, dn.p, w.p, n2, S, idx0, ma0, mi0, c0, s));
-  {
-    DevBuf<int> flag;
-    SQ_CHECK(flag.alloc(1));
-    SQ_CUDA(cudaMemsetAsync(flag.p, 0, sizeof(int), s));
-    if (n2 > 1) {
-      duplicate_kernel<NW><<<(unsigned)div_up(n2 - 1, 256), 256, 0, s>>>(ma0.p, mi0.p, idx0.p, n2, n, flag.p);
-      SQ_LAUNCH_CHECK();
-    }
-    int hf = 0;
-    SQ_CUDA(cudaMemcpyAsync(&hf, flag.p, sizeof(int), cudaMemcpyDeviceToHost, s));
-    SQ_CUDA(cudaStreamSynchronize(s));
-    if (hf & 1) { set_error("one_rdm: the determinant list holds a determinant twice"); return 2; }
-    if (hf & 2) { set_error("one_rdm: the list holds both (u,d) and its time-reversed partner (d,u); pass one representative per pair"); return 2; }
-  }
+  SQ_CHECK(prepare_dets<NW>(h, "one_rdm", n, dets_up, dets_dn, S, wts, ldw, up, dn, w, n2, idx0, ma0, mi0, c0));
   SQ_CHECK(make_view<NW>(norb, dn.p, up.p, w.p, n2, S, idx1, ma1, mi1, c1, s));
   up.release(); dn.release(); w.release(); idx0.release(); idx1.release();
 
@@ -345,6 +357,348 @@ int one_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *det
   if (n > INT32_MAX) { set_error("one_rdm: n exceeds the 32-bit row index"); return 2; }
   return h->NW == 1 ? one_rdm_impl<1>(h, n, dets_up, dets_dn, n_states, wts, ldw, rdm)
                     : one_rdm_impl<2>(h, n, dets_up, dets_dn, n_states, wts, ldw, rdm);
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// two-particle density matrix (sqmc_b200_two_rdm), one-word strings
+//
+//   Gamma^{st}_{pq,rs} = <Psi| a+_{p s} a+_{r t} a_{s t} a_{q s} |Psi>,   blocks b = 0 (alpha alpha), 1 (alpha beta), 2 (beta beta)
+//
+// Pairs of determinants: every determinant emits hole keys of three classes, each class is sorted by key, and every pair of
+// entries inside a run of equal keys (a bucket) is a connected pair met exactly once in that class:
+//   same spin (alpha; beta mirrored): key (u \ {a,b}, d).  A pair whose removed sets are disjoint is an alpha double and has
+//     exactly this one bucket.  A pair sharing one removed orbital r is an alpha single j -> i; it lies in N_alpha - 1 buckets,
+//     one per r in u_i & u_j, and in each adds its one term Gamma^{aa}_{x_i x_j, r r}.
+//   alpha beta: key (u \ {a}, d \ {b}).  Both removed orbitals differ: an alpha-beta double, one bucket.  Only a differs: an
+//     alpha single, met once per beta orbital b, adding Gamma^{ab}_{x_i x_j, b b}; only b differs: the beta mirror.
+// The diagonal terms c^2 of each determinant are added by a separate kernel that pre-reduces them per block in shared memory.
+// Signs are the products of single-excitation permutation factors (alpha string first: beta operators pass every alpha
+// electron twice), as in chem_single / chem_double.
+//
+// Only one representative per symmetry orbit is accumulated, and a fill kernel writes every element from its representative:
+//   Gamma_{pq,rs} = Gamma_{qp,sr};  same spin also Gamma_{pq,rs} = -Gamma_{rq,ps} = -Gamma_{ps,rq}, and 0 when p = r or q = s.
+// Same-spin representatives are indexed by the creator pair A = {p < r} and the annihilator pair B = {q < s}, A <= B; alpha-beta
+// ones by (p + norb q, r + norb s) or its Hermitian image, whichever is smaller.
+//
+// Determinism: each representative is a 128-bit two's-complement fixed-point integer per state k, in units of 2^(e_k - 120)
+// with 2^e_k >= sum_i c_ik^2 (by Cauchy-Schwarz no element exceeds that).  A term sign * c_i * c_j is rounded once to that grid
+// and added with a 64-bit atomic on the low word plus the carry and sign extension on the high word.  Integer addition does not
+// depend on order, so repeated calls and permuted rows give the same bits.
+static const int kFixBits = 120;
+
+__device__ __forceinline__ int par_between(uint64_t x, int a, int b) {  // parity of the electrons of x strictly between a and b
+  const int lo = min(a, b), hi = max(a, b);
+  return __popcll(x & ((1ull << hi) - 1ull) & ~((2ull << lo) - 1ull)) & 1;
+}
+
+// x (already on the fixed-point grid, |x| < 2^126) rounded to a 128-bit two's-complement integer (lo, hi)
+__device__ __forceinline__ void fix_to_i128(double x, uint64_t &lo, uint64_t &hi) {
+  if (fabs(x) < 9.0e18) {
+    const long long v = __double2ll_rn(x);
+    lo = (uint64_t)v;
+    hi = v < 0 ? ~0ull : 0ull;
+  } else {  // already an integer: the 53-bit mantissa shifted into place
+    int e;
+    const double m = frexp(x, &e);
+    const __int128 v = (__int128)(long long)ldexp(m, 53) << (e - 53);
+    lo = (uint64_t)v;
+    hi = (uint64_t)(v >> 64);
+  }
+}
+// adds (lo, hi) to the 128-bit value at slot[0] (low word), slot[1] (high word), global or shared memory
+__device__ __forceinline__ void i128_add(unsigned long long *slot, uint64_t lo, uint64_t hi) {
+  if ((lo | hi) == 0) return;
+  const unsigned long long old = atomicAdd(slot, (unsigned long long)lo);
+  const uint64_t h = hi + ((old + lo < old) ? 1ull : 0ull);
+  if (h) atomicAdd(slot + 1, (unsigned long long)h);
+}
+
+__device__ __forceinline__ int pair_index(int p, int r) { return r * (r - 1) / 2 + p; }  // p < r
+// representative of the same-spin element (p,q,r,s), p != r, q != s, inside an M x M block; sg: element = sg * representative
+__device__ __forceinline__ int64_t ss_slot(int p, int q, int r, int s, int M, int &sg) {
+  sg = 1;
+  if (p > r) { const int t = p; p = r; r = t; sg = -sg; }
+  if (q > s) { const int t = q; q = s; s = t; sg = -sg; }
+  const int64_t A = pair_index(p, r), B = pair_index(q, s);
+  return A <= B ? A + M * B : B + M * A;
+}
+__device__ __forceinline__ int64_t ab_slot(int p, int q, int r, int s, int norb) {
+  int64_t X = p + (int64_t)norb * q, Y = r + (int64_t)norb * s;
+  const int64_t X2 = q + (int64_t)norb * p, Y2 = s + (int64_t)norb * r;
+  if (X2 < X || (X2 == X && Y2 < Y)) { X = X2; Y = Y2; }
+  return X + (int64_t)norb * norb * Y;
+}
+
+struct Rdm2Acc {
+  unsigned long long *a;  // [S][per] slots of two words
+  const double *scale;    // [S] 2^(120 - e_k)
+  int64_t per, off_bb, off_ab;
+  int M, norb, S;
+};
+
+__global__ void electron_count_kernel(const uint64_t *u, const uint64_t *d, int64_t n, int nup, int ndn, int *bad) {
+  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (i < n && (__popcll(u[i]) != nup || __popcll(d[i]) != ndn)) atomicOr(bad, 1);
+}
+
+// same-spin keys: (x \ {a, b}, y) for every pair a < b of x; payload row << 16 | a | b << 8
+__global__ void rdm2_keys_same_kernel(const uint64_t *x, const uint64_t *y, int64_t n, int K, uint64_t *ku, uint64_t *kd, uint64_t *pay) {
+  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const uint64_t X = x[i], Y = y[i];
+  int64_t e = i * K;
+  for (uint64_t as = X; as; as &= as - 1) {
+    const int a = __ffsll((long long)as) - 1;
+    for (uint64_t bs = as & (as - 1); bs; bs &= bs - 1) {
+      const int b = __ffsll((long long)bs) - 1;
+      ku[e] = X & ~(1ull << a) & ~(1ull << b);
+      kd[e] = Y;
+      pay[e] = (uint64_t)i << 16 | (uint64_t)a | (uint64_t)b << 8;
+      e++;
+    }
+  }
+}
+// alpha-beta keys: (u \ {a}, d \ {b}); payload row << 16 | a | b << 8
+__global__ void rdm2_keys_ab_kernel(const uint64_t *u, const uint64_t *d, int64_t n, int K, uint64_t *ku, uint64_t *kd, uint64_t *pay) {
+  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const uint64_t U = u[i], D = d[i];
+  int64_t e = i * K;
+  for (uint64_t as = U; as; as &= as - 1) {
+    const int a = __ffsll((long long)as) - 1;
+    for (uint64_t bs = D; bs; bs &= bs - 1) {
+      const int b = __ffsll((long long)bs) - 1;
+      ku[e] = U & ~(1ull << a);
+      kd[e] = D & ~(1ull << b);
+      pay[e] = (uint64_t)i << 16 | (uint64_t)a | (uint64_t)b << 8;
+      e++;
+    }
+  }
+}
+
+// one thread per sorted entry i: every later entry j of the same bucket; boff: block offset of a same-spin class, -1: alpha beta
+__global__ void __launch_bounds__(256) rdm2_pair_kernel(const uint64_t *ku, const uint64_t *kd, const uint64_t *pay, int64_t m, int64_t boff,
+                                                        const double *coef, Rdm2Acc R) {
+  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (i >= m) return;
+  const uint64_t ki = ku[i], kdi = kd[i], pi = pay[i];
+  const int ai = (int)(pi & 0xff), bi = (int)((pi >> 8) & 0xff);
+  const double *ci = coef + (int64_t)(pi >> 16) * R.S;
+  for (int64_t j = i + 1; j < m && ku[j] == ki && kd[j] == kdi; j++) {
+    const uint64_t pj = pay[j];
+    const int aj = (int)(pj & 0xff), bj = (int)((pj >> 8) & 0xff);
+    int neg, sg = 1;
+    int64_t slot;
+    if (boff >= 0) {
+      int p, q, r, s;
+      if (ai != aj && ai != bj && bi != aj && bi != bj) {  // double: <i| a+_ai a+_bi a_bj a_aj |j> = <i| a+_ai a_aj a+_bi a_bj |j>
+        const uint64_t uj = ki | 1ull << aj | 1ull << bj;
+        neg = par_between(uj, bi, bj) ^ par_between(uj ^ (1ull << bj) ^ (1ull << bi), ai, aj);
+        p = ai; q = aj; r = bi; s = bj;
+      } else {  // single x_j -> x_i; the shared removed orbital r stays occupied in both
+        const int r0 = (ai == aj || ai == bj) ? ai : bi;
+        const int xi = ai == r0 ? bi : ai, xj = aj == r0 ? bj : aj;
+        neg = par_between(ki | 1ull << r0, xi, xj);
+        p = xi; q = xj; r = r0; s = r0;
+      }
+      slot = boff + ss_slot(p, q, r, s, R.M, sg);
+    } else if (ai != aj && bi != bj) {
+      neg = par_between(ki, ai, aj) ^ par_between(kdi, bi, bj);
+      slot = R.off_ab + ab_slot(ai, aj, bi, bj, R.norb);
+    } else if (ai != aj) {
+      neg = par_between(ki, ai, aj);
+      slot = R.off_ab + ab_slot(ai, aj, bi, bi, R.norb);
+    } else {
+      neg = par_between(kdi, bi, bj);
+      slot = R.off_ab + ab_slot(ai, ai, bi, bj, R.norb);
+    }
+    const double f = (neg ? -1.0 : 1.0) * sg;
+    const double *cj = coef + (int64_t)(pj >> 16) * R.S;
+    for (int k = 0; k < R.S; k++) {
+      uint64_t lo, hi;
+      fix_to_i128(f * (ci[k] * cj[k]) * R.scale[k], lo, hi);
+      i128_add(R.a + 2 * (k * R.per + slot), lo, hi);
+    }
+  }
+}
+
+// diagonal terms c_i^2: Gamma^{ss}_{pp,rr} (p < r occupied in the same string) and Gamma^{ab}_{pp,rr}, one state at a time,
+// summed per block in shared memory ([3][norb][norb] 128-bit values) and then added to the representatives
+__global__ void __launch_bounds__(256) rdm2_diag_kernel(const uint64_t *u, const uint64_t *d, int64_t n, const double *coef, Rdm2Acc R) {
+  extern __shared__ unsigned long long sd[];
+  const int norb = R.norb, nn = norb * norb;
+  for (int k = 0; k < R.S; k++) {
+    for (int t = threadIdx.x; t < 6 * nn; t += blockDim.x) sd[t] = 0ull;
+    __syncthreads();
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+      const double c = coef[i * R.S + k];
+      uint64_t lo, hi;
+      fix_to_i128((c * c) * R.scale[k], lo, hi);
+      if ((lo | hi) == 0) continue;
+      const uint64_t U = u[i], D = d[i];
+      for (uint64_t ps = U; ps; ps &= ps - 1) {
+        const int p = __ffsll((long long)ps) - 1;
+        for (uint64_t rs = ps & (ps - 1); rs; rs &= rs - 1) i128_add(sd + 2 * (p * norb + __ffsll((long long)rs) - 1), lo, hi);
+        for (uint64_t rs = D; rs; rs &= rs - 1) i128_add(sd + 2 * (2 * nn + p * norb + __ffsll((long long)rs) - 1), lo, hi);
+      }
+      for (uint64_t ps = D; ps; ps &= ps - 1) {
+        const int p = __ffsll((long long)ps) - 1;
+        for (uint64_t rs = ps & (ps - 1); rs; rs &= rs - 1) i128_add(sd + 2 * (nn + p * norb + __ffsll((long long)rs) - 1), lo, hi);
+      }
+    }
+    __syncthreads();
+    for (int t = threadIdx.x; t < 3 * nn; t += blockDim.x) {
+      const uint64_t lo = sd[2 * t], hi = sd[2 * t + 1];
+      if ((lo | hi) == 0) continue;
+      const int b = t / nn, p = (t % nn) / norb, r = t % norb;
+      int64_t slot;
+      if (b == 2) {
+        slot = R.off_ab + ab_slot(p, p, r, r, norb);
+      } else {
+        const int64_t A = pair_index(p, r);
+        slot = (b ? R.off_bb : 0) + A + R.M * A;
+      }
+      i128_add(R.a + 2 * (k * R.per + slot), lo, hi);
+    }
+    __syncthreads();
+  }
+}
+
+// every element of the output (column-major p, q, r, s, block, state) from its representative
+__global__ void rdm2_fill_kernel(Rdm2Acc R, const double *unscale, double *out) {
+  const int norb = R.norb;
+  const int64_t n4 = (int64_t)norb * norb * norb * norb, total = n4 * 3 * R.S;
+  for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < total; t += (int64_t)gridDim.x * blockDim.x) {
+    int64_t x = t;
+    const int p = (int)(x % norb); x /= norb;
+    const int q = (int)(x % norb); x /= norb;
+    const int r = (int)(x % norb); x /= norb;
+    const int s = (int)(x % norb); x /= norb;
+    const int b = (int)(x % 3);
+    const int k = (int)(x / 3);
+    int sg = 1;
+    int64_t slot;
+    if (b == 1) {
+      slot = R.off_ab + ab_slot(p, q, r, s, norb);
+    } else if (p == r || q == s) {
+      out[t] = 0.0;
+      continue;
+    } else {
+      slot = (b ? R.off_bb : 0) + ss_slot(p, q, r, s, R.M, sg);
+    }
+    const unsigned long long *v = R.a + 2 * (k * R.per + slot);
+    const double a = (ldexp((double)(long long)v[1], 64) + (double)v[0]) * unscale[k];
+    out[t] = sg < 0 ? -a : a;
+  }
+}
+
+static int two_rdm_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int S, const double *wts, int64_t ldw, double *rdm) {
+  cudaStream_t s = G.stream;
+  const ModelTables &T = h->T;
+  const int norb = T.norb;
+  HostMarks marks("SQMC_RDM2_PROFILE", "two_rdm");  // =1: phase split (synchronising) on stderr
+  DevBuf<uint64_t> up, dn, U, D;
+  DevBuf<double> w, c;
+  DevBuf<int32_t> idx0;
+  int64_t n2 = 0;
+  SQ_CHECK(prepare_dets<1>(h, "two_rdm", n, dets_up, dets_dn, S, wts, ldw, up, dn, w, n2, idx0, U, D, c));
+  up.release(); dn.release(); w.release(); idx0.release();
+  marks.mark("upload, expansion, checks");
+  {
+    DevBuf<int> bad;
+    SQ_CHECK(bad.alloc(1));
+    SQ_CUDA(cudaMemsetAsync(bad.p, 0, sizeof(int), s));
+    electron_count_kernel<<<(unsigned)div_up(n2, 256), 256, 0, s>>>(U.p, D.p, n2, T.nup, T.ndn, bad.p);
+    SQ_LAUNCH_CHECK();
+    int hb = 0;
+    SQ_CUDA(cudaMemcpyAsync(&hb, bad.p, sizeof(int), cudaMemcpyDeviceToHost, s));
+    SQ_CUDA(cudaStreamSynchronize(s));
+    if (hb) { set_error("two_rdm: a determinant does not hold %d alpha and %d beta electrons", T.nup, T.ndn); return 2; }
+  }
+  // grid exponent per state from sum_i w_ik^2 (the time_sym expansion keeps it); the margin keeps e_k the same whatever order
+  // the sum was taken in, unless the norm lies within a few ulps of 2^e / (1 + 2^-20)
+  std::vector<double> hs(2 * S);
+  for (int k = 0; k < S; k++) {
+    double n2k = 0.0;
+    for (int64_t i = 0; i < n; i++) n2k += wts[k * ldw + i] * wts[k * ldw + i];
+    int e = 0;
+    if (n2k > 0.0) frexp(n2k * (1.0 + 0x1p-20), &e);
+    hs[k] = ldexp(1.0, kFixBits - e);
+    hs[S + k] = ldexp(1.0, e - kFixBits);
+  }
+  const int M = norb * (norb - 1) / 2;
+  const int64_t n4 = (int64_t)norb * norb * norb * norb;
+  Rdm2Acc R;
+  R.M = M; R.norb = norb; R.S = S;
+  R.off_bb = (int64_t)M * M;
+  R.off_ab = 2 * R.off_bb;
+  R.per = R.off_ab + n4;
+  DevBuf<unsigned long long> acc;
+  DevBuf<double> scale;
+  SQ_CHECK(acc.alloc(2 * S * R.per));
+  SQ_CHECK(scale.alloc(2 * S));
+  SQ_CUDA(cudaMemsetAsync(acc.p, 0, (size_t)acc.n * sizeof(unsigned long long), s));
+  SQ_CUDA(cudaMemcpyAsync(scale.p, hs.data(), 2 * S * sizeof(double), cudaMemcpyHostToDevice, s));
+  R.a = acc.p;
+  R.scale = scale.p;
+
+  const size_t dsh = (size_t)6 * norb * norb * sizeof(unsigned long long);
+  SQ_CUDA(cudaFuncSetAttribute(rdm2_diag_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dsh));
+  rdm2_diag_kernel<<<(unsigned)std::min<int64_t>(div_up(n2, 256), 2 * G.sm_count), 256, dsh, s>>>(U.p, D.p, n2, c.p, R);
+  SQ_LAUNCH_CHECK();
+  marks.mark("diagonal");
+
+  // class 0: alpha holes (block 0), 1: beta holes (block 2), 2: one hole of each spin (block 1)
+  for (int cls = 0; cls < 3; cls++) {
+    const int K = cls == 0 ? T.nup * (T.nup - 1) / 2 : cls == 1 ? T.ndn * (T.ndn - 1) / 2 : T.nup * T.ndn;
+    if (K == 0 || n2 < 2) continue;
+    const int64_t m = n2 * K;
+    if (m > INT32_MAX) { set_error("two_rdm: %lld hole keys (%lld determinants x %d) exceed the 32-bit sort index", (long long)m, (long long)n2, K); return 2; }
+    DevBuf<uint64_t> ku, kd, pay, sku, skd, spay;
+    DevBuf<int32_t> idx;
+    SQ_CHECK(ku.alloc(m));
+    SQ_CHECK(kd.alloc(m));
+    SQ_CHECK(pay.alloc(m));
+    if (cls == 2) rdm2_keys_ab_kernel<<<(unsigned)div_up(n2, 256), 256, 0, s>>>(U.p, D.p, n2, K, ku.p, kd.p, pay.p);
+    else rdm2_keys_same_kernel<<<(unsigned)div_up(n2, 256), 256, 0, s>>>(cls ? D.p : U.p, cls ? U.p : D.p, n2, K, ku.p, kd.p, pay.p);
+    SQ_LAUNCH_CHECK();
+    SQ_CHECK(idx.alloc(m));
+    SQ_CHECK(sort_pairs_index(1, norb, ku.p, kd.p, idx.p, m, s));
+    SQ_CHECK(sku.alloc(m));
+    SQ_CHECK(gather_strings(1, ku.p, idx.p, sku.p, m, s));
+    ku.release();
+    SQ_CHECK(skd.alloc(m));
+    SQ_CHECK(gather_strings(1, kd.p, idx.p, skd.p, m, s));
+    kd.release();
+    SQ_CHECK(spay.alloc(m));
+    SQ_CHECK(gather_strings(1, pay.p, idx.p, spay.p, m, s));
+    pay.release(); idx.release();
+    marks.mark(cls == 0 ? "alpha alpha keys + sort" : cls == 1 ? "beta beta keys + sort" : "alpha beta keys + sort");
+    rdm2_pair_kernel<<<(unsigned)div_up(m, 256), 256, 0, s>>>(sku.p, skd.p, spay.p, m, cls == 2 ? -1 : cls == 0 ? 0 : R.off_bb, c.p, R);
+    SQ_LAUNCH_CHECK();
+    marks.mark(cls == 0 ? "alpha alpha pairs" : cls == 1 ? "beta beta pairs" : "alpha beta pairs");
+  }
+  DevBuf<double> out;
+  SQ_CHECK(out.alloc(3 * S * n4));
+  rdm2_fill_kernel<<<(unsigned)std::min<int64_t>(div_up(3 * S * n4, 256), 64 * G.sm_count), 256, 0, s>>>(R, scale.p + S, out.p);
+  SQ_LAUNCH_CHECK();
+  SQ_CUDA(cudaMemcpyAsync(rdm, out.p, (size_t)out.n * sizeof(double), cudaMemcpyDeviceToHost, s));
+  SQ_CUDA(cudaStreamSynchronize(s));
+  marks.mark("fill + copy out");
+  return 0;
+}
+
+int two_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw, double *rdm) {
+  if (n <= 0) { set_error("two_rdm: n must be positive"); return 2; }
+  if (n_states < 1) { set_error("two_rdm: n_states must be >= 1"); return 2; }
+  if (ldw < n) { set_error("two_rdm: ldw (%lld) must be >= n (%lld)", (long long)ldw, (long long)n); return 2; }
+  if (n > INT32_MAX) { set_error("two_rdm: n exceeds the 32-bit row index"); return 2; }
+  if (h->T.norb > 64) {
+    set_error("two_rdm: norb = %d > 64 is not supported (the dense output holds 3*norb^4 doubles per state, and strings of more than one word are not handled)",
+              h->T.norb);
+    return 2;
+  }
+  return two_rdm_impl(h, n, dets_up, dets_dn, n_states, wts, ldw, rdm);
 }
 
 }  // namespace sqmc
