@@ -137,6 +137,23 @@ int sqmc_b200_one_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const
 int sqmc_b200_two_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states,
                       const double *wts, int64_t ldw, double *rdm2);
 
+/* ---- orbital gradient and Hessian (orbital optimisation) ------------------------------------------------------------
+ * Derivatives at kappa = 0 of the state-averaged variational energy E(kappa) = E_core + sum h'D + 1/2 sum g'd under a real orbital
+ * rotation kappa = sum_{p>q} k_pq (E_pq - E_qp) (Helgaker, Jorgensen, Olsen, 10.8.1), chem handles only, norb <= 64:
+ *   D_pq = sum_k w_k (gamma^a + gamma^b)_pq / ||Psi_k||^2,  d_pqrs = sum_k w_k (G^aa + G^bb + G^ab_pq,rs + G^ab_rs,pq) / ||Psi_k||^2,
+ *   with h_pq, g_pqrs = (pq|rs) read from the handle's integral table in the library's orbital numbering.
+ * fock:    norb^2 doubles, F_pq = sum_m D_pm h_qm + sum_mnt d_pmnt g_qmnt at p + norb*q; the gradient is 2 (F_pq - F_qp).
+ * hessian: norb^4 doubles, E2_pq,rs = (1 - P_pq)(1 - P_rs)[2 D_pr h_qs - (F_pr + F_rp) delta_qs + 2 Y_pqrs],
+ *          Y_pqrs = sum_mn [(d_pmrn + d_pmnr) g_qmsn + d_prmn g_qsmn], at p + norb*(q + norb*(r + norb*s)).
+ * energy:  1 double, E_core + sum h D + 1/2 sum g d = sum_k w_k E_k.
+ * Arguments, orbital numbering, time_sym handling and errors are those of sqmc_b200_two_rdm; in addition the handle must be
+ * chem, hold at least two electrons, and state_weights (n_states values) must be >= 0 and sum to 1 within 1e-12.
+ * The density matrices and integrals stay on the device; every output is summed in a fixed order, so the result is
+ * bit-identical across calls and row permutations. */
+int sqmc_b200_orbital_derivatives(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states,
+                                  const double *wts, int64_t ldw, const double *state_weights,
+                                  double *fock, double *hessian, double *energy);
+
 /* ---- sparse H build --------------------------------------------------------
  * Replaces generate_sparse_ham_chem_upper_triangular (chemistry.f90:7639),
  * its _mpi twin (:8012), generate_sparse_ham_heg_upper_triangular

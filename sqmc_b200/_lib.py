@@ -22,7 +22,7 @@ SYMBOLS = [
     "sqmc_b200_hci_new_dets", "sqmc_b200_set_hf_to_psit",
     "sqmc_b200_set_ownership", "sqmc_b200_matvec_local", "sqmc_b200_projector_local", "sqmc_b200_davidson_local",
     "sqmc_b200_last_build_incremental", "sqmc_b200_alloc_stall_ms", "sqmc_b200_register_host", "sqmc_b200_unregister_host", "sqmc_b200_exchange_mode",
-    "sqmc_b200_one_rdm", "sqmc_b200_two_rdm",
+    "sqmc_b200_one_rdm", "sqmc_b200_two_rdm", "sqmc_b200_orbital_derivatives",
 ]
 
 
@@ -64,6 +64,7 @@ def load():
     L.sqmc_b200_set_row_bundle.argtypes = [vp, i32]
     L.sqmc_b200_one_rdm.argtypes = [vp, i64, vp, vp, i32, vp, i64, vp]
     L.sqmc_b200_two_rdm.argtypes = [vp, i64, vp, vp, i32, vp, i64, vp]
+    L.sqmc_b200_orbital_derivatives.argtypes = [vp, i64, vp, vp, i32, vp, i64, vp, vp, vp, vp]
     L.sqmc_b200_pt2.argtypes = [vp, i64, vp, vp, vp, dbl, dbl, vp, vp]
     L.sqmc_b200_pt2_sample.argtypes = [vp, i64, vp, vp, i64, vp, vp, vp, vp, i32, dbl, dbl, dbl, vp, vp]
     L.sqmc_b200_pt2_alias.argtypes = [vp, i64, vp, vp, vp, dbl, dbl, dbl, i32, dbl, vp, i32, vp, vp, vp, vp, vp]

@@ -336,6 +336,34 @@ class SparseHamiltonian:
         out = np.ascontiguousarray(out.transpose(0, 1, 5, 4, 3, 2))
         return out[0] if one else out
 
+    def orbital_derivatives(self, dets_up, dets_dn, wts, state_weights=None):
+        """Orbital gradient and Hessian at kappa = 0 of the state-averaged variational energy
+        E(kappa) = E_core + sum h'D + 1/2 sum g'd, h' = U^T h U and (pq|rs)' rotated alike (natorb.rotate_fcidump with C = U),
+        U = expm(-kappa), kappa[p,q] = k_pq = -kappa[q,p] (p > q), in the library's orbital numbering (chem only, norb <= 64).  D and d are the
+        spin-summed density matrices of every state normalised to ||Psi_k|| = 1 and averaged with state_weights (default equal).
+        The determinant list, wts and time_sym handling are those of two_rdm.
+        -> dict(fock [p, q] = F_pq, gradient = 2 (F - F^T), hessian [p, q, r, s] = d^2 E / dk_pq dk_rs (extended
+        antisymmetrically to p < q, r < s), energy = sum_k w_k E_k)."""
+        up = np.ascontiguousarray(dets_up, dtype=np.uint64).reshape(-1, 2)
+        dn = np.ascontiguousarray(dets_dn, dtype=np.uint64).reshape(-1, 2)
+        w = np.asarray(wts, dtype=np.float64)
+        w = np.asfortranarray(w.reshape(-1, 1) if w.ndim == 1 else w)
+        if len(dn) != len(up) or w.shape[0] != len(up):
+            raise ValueError("orbital_derivatives: dets_up, dets_dn and wts must have the same number of rows")
+        norb, ns = self.system.norb, w.shape[1]
+        sw = np.full(max(ns, 1), 1.0 / max(ns, 1)) if state_weights is None else np.ascontiguousarray(state_weights, dtype=np.float64).reshape(-1)
+        if len(sw) != ns:
+            raise ValueError("orbital_derivatives: state_weights holds %d values for %d states" % (len(sw), ns))
+        small = norb <= 64   # the library rejects norb > 64
+        fock = np.zeros((norb, norb) if small else 1)
+        hess = np.zeros((norb,) * 4 if small else 1)
+        e = np.zeros(1)
+        check(self._L.sqmc_b200_orbital_derivatives(self._h, len(up), _p(up), _p(dn), ns, _p(w), max(w.shape[0], 1), _p(sw), _p(fock),
+                                                    _p(hess), _p(e)))
+        # (p,q) at p + norb*q and (p,q,r,s) at p + norb*(q + norb*(r + norb*s)): read in C order they come out reversed
+        fock = np.ascontiguousarray(fock.T)
+        return dict(fock=fock, gradient=2.0 * (fock - fock.T), hessian=np.ascontiguousarray(hess.transpose(3, 2, 1, 0)), energy=float(e[0]))
+
     def second_order_pt(self, dets_up, dets_dn, wts, var_energy, eps_pt):
         """Deterministic second-order PT with the HCI screened sum (second_order_pt, hci.f90:1100-1182) -> (delta_e_2pt, ndets_connected)."""
         up = np.ascontiguousarray(dets_up, dtype=np.uint64).reshape(-1, 2)

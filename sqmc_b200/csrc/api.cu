@@ -458,6 +458,16 @@ int sqmc_b200_two_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const
   return two_rdm(h, n, dets_up, dets_dn, n_states, wts, ldw, rdm2);
 }
 
+int sqmc_b200_orbital_derivatives(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts,
+                                  int64_t ldw, const double *state_weights, double *fock, double *hessian, double *energy) {
+  SQ_CHECK(require_init());
+  if (!h || !dets_up || !dets_dn || !wts || !state_weights || !fock || !hessian || !energy) {
+    set_error("orbital_derivatives: null argument");
+    return 2;
+  }
+  return orbital_derivatives(h, n, dets_up, dets_dn, n_states, wts, ldw, state_weights, fock, hessian, energy);
+}
+
 int sqmc_b200_pt2(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, const double *wts, double var_energy, double eps_pt,
                   double *delta_e, int64_t *n_connected) {
   SQ_CHECK(require_init());

@@ -279,4 +279,6 @@ int lanczos(sqmc_b200_handle *h, const double *v0, double *evec, double *eig3, d
 // rdm.cu
 int one_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw, double *rdm);
 int two_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw, double *rdm2);
+int orbital_derivatives(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw,
+                        const double *state_weights, double *fock, double *hessian, double *energy);
 }  // namespace sqmc

@@ -592,16 +592,35 @@ __global__ void rdm2_fill_kernel(Rdm2Acc R, const double *unscale, double *out) 
   }
 }
 
-static int two_rdm_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int S, const double *wts, int64_t ldw, double *rdm) {
+// sum_i c_ik^2 per state over the sorted view (its order does not depend on the caller's rows): thread t sums rows t, t + 256,
+// ... in order, then a fixed tree
+__global__ void __launch_bounds__(256) norm2_kernel(const double *c, int64_t n, int S, double *norm2) {
+  __shared__ double red[256];
+  const int k = blockIdx.x;
+  double a = 0.0;
+  for (int64_t i = threadIdx.x; i < n; i += 256) a += c[i * S + k] * c[i * S + k];
+  red[threadIdx.x] = a;
+  __syncthreads();
+  for (int hh = 128; hh > 0; hh >>= 1) {
+    if (threadIdx.x < hh) red[threadIdx.x] += red[threadIdx.x + hh];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) norm2[k] = red[0];
+}
+
+// The accumulation both two-particle entry points share: upload, time_sym expansion, checks, the diagonal and the three key
+// classes with their pairs.  On return acc / scale hold the representatives of R (scale[S + k]: the factor back to doubles);
+// norm2 (device, S doubles, may be null) receives ||Psi_k||^2 summed in a fixed order.
+static int rdm2_accumulate(sqmc_b200_handle *h, const char *who, int64_t n, const void *dets_up, const void *dets_dn, int S, const double *wts,
+                           int64_t ldw, HostMarks &marks, DevBuf<unsigned long long> &acc, DevBuf<double> &scale, Rdm2Acc &R, double *norm2) {
   cudaStream_t s = G.stream;
   const ModelTables &T = h->T;
   const int norb = T.norb;
-  HostMarks marks("SQMC_RDM2_PROFILE", "two_rdm");  // =1: phase split (synchronising) on stderr
   DevBuf<uint64_t> up, dn, U, D;
   DevBuf<double> w, c;
   DevBuf<int32_t> idx0;
   int64_t n2 = 0;
-  SQ_CHECK(prepare_dets<1>(h, "two_rdm", n, dets_up, dets_dn, S, wts, ldw, up, dn, w, n2, idx0, U, D, c));
+  SQ_CHECK(prepare_dets<1>(h, who, n, dets_up, dets_dn, S, wts, ldw, up, dn, w, n2, idx0, U, D, c));
   up.release(); dn.release(); w.release(); idx0.release();
   marks.mark("upload, expansion, checks");
   {
@@ -613,7 +632,11 @@ static int two_rdm_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, con
     int hb = 0;
     SQ_CUDA(cudaMemcpyAsync(&hb, bad.p, sizeof(int), cudaMemcpyDeviceToHost, s));
     SQ_CUDA(cudaStreamSynchronize(s));
-    if (hb) { set_error("two_rdm: a determinant does not hold %d alpha and %d beta electrons", T.nup, T.ndn); return 2; }
+    if (hb) { set_error("%s: a determinant does not hold %d alpha and %d beta electrons", who, T.nup, T.ndn); return 2; }
+  }
+  if (norm2) {
+    norm2_kernel<<<S, 256, 0, s>>>(c.p, n2, S, norm2);
+    SQ_LAUNCH_CHECK();
   }
   // grid exponent per state from sum_i w_ik^2 (the time_sym expansion keeps it); the margin keeps e_k the same whatever order
   // the sum was taken in, unless the norm lies within a few ulps of 2^e / (1 + 2^-20)
@@ -628,13 +651,10 @@ static int two_rdm_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, con
   }
   const int M = norb * (norb - 1) / 2;
   const int64_t n4 = (int64_t)norb * norb * norb * norb;
-  Rdm2Acc R;
   R.M = M; R.norb = norb; R.S = S;
   R.off_bb = (int64_t)M * M;
   R.off_ab = 2 * R.off_bb;
   R.per = R.off_ab + n4;
-  DevBuf<unsigned long long> acc;
-  DevBuf<double> scale;
   SQ_CHECK(acc.alloc(2 * S * R.per));
   SQ_CHECK(scale.alloc(2 * S));
   SQ_CUDA(cudaMemsetAsync(acc.p, 0, (size_t)acc.n * sizeof(unsigned long long), s));
@@ -653,7 +673,7 @@ static int two_rdm_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, con
     const int K = cls == 0 ? T.nup * (T.nup - 1) / 2 : cls == 1 ? T.ndn * (T.ndn - 1) / 2 : T.nup * T.ndn;
     if (K == 0 || n2 < 2) continue;
     const int64_t m = n2 * K;
-    if (m > INT32_MAX) { set_error("two_rdm: %lld hole keys (%lld determinants x %d) exceed the 32-bit sort index", (long long)m, (long long)n2, K); return 2; }
+    if (m > INT32_MAX) { set_error("%s: %lld hole keys (%lld determinants x %d) exceed the 32-bit sort index", who, (long long)m, (long long)n2, K); return 2; }
     DevBuf<uint64_t> ku, kd, pay, sku, skd, spay;
     DevBuf<int32_t> idx;
     SQ_CHECK(ku.alloc(m));
@@ -678,6 +698,18 @@ static int two_rdm_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, con
     SQ_LAUNCH_CHECK();
     marks.mark(cls == 0 ? "alpha alpha pairs" : cls == 1 ? "beta beta pairs" : "alpha beta pairs");
   }
+  return 0;
+}
+
+static int two_rdm_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int S, const double *wts, int64_t ldw, double *rdm) {
+  cudaStream_t s = G.stream;
+  const int norb = h->T.norb;
+  HostMarks marks("SQMC_RDM2_PROFILE", "two_rdm");  // =1: phase split (synchronising) on stderr
+  DevBuf<unsigned long long> acc;
+  DevBuf<double> scale;
+  Rdm2Acc R;
+  SQ_CHECK(rdm2_accumulate(h, "two_rdm", n, dets_up, dets_dn, S, wts, ldw, marks, acc, scale, R, nullptr));
+  const int64_t n4 = (int64_t)norb * norb * norb * norb;
   DevBuf<double> out;
   SQ_CHECK(out.alloc(3 * S * n4));
   rdm2_fill_kernel<<<(unsigned)std::min<int64_t>(div_up(3 * S * n4, 256), 64 * G.sm_count), 256, 0, s>>>(R, scale.p + S, out.p);
@@ -688,17 +720,297 @@ static int two_rdm_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, con
   return 0;
 }
 
-int two_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw, double *rdm) {
-  if (n <= 0) { set_error("two_rdm: n must be positive"); return 2; }
-  if (n_states < 1) { set_error("two_rdm: n_states must be >= 1"); return 2; }
-  if (ldw < n) { set_error("two_rdm: ldw (%lld) must be >= n (%lld)", (long long)ldw, (long long)n); return 2; }
-  if (n > INT32_MAX) { set_error("two_rdm: n exceeds the 32-bit row index"); return 2; }
+// argument checks both two-particle entry points share
+static int rdm2_check_args(sqmc_b200_handle *h, const char *who, int64_t n, int n_states, int64_t ldw) {
+  if (n <= 0) { set_error("%s: n must be positive", who); return 2; }
+  if (n_states < 1) { set_error("%s: n_states must be >= 1", who); return 2; }
+  if (ldw < n) { set_error("%s: ldw (%lld) must be >= n (%lld)", who, (long long)ldw, (long long)n); return 2; }
+  if (n > INT32_MAX) { set_error("%s: n exceeds the 32-bit row index", who); return 2; }
   if (h->T.norb > 64) {
-    set_error("two_rdm: norb = %d > 64 is not supported (the dense output holds 3*norb^4 doubles per state, and strings of more than one word are not handled)",
-              h->T.norb);
+    set_error("%s: norb = %d > 64 is not supported (the dense output holds 3*norb^4 doubles per state, and strings of more than one word are not handled)",
+              who, h->T.norb);
     return 2;
   }
+  return 0;
+}
+
+int two_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw, double *rdm) {
+  SQ_CHECK(rdm2_check_args(h, "two_rdm", n, n_states, ldw));
   return two_rdm_impl(h, n, dets_up, dets_dn, n_states, wts, ldw, rdm);
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// orbital gradient and Hessian of the variational energy (sqmc_b200_orbital_derivatives), chem, norb <= 64
+//
+// Helgaker, Jorgensen, Olsen, Molecular Electronic-Structure Theory, 10.8.1 (real orbitals, kappa = sum_{p>q} k_pq E-_pq):
+//   D_pq   = sum_k w_k (gamma^a + gamma^b)_pq / ||Psi_k||^2,   d_pqrs = sum_k w_k (G^aa + G^bb + G^ab_pq,rs + G^ab_rs,pq) / ||Psi_k||^2
+//   F_pq   = sum_m D_pm h_qm + sum_mnt d_pmnt g_qmnt                                 (gradient 2 (F_pq - F_qp))
+//   Y_pqrs = sum_mn [(d_pmrn + d_pmnr) g_qmsn + d_prmn g_qsmn]
+//   E2_pq,rs = (1 - P_pq)(1 - P_rs) [2 D_pr h_qs - (F_pr + F_rp) delta_qs + 2 Y_pqrs]
+// d is filled from the two_rdm representatives and never leaves the device; D is its partial trace sum_r d_pqrr / (N - 1).
+// F and Y are both products C = A B^T of column-major matrices in FP64 (orb_gemm_kernel): F with A = [D | d] (norb x
+// (norb + norb^3)) and B = [h | g]; Y with rows (p + norb r), columns (q + norb s) and A = [X | d], B = [G | g] over
+// (m + norb n), X = d_pmrn + d_pmnr, G = g_qmsn (the d_prmn g_qsmn term reads d and g as they are stored).  Every output is
+// summed by one thread in k order, and split-K partials are added in a fixed order: no atomics anywhere.
+
+// d (p,q,r,s at p + norb (q + norb (r + norb s))) from the representatives, spin summed and state averaged; f[k] = w_k / ||Psi_k||^2
+__global__ void orbd_fill_kernel(Rdm2Acc R, const double *unscale, const double *state_w, const double *norm2, double *d) {
+  const int norb = R.norb;
+  const int64_t n4 = (int64_t)norb * norb * norb * norb;
+  for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < n4; t += (int64_t)gridDim.x * blockDim.x) {
+    int64_t x = t;
+    const int p = (int)(x % norb); x /= norb;
+    const int q = (int)(x % norb); x /= norb;
+    const int r = (int)(x % norb);
+    const int s = (int)(x / norb);
+    double v = 0.0;
+    for (int k = 0; k < R.S; k++) {
+      const unsigned long long *a = R.a + 2 * (int64_t)k * R.per;
+      auto val = [&](int64_t slot) { return (ldexp((double)(long long)a[2 * slot + 1], 64) + (double)a[2 * slot]) * unscale[k]; };
+      double e = val(R.off_ab + ab_slot(p, q, r, s, norb)) + val(R.off_ab + ab_slot(r, s, p, q, norb));
+      if (p != r && q != s) {
+        int sg;
+        const int64_t slot = ss_slot(p, q, r, s, R.M, sg);
+        const double ss = val(slot) + val(R.off_bb + slot);
+        e += sg < 0 ? -ss : ss;
+      }
+      v += (state_w[k] / norm2[k]) * e;
+    }
+    d[t] = v;
+  }
+}
+
+// D_pq = sum_r d_pqrr / (N - 1), r in order
+__global__ void orbd_trace_kernel(const double *d, int norb, double inv_nm1, double *D) {
+  const int t = blockIdx.x * blockDim.x + threadIdx.x;
+  const int nn = norb * norb;
+  if (t >= nn) return;
+  double a = 0.0;
+  for (int r = 0; r < norb; r++) a += d[t + (int64_t)nn * (r + (int64_t)norb * r)];
+  D[t] = a * inv_nm1;
+}
+
+// dense h (p + norb q) and g (p + norb (q + norb (r + norb s))) from the handle's integral table, as ChemCtx::I reads it
+__global__ void orbd_integrals_kernel(const double *ints, const int32_t *c2, int norb, double *hd, double *gd) {
+  const int n1 = norb + 1;
+  const int64_t nn = (int64_t)norb * norb, n4 = nn * nn;
+  const long long core = c2[norb * n1 + norb];
+  for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < n4 + nn; t += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t u = t < n4 ? t : t - n4;
+    const long long a = c2[(u / norb % norb) * n1 + u % norb];
+    const long long b = t < n4 ? c2[(u / nn / norb) * n1 + u / nn % norb] : core;
+    const long long idx = a > b ? a * (a - 1) / 2 + b : b * (b - 1) / 2 + a;
+    (t < n4 ? gd : hd)[u] = ints[idx - 1];
+  }
+}
+
+// X[(p + norb r) + norb^2 (m + norb n)] = d_pmrn + d_pmnr and G[(q + norb s) + norb^2 (m + norb n)] = g_qmsn
+__global__ void orbd_y_operands_kernel(const double *d, const double *g, int norb, double *X, double *Gq) {
+  const int64_t nn = (int64_t)norb * norb, n4 = nn * nn;
+  for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < n4; t += (int64_t)gridDim.x * blockDim.x) {
+    int64_t x = t;
+    const int64_t p = x % norb; x /= norb;
+    const int64_t r = x % norb; x /= norb;
+    const int64_t m = x % norb;
+    const int64_t n = x / norb;
+    X[t] = d[p + norb * (m + norb * (r + norb * n))] + d[p + norb * (m + norb * (n + norb * r))];
+    Gq[t] = g[p + norb * (m + norb * (r + norb * n))];
+  }
+}
+
+static const int kGemmTile = 64, kGemmK = 16, kGemmThreads = 256;
+struct GemmSeg {  // A(i, k) = a[i + M k], B(j, k) = b[j + N k] for k < K
+  const double *a, *b;
+  int64_t K;
+};
+
+// part[z][i + M j] = sum over the k of chunk z of A(i,k) B(j,k), k running over segment 0 then segment 1.  64 x 64 tile per
+// block, 4 x 4 outputs per thread (rows tx + 16 x, columns ty + 16 y), 16-deep k slices staged in shared memory.
+__global__ void __launch_bounds__(kGemmThreads) orb_gemm_kernel(GemmSeg s0, GemmSeg s1, int M, int N, int64_t kchunk, double *part) {
+  __shared__ double As[kGemmK][kGemmTile], Bs[kGemmK][kGemmTile];
+  const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
+  const int i0 = blockIdx.x * kGemmTile, j0 = blockIdx.y * kGemmTile;
+  const int64_t K = s0.K + s1.K;
+  const int64_t kb = blockIdx.z * kchunk, ke = min(K, kb + kchunk);
+  double acc[4][4];
+#pragma unroll
+  for (int x = 0; x < 4; x++)
+#pragma unroll
+    for (int y = 0; y < 4; y++) acc[x][y] = 0.0;
+  for (int64_t k0 = kb; k0 < ke; k0 += kGemmK) {
+#pragma unroll
+    for (int e = threadIdx.x; e < kGemmK * kGemmTile; e += kGemmThreads) {
+      const int kk = e / kGemmTile, ii = e % kGemmTile;
+      const int64_t k = k0 + kk;
+      double av = 0.0, bv = 0.0;
+      if (k < ke) {
+        const bool first = k < s0.K;
+        const int64_t kl = first ? k : k - s0.K;
+        if (i0 + ii < M) av = (first ? s0.a : s1.a)[i0 + ii + (int64_t)M * kl];
+        if (j0 + ii < N) bv = (first ? s0.b : s1.b)[j0 + ii + (int64_t)N * kl];
+      }
+      As[kk][ii] = av;
+      Bs[kk][ii] = bv;
+    }
+    __syncthreads();
+#pragma unroll
+    for (int kk = 0; kk < kGemmK; kk++) {
+      double a[4], b[4];
+#pragma unroll
+      for (int x = 0; x < 4; x++) a[x] = As[kk][tx + 16 * x];
+#pragma unroll
+      for (int y = 0; y < 4; y++) b[y] = Bs[kk][ty + 16 * y];
+#pragma unroll
+      for (int x = 0; x < 4; x++)
+#pragma unroll
+        for (int y = 0; y < 4; y++) acc[x][y] = fma(a[x], b[y], acc[x][y]);
+    }
+    __syncthreads();
+  }
+  double *c = part + (int64_t)blockIdx.z * M * N;
+#pragma unroll
+  for (int x = 0; x < 4; x++)
+#pragma unroll
+    for (int y = 0; y < 4; y++) {
+      const int i = i0 + tx + 16 * x, j = j0 + ty + 16 * y;
+      if (i < M && j < N) c[i + (int64_t)M * j] = acc[x][y];
+    }
+}
+
+// out[t] = sum_z part[z][t], z in order
+__global__ void orb_splitk_reduce_kernel(const double *part, int64_t mn, int nz, double *out) {
+  for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < mn; t += (int64_t)gridDim.x * blockDim.x) {
+    double a = 0.0;
+    for (int z = 0; z < nz; z++) a += part[z * mn + t];
+    out[t] = a;
+  }
+}
+
+// C = A B^T (M x N, column-major) over the two segments; split-K when the output has too few tiles to fill the GPU
+static int orb_gemm(GemmSeg s0, GemmSeg s1, int M, int N, double *C, cudaStream_t s) {
+  const int64_t K = s0.K + s1.K;
+  const int64_t tiles = div_up(M, kGemmTile) * div_up(N, kGemmTile);
+  const int64_t kslices = div_up(K, kGemmK);
+  const int nz = (int)std::max<int64_t>(1, std::min<int64_t>(kslices, div_up(2 * G.sm_count, tiles)));
+  const int64_t kchunk = div_up(kslices, nz) * kGemmK;
+  const int nzu = (int)div_up(K, kchunk);
+  DevBuf<double> part;
+  if (nzu > 1) SQ_CHECK(part.alloc((int64_t)nzu * M * N));
+  dim3 grid((unsigned)div_up(M, kGemmTile), (unsigned)div_up(N, kGemmTile), (unsigned)nzu);
+  orb_gemm_kernel<<<grid, kGemmThreads, 0, s>>>(s0, s1, M, N, kchunk, nzu > 1 ? part.p : C);
+  SQ_LAUNCH_CHECK();
+  if (nzu > 1) {
+    const int64_t mn = (int64_t)M * N;
+    orb_splitk_reduce_kernel<<<(unsigned)std::min<int64_t>(div_up(mn, 256), 8 * G.sm_count), 256, 0, s>>>(part.p, mn, nzu, C);
+    SQ_LAUNCH_CHECK();
+  }
+  return 0;
+}
+
+// E2 from D, h, F and Y (Y[(p + norb r) + norb^2 (q + norb s)]); the four permuted terms added in a fixed order
+__global__ void orbd_hessian_kernel(const double *D, const double *hd, const double *F, const double *Y, int norb, double *E2) {
+  const int64_t nn = (int64_t)norb * norb, n4 = nn * nn;
+  for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < n4; t += (int64_t)gridDim.x * blockDim.x) {
+    int64_t x = t;
+    const int p = (int)(x % norb); x /= norb;
+    const int q = (int)(x % norb); x /= norb;
+    const int r = (int)(x % norb);
+    const int s = (int)(x / norb);
+    auto f = [&](int a, int b, int c, int e) {
+      double v = 2.0 * D[a + (int64_t)norb * c] * hd[b + (int64_t)norb * e];
+      if (b == e) v -= F[a + (int64_t)norb * c] + F[c + (int64_t)norb * a];
+      return v + 2.0 * Y[(a + (int64_t)norb * c) + nn * (b + (int64_t)norb * e)];
+    };
+    E2[t] = ((f(p, q, r, s) - f(q, p, r, s)) - f(p, q, s, r)) + f(q, p, s, r);
+  }
+}
+
+// energy = E_core + 1/2 (sum_pq h_pq D_pq + sum_p F_pp), one block, fixed order
+__global__ void __launch_bounds__(256) orbd_energy_kernel(const double *D, const double *hd, const double *F, int norb, double ecore, double *e) {
+  __shared__ double red[256];
+  const int nn = norb * norb;
+  double a = 0.0;
+  for (int t = threadIdx.x; t < nn; t += 256) a += hd[t] * D[t];
+  for (int p = threadIdx.x; p < norb; p += 256) a += F[p + norb * p];
+  red[threadIdx.x] = a;
+  __syncthreads();
+  for (int hh = 128; hh > 0; hh >>= 1) {
+    if (threadIdx.x < hh) red[threadIdx.x] += red[threadIdx.x + hh];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) *e = ecore + 0.5 * red[0];
+}
+
+static int orbital_derivatives_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int S, const double *wts,
+                                    int64_t ldw, const double *state_weights, double *fock, double *hessian, double *energy) {
+  cudaStream_t s = G.stream;
+  const ModelTables &T = h->T;
+  const int norb = T.norb;
+  const int64_t nn = (int64_t)norb * norb, n4 = nn * nn;
+  HostMarks marks("SQMC_ORBD_PROFILE", "orbital_derivatives");  // =1: phase split (synchronising) on stderr
+  DevBuf<double> norm2, sw;
+  SQ_CHECK(norm2.alloc(S));
+  SQ_CHECK(sw.alloc(S));
+  SQ_CUDA(cudaMemcpyAsync(sw.p, state_weights, S * sizeof(double), cudaMemcpyHostToDevice, s));
+  DevBuf<double> d, D;
+  {
+    DevBuf<unsigned long long> acc;
+    DevBuf<double> scale;
+    Rdm2Acc R;
+    SQ_CHECK(rdm2_accumulate(h, "orbital_derivatives", n, dets_up, dets_dn, S, wts, ldw, marks, acc, scale, R, norm2.p));
+    SQ_CHECK(d.alloc(n4));
+    orbd_fill_kernel<<<(unsigned)std::min<int64_t>(div_up(n4, 256), 64 * G.sm_count), 256, 0, s>>>(R, scale.p + S, sw.p, norm2.p, d.p);
+    SQ_LAUNCH_CHECK();
+  }
+  SQ_CHECK(D.alloc(nn));
+  orbd_trace_kernel<<<(unsigned)div_up(nn, 256), 256, 0, s>>>(d.p, norb, 1.0 / (T.nup + T.ndn - 1), D.p);
+  SQ_LAUNCH_CHECK();
+  DevBuf<double> hd, gd;
+  SQ_CHECK(hd.alloc(nn));
+  SQ_CHECK(gd.alloc(n4));
+  orbd_integrals_kernel<<<(unsigned)std::min<int64_t>(div_up(n4 + nn, 256), 64 * G.sm_count), 256, 0, s>>>(T.integrals, T.combine_2, norb, hd.p, gd.p);
+  SQ_LAUNCH_CHECK();
+  marks.mark("d, D, dense integrals");
+  DevBuf<double> F, X, Gq, Y, E2, e;
+  SQ_CHECK(F.alloc(nn));
+  SQ_CHECK(orb_gemm(GemmSeg{D.p, hd.p, norb}, GemmSeg{d.p, gd.p, nn * norb}, norb, norb, F.p, s));
+  SQ_CHECK(X.alloc(n4));
+  SQ_CHECK(Gq.alloc(n4));
+  orbd_y_operands_kernel<<<(unsigned)std::min<int64_t>(div_up(n4, 256), 64 * G.sm_count), 256, 0, s>>>(d.p, gd.p, norb, X.p, Gq.p);
+  SQ_LAUNCH_CHECK();
+  SQ_CHECK(Y.alloc(n4));
+  SQ_CHECK(orb_gemm(GemmSeg{X.p, Gq.p, nn}, GemmSeg{d.p, gd.p, nn}, (int)nn, (int)nn, Y.p, s));
+  X.release(); Gq.release(); d.release(); gd.release();
+  SQ_CHECK(E2.alloc(n4));
+  orbd_hessian_kernel<<<(unsigned)std::min<int64_t>(div_up(n4, 256), 64 * G.sm_count), 256, 0, s>>>(D.p, hd.p, F.p, Y.p, norb, E2.p);
+  SQ_LAUNCH_CHECK();
+  SQ_CHECK(e.alloc(1));
+  orbd_energy_kernel<<<1, 256, 0, s>>>(D.p, hd.p, F.p, norb, T.enuc, e.p);  // T.enuc: table entry _index(n1, n1, n1, n1)
+  SQ_LAUNCH_CHECK();
+  marks.mark("contractions");
+  SQ_CUDA(cudaMemcpyAsync(fock, F.p, nn * sizeof(double), cudaMemcpyDeviceToHost, s));
+  SQ_CUDA(cudaMemcpyAsync(hessian, E2.p, n4 * sizeof(double), cudaMemcpyDeviceToHost, s));
+  SQ_CUDA(cudaMemcpyAsync(energy, e.p, sizeof(double), cudaMemcpyDeviceToHost, s));
+  SQ_CUDA(cudaStreamSynchronize(s));
+  marks.mark("copy out");
+  return 0;
+}
+
+int orbital_derivatives(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw,
+                        const double *state_weights, double *fock, double *hessian, double *energy) {
+  if (h->T.model != MODEL_CHEM) {
+    set_error("orbital_derivatives: only chem handles have orbitals to optimise (heg and hubbardk orbitals are fixed by momentum)");
+    return 2;
+  }
+  SQ_CHECK(rdm2_check_args(h, "orbital_derivatives", n, n_states, ldw));
+  if (h->T.nup + h->T.ndn < 2) { set_error("orbital_derivatives: needs at least two electrons"); return 2; }
+  double sum = 0.0;
+  for (int k = 0; k < n_states; k++) {
+    if (!(state_weights[k] >= 0.0)) { set_error("orbital_derivatives: state_weights[%d] = %g is negative", k, state_weights[k]); return 2; }
+    sum += state_weights[k];
+  }
+  if (!(fabs(sum - 1.0) <= 1e-12)) { set_error("orbital_derivatives: state_weights sum to %.17g, not 1", sum); return 2; }
+  return orbital_derivatives_impl(h, n, dets_up, dets_dn, n_states, wts, ldw, state_weights, fock, hessian, energy);
 }
 
 }  // namespace sqmc
