@@ -154,6 +154,29 @@ int sqmc_b200_orbital_derivatives(sqmc_b200_handle *h, int64_t n, const void *de
                                   const double *wts, int64_t ldw, const double *state_weights,
                                   double *fock, double *hessian, double *energy);
 
+/* ---- sigma-vector over a determinant list (orbital optimisation) ----------------------------------------------------
+ * y = H x (kappa == NULL: the handle's own integrals, core energy included) or y = H^kappa x (kappa != NULL: the Hamiltonian
+ * with one-index-transformed integrals h^k = kappa h - h kappa, g^k_pqrs = sum_m (k_pm g_mqrs + k_qm g_pmrs + k_rm g_pqms +
+ * k_sm g_pqrm), no core term), i.e. d/dt H(U(t)) at t = 0 for U(t) = expm(-t kappa) with rotate_fcidump's rule.
+ * kappa: norb^2 doubles, antisymmetric, kappa_pq at p + norb*q in the library's orbital numbering.  x: n_states columns of
+ * leading dimension ldx; y: n x n_states, column-major with leading dimension n, in the caller's row order.
+ * No built matrix is needed or used: every pair of the list connected by a single or double excitation is visited, whatever
+ * its matrix element.  Arguments, orbital numbering, time_sym handling (x and y over the representatives) and errors are
+ * those of sqmc_b200_orbital_derivatives without state weights.  y is summed as 128-bit fixed-point integers, so it is
+ * bit-identical across calls and row permutations. */
+int sqmc_b200_sigma(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states,
+                    const double *x, int64_t ldx, const double *kappa, double *y);
+
+/* ---- orbital-gradient response (orbital optimisation) ---------------------------------------------------------------
+ * response (norb^2 doubles, (p,q) at p + norb*q, antisymmetric) = d/dt at t = 0 of the gradient 2 (F - F^T) that
+ * sqmc_b200_orbital_derivatives returns for the vectors wts + t dwts (both n_states columns of leading dimension ldw),
+ * normalisation term included.  It is 2 (F' - F'^T) with F' built from the symmetrised transition densities of (c_k, dc_k');
+ * the O(norb^6) Hessian product is not formed.  Arguments and errors are those of sqmc_b200_orbital_derivatives; the result is
+ * bit-identical across calls and row permutations. */
+int sqmc_b200_orbital_gradient_response(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states,
+                                        const double *wts, const double *dwts, int64_t ldw, const double *state_weights,
+                                        double *response);
+
 /* ---- sparse H build --------------------------------------------------------
  * Replaces generate_sparse_ham_chem_upper_triangular (chemistry.f90:7639),
  * its _mpi twin (:8012), generate_sparse_ham_heg_upper_triangular

@@ -364,6 +364,54 @@ class SparseHamiltonian:
         fock = np.ascontiguousarray(fock.T)
         return dict(fock=fock, gradient=2.0 * (fock - fock.T), hessian=np.ascontiguousarray(hess.transpose(3, 2, 1, 0)), energy=float(e[0]))
 
+    def sigma(self, dets_up, dets_dn, x, kappa=None):
+        """y = H x over the determinant list (any order, no built matrix needed or used; on time_sym systems the representatives),
+        x (n,) or (n, n_states), y of the same shape in the caller's row order; chem only, norb <= 64.
+        kappa None: the handle's own integrals, core energy included.  kappa (norb, norb) antisymmetric, kappa[p, q] = k_pq in the
+        library's orbital numbering (the convention of orbital_derivatives): y = H^kappa x, H^kappa = d/dt H(U(t)) at t = 0 for
+        U(t) = expm(-t kappa) with natorb.rotate_fcidump's rule (h^k = kappa h - h kappa, g^k one-index transformed on each
+        index), no core term.  Every pair connected by a single or double excitation counts, whatever its matrix element."""
+        up = np.ascontiguousarray(dets_up, dtype=np.uint64).reshape(-1, 2)
+        dn = np.ascontiguousarray(dets_dn, dtype=np.uint64).reshape(-1, 2)
+        v = np.asarray(x, dtype=np.float64)
+        one = v.ndim == 1
+        v = np.asfortranarray(v.reshape(-1, 1) if one else v)
+        if len(dn) != len(up) or v.shape[0] != len(up):
+            raise ValueError("sigma: dets_up, dets_dn and x must have the same number of rows")
+        norb = self.system.norb
+        k = None
+        if kappa is not None:
+            k = np.asarray(kappa, dtype=np.float64)
+            if k.shape != (norb, norb):
+                raise ValueError("sigma: kappa must have shape (%d, %d)" % (norb, norb))
+            k = np.asfortranarray(k)   # kappa_pq at p + norb*q
+        y = np.zeros(v.shape, order="F")
+        check(self._L.sqmc_b200_sigma(self._h, len(up), _p(up), _p(dn), v.shape[1], _p(v), max(v.shape[0], 1), _p(k), _p(y)))
+        return y[:, 0].copy() if one else np.ascontiguousarray(y)
+
+    def orbital_gradient_response(self, dets_up, dets_dn, wts, dwts, state_weights=None):
+        """d/dt at t = 0 of orbital_derivatives(dets_up, dets_dn, wts + t dwts, state_weights)["gradient"], the normalisation of
+        every state included: the (norb, norb) antisymmetric response of the orbital gradient to a change of the CI vectors.
+        Arguments, orbital numbering and errors are those of orbital_derivatives; dwts has the shape of wts."""
+        up = np.ascontiguousarray(dets_up, dtype=np.uint64).reshape(-1, 2)
+        dn = np.ascontiguousarray(dets_dn, dtype=np.uint64).reshape(-1, 2)
+        w = np.asarray(wts, dtype=np.float64)
+        dw = np.asarray(dwts, dtype=np.float64)
+        if dw.shape != w.shape:
+            raise ValueError("orbital_gradient_response: dwts has shape %s, wts %s" % (dw.shape, w.shape))
+        w = np.asfortranarray(w.reshape(-1, 1) if w.ndim == 1 else w)
+        dw = np.asfortranarray(dw.reshape(w.shape))
+        if len(dn) != len(up) or w.shape[0] != len(up):
+            raise ValueError("orbital_gradient_response: dets_up, dets_dn and wts must have the same number of rows")
+        norb, ns = self.system.norb, w.shape[1]
+        sw = np.full(max(ns, 1), 1.0 / max(ns, 1)) if state_weights is None else np.ascontiguousarray(state_weights, dtype=np.float64).reshape(-1)
+        if len(sw) != ns:
+            raise ValueError("orbital_gradient_response: state_weights holds %d values for %d states" % (len(sw), ns))
+        out = np.zeros((norb, norb) if norb <= 64 else 1)   # the library rejects norb > 64
+        check(self._L.sqmc_b200_orbital_gradient_response(self._h, len(up), _p(up), _p(dn), ns, _p(w), _p(dw), max(w.shape[0], 1), _p(sw),
+                                                          _p(out)))
+        return np.ascontiguousarray(out.T)   # (p,q) at p + norb*q
+
     def second_order_pt(self, dets_up, dets_dn, wts, var_energy, eps_pt):
         """Deterministic second-order PT with the HCI screened sum (second_order_pt, hci.f90:1100-1182) -> (delta_e_2pt, ndets_connected)."""
         up = np.ascontiguousarray(dets_up, dtype=np.uint64).reshape(-1, 2)

@@ -468,6 +468,23 @@ int sqmc_b200_orbital_derivatives(sqmc_b200_handle *h, int64_t n, const void *de
   return orbital_derivatives(h, n, dets_up, dets_dn, n_states, wts, ldw, state_weights, fock, hessian, energy);
 }
 
+int sqmc_b200_sigma(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *x, int64_t ldx,
+                    const double *kappa, double *y) {
+  SQ_CHECK(require_init());
+  if (!h || !dets_up || !dets_dn || !x || !y) { set_error("sigma: null argument"); return 2; }
+  return sigma(h, n, dets_up, dets_dn, n_states, x, ldx, kappa, y);
+}
+
+int sqmc_b200_orbital_gradient_response(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts,
+                                        const double *dwts, int64_t ldw, const double *state_weights, double *response) {
+  SQ_CHECK(require_init());
+  if (!h || !dets_up || !dets_dn || !wts || !dwts || !state_weights || !response) {
+    set_error("orbital_gradient_response: null argument");
+    return 2;
+  }
+  return orbital_gradient_response(h, n, dets_up, dets_dn, n_states, wts, dwts, ldw, state_weights, response);
+}
+
 int sqmc_b200_pt2(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, const double *wts, double var_energy, double eps_pt,
                   double *delta_e, int64_t *n_connected) {
   SQ_CHECK(require_init());

@@ -281,4 +281,8 @@ int one_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *det
 int two_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw, double *rdm2);
 int orbital_derivatives(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw,
                         const double *state_weights, double *fock, double *hessian, double *energy);
+int sigma(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *x, int64_t ldx,
+          const double *kappa, double *y);
+int orbital_gradient_response(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts,
+                              const double *dwts, int64_t ldw, const double *state_weights, double *response);
 }  // namespace sqmc

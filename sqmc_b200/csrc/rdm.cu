@@ -21,6 +21,7 @@
 #include <thrust/iterator/counting_iterator.h>
 
 #include <cub/cub.cuh>
+#include <cstring>
 #include <vector>
 
 #include "handle.h"
@@ -249,10 +250,11 @@ static int make_view(int norb, const uint64_t *major, const uint64_t *minor, con
 
 // The part both density matrices share: upload, the time_sym expansion to n2 plain determinants (up, dn, w column-major
 // n2 x S), and view 0 (sorted by (up, dn): idx0, ma0 = up, mi0 = dn, c0 interleaved) with the duplicate and partner check.
+// sel_out (time_sym, optional): the representatives whose partner (d,u) is expanded entry n + j, j < n2 - n.
 template <int NW>
 static int prepare_dets(sqmc_b200_handle *h, const char *who, int64_t n, const void *dets_up, const void *dets_dn, int S, const double *wts,
                         int64_t ldw, DevBuf<uint64_t> &up, DevBuf<uint64_t> &dn, DevBuf<double> &w, int64_t &n2, DevBuf<int32_t> &idx0,
-                        DevBuf<uint64_t> &ma0, DevBuf<uint64_t> &mi0, DevBuf<double> &c0) {
+                        DevBuf<uint64_t> &ma0, DevBuf<uint64_t> &mi0, DevBuf<double> &c0, DevBuf<int32_t> *sel_out = nullptr) {
   cudaStream_t s = G.stream;
   const ModelTables &T = h->T;
   const int norb = T.norb;
@@ -292,6 +294,11 @@ static int prepare_dets(sqmc_b200_handle *h, const char *who, int64_t n, const v
     SQ_LAUNCH_CHECK();
     up.release(); dn.release(); w.release();
     up.p = eu.take(); dn.p = ed.take(); w.p = ew.take();
+    if (sel_out) {
+      sel_out->release();
+      sel_out->n = sel.n;
+      sel_out->p = sel.take();
+    }
     up.n = dn.n = n2 * NW;
     w.n = n2 * S;
   }
@@ -434,6 +441,7 @@ struct Rdm2Acc {
   const double *scale;    // [S] 2^(120 - e_k)
   int64_t per, off_bb, off_ab;
   int M, norb, S;
+  int cs;                 // coefficients per row: S, or 2S in the two-vector mode (a_k at k, b_k at S + k)
 };
 
 __global__ void electron_count_kernel(const uint64_t *u, const uint64_t *d, int64_t n, int nup, int ndn, int *bad) {
@@ -476,54 +484,66 @@ __global__ void rdm2_keys_ab_kernel(const uint64_t *u, const uint64_t *d, int64_
   }
 }
 
-// one thread per sorted entry i: every later entry j of the same bucket; boff: block offset of a same-spin class, -1: alpha beta
+// The representative slot of the pair (i, j) of one bucket (entries ki / kdi / ai / bi of i and aj / bj of j) and the sign f
+// of <i| operator |j> on it; boff: block offset of a same-spin class, -1: alpha beta
+__device__ __forceinline__ int64_t rdm2_pair_slot(uint64_t ki, uint64_t kdi, int ai, int bi, int aj, int bj, int64_t boff, int M, int norb,
+                                                  int64_t off_ab, double &f) {
+  int neg, sg = 1;
+  int64_t slot;
+  if (boff >= 0) {
+    int p, q, r, s;
+    if (ai != aj && ai != bj && bi != aj && bi != bj) {  // double: <i| a+_ai a+_bi a_bj a_aj |j> = <i| a+_ai a_aj a+_bi a_bj |j>
+      const uint64_t uj = ki | 1ull << aj | 1ull << bj;
+      neg = par_between(uj, bi, bj) ^ par_between(uj ^ (1ull << bj) ^ (1ull << bi), ai, aj);
+      p = ai; q = aj; r = bi; s = bj;
+    } else {  // single x_j -> x_i; the shared removed orbital r stays occupied in both
+      const int r0 = (ai == aj || ai == bj) ? ai : bi;
+      const int xi = ai == r0 ? bi : ai, xj = aj == r0 ? bj : aj;
+      neg = par_between(ki | 1ull << r0, xi, xj);
+      p = xi; q = xj; r = r0; s = r0;
+    }
+    slot = boff + ss_slot(p, q, r, s, M, sg);
+  } else if (ai != aj && bi != bj) {
+    neg = par_between(ki, ai, aj) ^ par_between(kdi, bi, bj);
+    slot = off_ab + ab_slot(ai, aj, bi, bj, norb);
+  } else if (ai != aj) {
+    neg = par_between(ki, ai, aj);
+    slot = off_ab + ab_slot(ai, aj, bi, bi, norb);
+  } else {
+    neg = par_between(kdi, bi, bj);
+    slot = off_ab + ab_slot(ai, ai, bi, bj, norb);
+  }
+  f = (neg ? -1.0 : 1.0) * sg;
+  return slot;
+}
+
+// one thread per sorted entry i: every later entry j of the same bucket; boff: block offset of a same-spin class, -1: alpha beta.
+// TWO = false: the term f c_i c_j of each state; TWO = true: the symmetrised transition term f (a_i b_j + b_i a_j) / 2.
+template <bool TWO>
 __global__ void __launch_bounds__(256) rdm2_pair_kernel(const uint64_t *ku, const uint64_t *kd, const uint64_t *pay, int64_t m, int64_t boff,
                                                         const double *coef, Rdm2Acc R) {
   const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (i >= m) return;
   const uint64_t ki = ku[i], kdi = kd[i], pi = pay[i];
   const int ai = (int)(pi & 0xff), bi = (int)((pi >> 8) & 0xff);
-  const double *ci = coef + (int64_t)(pi >> 16) * R.S;
+  const double *ci = coef + (int64_t)(pi >> 16) * R.cs;
   for (int64_t j = i + 1; j < m && ku[j] == ki && kd[j] == kdi; j++) {
     const uint64_t pj = pay[j];
-    const int aj = (int)(pj & 0xff), bj = (int)((pj >> 8) & 0xff);
-    int neg, sg = 1;
-    int64_t slot;
-    if (boff >= 0) {
-      int p, q, r, s;
-      if (ai != aj && ai != bj && bi != aj && bi != bj) {  // double: <i| a+_ai a+_bi a_bj a_aj |j> = <i| a+_ai a_aj a+_bi a_bj |j>
-        const uint64_t uj = ki | 1ull << aj | 1ull << bj;
-        neg = par_between(uj, bi, bj) ^ par_between(uj ^ (1ull << bj) ^ (1ull << bi), ai, aj);
-        p = ai; q = aj; r = bi; s = bj;
-      } else {  // single x_j -> x_i; the shared removed orbital r stays occupied in both
-        const int r0 = (ai == aj || ai == bj) ? ai : bi;
-        const int xi = ai == r0 ? bi : ai, xj = aj == r0 ? bj : aj;
-        neg = par_between(ki | 1ull << r0, xi, xj);
-        p = xi; q = xj; r = r0; s = r0;
-      }
-      slot = boff + ss_slot(p, q, r, s, R.M, sg);
-    } else if (ai != aj && bi != bj) {
-      neg = par_between(ki, ai, aj) ^ par_between(kdi, bi, bj);
-      slot = R.off_ab + ab_slot(ai, aj, bi, bj, R.norb);
-    } else if (ai != aj) {
-      neg = par_between(ki, ai, aj);
-      slot = R.off_ab + ab_slot(ai, aj, bi, bi, R.norb);
-    } else {
-      neg = par_between(kdi, bi, bj);
-      slot = R.off_ab + ab_slot(ai, ai, bi, bj, R.norb);
-    }
-    const double f = (neg ? -1.0 : 1.0) * sg;
-    const double *cj = coef + (int64_t)(pj >> 16) * R.S;
+    double f;
+    const int64_t slot = rdm2_pair_slot(ki, kdi, ai, bi, (int)(pj & 0xff), (int)((pj >> 8) & 0xff), boff, R.M, R.norb, R.off_ab, f);
+    const double *cj = coef + (int64_t)(pj >> 16) * R.cs;
     for (int k = 0; k < R.S; k++) {
       uint64_t lo, hi;
-      fix_to_i128(f * (ci[k] * cj[k]) * R.scale[k], lo, hi);
+      if constexpr (TWO) fix_to_i128(f * (0.5 * (ci[k] * cj[R.S + k] + ci[R.S + k] * cj[k])) * R.scale[k], lo, hi);
+      else fix_to_i128(f * (ci[k] * cj[k]) * R.scale[k], lo, hi);
       i128_add(R.a + 2 * (k * R.per + slot), lo, hi);
     }
   }
 }
 
-// diagonal terms c_i^2: Gamma^{ss}_{pp,rr} (p < r occupied in the same string) and Gamma^{ab}_{pp,rr}, one state at a time,
-// summed per block in shared memory ([3][norb][norb] 128-bit values) and then added to the representatives
+// diagonal terms c_i^2 (TWO: a_i b_i): Gamma^{ss}_{pp,rr} (p < r occupied in the same string) and Gamma^{ab}_{pp,rr}, one state
+// at a time, summed per block in shared memory ([3][norb][norb] 128-bit values) and then added to the representatives
+template <bool TWO>
 __global__ void __launch_bounds__(256) rdm2_diag_kernel(const uint64_t *u, const uint64_t *d, int64_t n, const double *coef, Rdm2Acc R) {
   extern __shared__ unsigned long long sd[];
   const int norb = R.norb, nn = norb * norb;
@@ -531,9 +551,9 @@ __global__ void __launch_bounds__(256) rdm2_diag_kernel(const uint64_t *u, const
     for (int t = threadIdx.x; t < 6 * nn; t += blockDim.x) sd[t] = 0ull;
     __syncthreads();
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-      const double c = coef[i * R.S + k];
+      const double c = coef[i * R.cs + k];
       uint64_t lo, hi;
-      fix_to_i128((c * c) * R.scale[k], lo, hi);
+      fix_to_i128((TWO ? c * coef[i * R.cs + R.S + k] : c * c) * R.scale[k], lo, hi);
       if ((lo | hi) == 0) continue;
       const uint64_t U = u[i], D = d[i];
       for (uint64_t ps = U; ps; ps &= ps - 1) {
@@ -608,66 +628,65 @@ __global__ void __launch_bounds__(256) norm2_kernel(const double *c, int64_t n, 
   if (threadIdx.x == 0) norm2[k] = red[0];
 }
 
-// The accumulation both two-particle entry points share: upload, time_sym expansion, checks, the diagonal and the three key
-// classes with their pairs.  On return acc / scale hold the representatives of R (scale[S + k]: the factor back to doubles);
-// norm2 (device, S doubles, may be null) receives ||Psi_k||^2 summed in a fixed order.
-static int rdm2_accumulate(sqmc_b200_handle *h, const char *who, int64_t n, const void *dets_up, const void *dets_dn, int S, const double *wts,
-                           int64_t ldw, HostMarks &marks, DevBuf<unsigned long long> &acc, DevBuf<double> &scale, Rdm2Acc &R, double *norm2) {
-  cudaStream_t s = G.stream;
-  const ModelTables &T = h->T;
-  const int norb = T.norb;
-  DevBuf<uint64_t> up, dn, U, D;
-  DevBuf<double> w, c;
-  DevBuf<int32_t> idx0;
-  int64_t n2 = 0;
-  SQ_CHECK(prepare_dets<1>(h, who, n, dets_up, dets_dn, S, wts, ldw, up, dn, w, n2, idx0, U, D, c));
-  up.release(); dn.release(); w.release(); idx0.release();
-  marks.mark("upload, expansion, checks");
-  {
-    DevBuf<int> bad;
-    SQ_CHECK(bad.alloc(1));
-    SQ_CUDA(cudaMemsetAsync(bad.p, 0, sizeof(int), s));
-    electron_count_kernel<<<(unsigned)div_up(n2, 256), 256, 0, s>>>(U.p, D.p, n2, T.nup, T.ndn, bad.p);
-    SQ_LAUNCH_CHECK();
-    int hb = 0;
-    SQ_CUDA(cudaMemcpyAsync(&hb, bad.p, sizeof(int), cudaMemcpyDeviceToHost, s));
-    SQ_CUDA(cudaStreamSynchronize(s));
-    if (hb) { set_error("%s: a determinant does not hold %d alpha and %d beta electrons", who, T.nup, T.ndn); return 2; }
-  }
-  if (norm2) {
-    norm2_kernel<<<S, 256, 0, s>>>(c.p, n2, S, norm2);
-    SQ_LAUNCH_CHECK();
-  }
-  // grid exponent per state from sum_i w_ik^2 (the time_sym expansion keeps it); the margin keeps e_k the same whatever order
-  // the sum was taken in, unless the norm lies within a few ulps of 2^e / (1 + 2^-20)
-  std::vector<double> hs(2 * S);
-  for (int k = 0; k < S; k++) {
-    double n2k = 0.0;
-    for (int64_t i = 0; i < n; i++) n2k += wts[k * ldw + i] * wts[k * ldw + i];
-    int e = 0;
-    if (n2k > 0.0) frexp(n2k * (1.0 + 0x1p-20), &e);
-    hs[k] = ldexp(1.0, kFixBits - e);
-    hs[S + k] = ldexp(1.0, e - kFixBits);
-  }
-  const int M = norb * (norb - 1) / 2;
-  const int64_t n4 = (int64_t)norb * norb * norb * norb;
-  R.M = M; R.norb = norb; R.S = S;
-  R.off_bb = (int64_t)M * M;
-  R.off_ab = 2 * R.off_bb;
-  R.per = R.off_ab + n4;
-  SQ_CHECK(acc.alloc(2 * S * R.per));
-  SQ_CHECK(scale.alloc(2 * S));
-  SQ_CUDA(cudaMemsetAsync(acc.p, 0, (size_t)acc.n * sizeof(unsigned long long), s));
-  SQ_CUDA(cudaMemcpyAsync(scale.p, hs.data(), 2 * S * sizeof(double), cudaMemcpyHostToDevice, s));
-  R.a = acc.p;
-  R.scale = scale.p;
-
-  const size_t dsh = (size_t)6 * norb * norb * sizeof(unsigned long long);
-  SQ_CUDA(cudaFuncSetAttribute(rdm2_diag_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dsh));
-  rdm2_diag_kernel<<<(unsigned)std::min<int64_t>(div_up(n2, 256), 2 * G.sm_count), 256, dsh, s>>>(U.p, D.p, n2, c.p, R);
+// every determinant of the sorted view holds T.nup alpha and T.ndn beta electrons
+static int rdm2_electron_check(const ModelTables &T, const char *who, const uint64_t *U, const uint64_t *D, int64_t n2, cudaStream_t s) {
+  DevBuf<int> bad;
+  SQ_CHECK(bad.alloc(1));
+  SQ_CUDA(cudaMemsetAsync(bad.p, 0, sizeof(int), s));
+  electron_count_kernel<<<(unsigned)div_up(n2, 256), 256, 0, s>>>(U, D, n2, T.nup, T.ndn, bad.p);
   SQ_LAUNCH_CHECK();
-  marks.mark("diagonal");
+  int hb = 0;
+  SQ_CUDA(cudaMemcpyAsync(&hb, bad.p, sizeof(int), cudaMemcpyDeviceToHost, s));
+  SQ_CUDA(cudaStreamSynchronize(s));
+  if (hb) { set_error("%s: a determinant does not hold %d alpha and %d beta electrons", who, T.nup, T.ndn); return 2; }
+  return 0;
+}
 
+// per state k over the sorted view (two-vector layout, 2S coefficients per row): out[k] = sum_i a_ik^2, out[S + k] =
+// sum_i a_ik b_ik; thread t sums rows t, t + 256, ... in order, then a fixed tree
+__global__ void __launch_bounds__(256) dots_kernel(const double *c, int64_t n, int S, double *out) {
+  __shared__ double red[2][256];
+  const int k = blockIdx.x;
+  double aa = 0.0, ab = 0.0;
+  for (int64_t i = threadIdx.x; i < n; i += 256) {
+    const double a = c[i * 2 * S + k];
+    aa += a * a;
+    ab += a * c[i * 2 * S + S + k];
+  }
+  red[0][threadIdx.x] = aa;
+  red[1][threadIdx.x] = ab;
+  __syncthreads();
+  for (int hh = 128; hh > 0; hh >>= 1) {
+    if (threadIdx.x < hh) {
+      red[0][threadIdx.x] += red[0][threadIdx.x + hh];
+      red[1][threadIdx.x] += red[1][threadIdx.x + hh];
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) {
+    out[k] = red[0][0];
+    out[S + k] = red[1][0];
+  }
+}
+
+// b_k -= (<a_k|b_k> / ||a_k||^2) a_k: the change of a_k along itself only rescales it and leaves the normalised densities alone
+__global__ void project_out_kernel(double *c, int64_t n, int S, const double *dots) {
+  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (t >= n * S) return;
+  const int64_t i = t / S;
+  const int k = (int)(t % S);
+  const double aa = dots[k];
+  if (aa > 0.0) c[i * 2 * S + S + k] -= (dots[S + k] / aa) * c[i * 2 * S + k];
+}
+
+// The pair enumeration the two-particle entry points share: the three hole-key classes of the sorted view (U, D: n2 one-word
+// strings), each sorted by key; visit(sku, skd, spay, m, boff) is called once per class with the sorted keys and payloads
+// (boff: block offset of a same-spin class, -1: alpha beta).
+template <class Visit>
+static int rdm2_for_each_class(const ModelTables &T, const char *who, const uint64_t *U, const uint64_t *D, int64_t n2, const Rdm2Acc &R,
+                               HostMarks &marks, Visit visit) {
+  cudaStream_t s = G.stream;
+  const int norb = T.norb;
   // class 0: alpha holes (block 0), 1: beta holes (block 2), 2: one hole of each spin (block 1)
   for (int cls = 0; cls < 3; cls++) {
     const int K = cls == 0 ? T.nup * (T.nup - 1) / 2 : cls == 1 ? T.ndn * (T.ndn - 1) / 2 : T.nup * T.ndn;
@@ -679,8 +698,8 @@ static int rdm2_accumulate(sqmc_b200_handle *h, const char *who, int64_t n, cons
     SQ_CHECK(ku.alloc(m));
     SQ_CHECK(kd.alloc(m));
     SQ_CHECK(pay.alloc(m));
-    if (cls == 2) rdm2_keys_ab_kernel<<<(unsigned)div_up(n2, 256), 256, 0, s>>>(U.p, D.p, n2, K, ku.p, kd.p, pay.p);
-    else rdm2_keys_same_kernel<<<(unsigned)div_up(n2, 256), 256, 0, s>>>(cls ? D.p : U.p, cls ? U.p : D.p, n2, K, ku.p, kd.p, pay.p);
+    if (cls == 2) rdm2_keys_ab_kernel<<<(unsigned)div_up(n2, 256), 256, 0, s>>>(U, D, n2, K, ku.p, kd.p, pay.p);
+    else rdm2_keys_same_kernel<<<(unsigned)div_up(n2, 256), 256, 0, s>>>(cls ? D : U, cls ? U : D, n2, K, ku.p, kd.p, pay.p);
     SQ_LAUNCH_CHECK();
     SQ_CHECK(idx.alloc(m));
     SQ_CHECK(sort_pairs_index(1, norb, ku.p, kd.p, idx.p, m, s));
@@ -694,11 +713,95 @@ static int rdm2_accumulate(sqmc_b200_handle *h, const char *who, int64_t n, cons
     SQ_CHECK(gather_strings(1, pay.p, idx.p, spay.p, m, s));
     pay.release(); idx.release();
     marks.mark(cls == 0 ? "alpha alpha keys + sort" : cls == 1 ? "beta beta keys + sort" : "alpha beta keys + sort");
-    rdm2_pair_kernel<<<(unsigned)div_up(m, 256), 256, 0, s>>>(sku.p, skd.p, spay.p, m, cls == 2 ? -1 : cls == 0 ? 0 : R.off_bb, c.p, R);
-    SQ_LAUNCH_CHECK();
+    SQ_CHECK(visit(sku.p, skd.p, spay.p, m, cls == 2 ? (int64_t)-1 : cls == 0 ? (int64_t)0 : R.off_bb));
     marks.mark(cls == 0 ? "alpha alpha pairs" : cls == 1 ? "beta beta pairs" : "alpha beta pairs");
   }
   return 0;
+}
+
+// slot layout of the representatives (aa, bb, ab) for norb orbitals and S states
+static void rdm2_layout(Rdm2Acc &R, int norb, int S) {
+  const int M = norb * (norb - 1) / 2;
+  R.M = M; R.norb = norb; R.S = S; R.cs = S;
+  R.off_bb = (int64_t)M * M;
+  R.off_ab = 2 * R.off_bb;
+  R.per = R.off_ab + (int64_t)norb * norb * norb * norb;
+}
+
+// The accumulation both two-particle entry points share: upload, time_sym expansion, checks, the diagonal and the three key
+// classes with their pairs.  On return acc / scale hold the representatives of R (scale[S + k]: the factor back to doubles);
+// norm2 (device, S doubles, may be null) receives ||Psi_k||^2 summed in a fixed order.
+// two = true: wts holds 2S columns, a_k = column k and b_k = column S + k; b_k is first made orthogonal to a_k on the device, and
+// the representatives are those of the symmetrised transition density (<a_k| E |b_k> + <b_k| E |a_k>) / 2, on a grid from
+// ||a_k|| ||b_k|| (Cauchy-Schwarz again); norm2 receives ||a_k||^2.
+static int rdm2_accumulate(sqmc_b200_handle *h, const char *who, int64_t n, const void *dets_up, const void *dets_dn, int S, const double *wts,
+                           int64_t ldw, HostMarks &marks, DevBuf<unsigned long long> &acc, DevBuf<double> &scale, Rdm2Acc &R, double *norm2,
+                           bool two = false) {
+  cudaStream_t s = G.stream;
+  const ModelTables &T = h->T;
+  const int norb = T.norb;
+  DevBuf<uint64_t> up, dn, U, D;
+  DevBuf<double> w, c;
+  DevBuf<int32_t> idx0;
+  int64_t n2 = 0;
+  SQ_CHECK(prepare_dets<1>(h, who, n, dets_up, dets_dn, two ? 2 * S : S, wts, ldw, up, dn, w, n2, idx0, U, D, c));
+  up.release(); dn.release(); w.release(); idx0.release();
+  marks.mark("upload, expansion, checks");
+  SQ_CHECK(rdm2_electron_check(T, who, U.p, D.p, n2, s));
+  if (two) {
+    DevBuf<double> dots;
+    SQ_CHECK(dots.alloc(2 * S));
+    dots_kernel<<<S, 256, 0, s>>>(c.p, n2, S, dots.p);
+    SQ_LAUNCH_CHECK();
+    project_out_kernel<<<(unsigned)div_up(n2 * S, 256), 256, 0, s>>>(c.p, n2, S, dots.p);
+    SQ_LAUNCH_CHECK();
+    if (norm2) SQ_CUDA(cudaMemcpyAsync(norm2, dots.p, S * sizeof(double), cudaMemcpyDeviceToDevice, s));
+  } else if (norm2) {
+    norm2_kernel<<<S, 256, 0, s>>>(c.p, n2, S, norm2);
+    SQ_LAUNCH_CHECK();
+  }
+  // grid exponent per state from sum_i w_ik^2 (the time_sym expansion keeps it); the margin keeps e_k the same whatever order
+  // the sum was taken in, unless the norm lies within a few ulps of 2^e / (1 + 2^-20)
+  std::vector<double> hs(2 * S);
+  for (int k = 0; k < S; k++) {
+    double n2k = 0.0;
+    if (two) {
+      double na = 0.0, nb = 0.0;
+      for (int64_t i = 0; i < n; i++) na += wts[k * ldw + i] * wts[k * ldw + i];
+      for (int64_t i = 0; i < n; i++) nb += wts[(S + k) * ldw + i] * wts[(S + k) * ldw + i];
+      n2k = sqrt(na * nb);
+    } else {
+      for (int64_t i = 0; i < n; i++) n2k += wts[k * ldw + i] * wts[k * ldw + i];
+    }
+    int e = 0;
+    if (n2k > 0.0) frexp(n2k * (1.0 + 0x1p-20), &e);
+    hs[k] = ldexp(1.0, kFixBits - e);
+    hs[S + k] = ldexp(1.0, e - kFixBits);
+  }
+  rdm2_layout(R, norb, S);
+  if (two) R.cs = 2 * S;
+  SQ_CHECK(acc.alloc(2 * S * R.per));
+  SQ_CHECK(scale.alloc(2 * S));
+  SQ_CUDA(cudaMemsetAsync(acc.p, 0, (size_t)acc.n * sizeof(unsigned long long), s));
+  SQ_CUDA(cudaMemcpyAsync(scale.p, hs.data(), 2 * S * sizeof(double), cudaMemcpyHostToDevice, s));
+  R.a = acc.p;
+  R.scale = scale.p;
+
+  const size_t dsh = (size_t)6 * norb * norb * sizeof(unsigned long long);
+  auto diag = two ? rdm2_diag_kernel<true> : rdm2_diag_kernel<false>;
+  SQ_CUDA(cudaFuncSetAttribute(diag, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dsh));
+  diag<<<(unsigned)std::min<int64_t>(div_up(n2, 256), 2 * G.sm_count), 256, dsh, s>>>(U.p, D.p, n2, c.p, R);
+  SQ_LAUNCH_CHECK();
+  marks.mark("diagonal");
+
+  const Rdm2Acc Rc = R;
+  const double *cp = c.p;
+  return rdm2_for_each_class(T, who, U.p, D.p, n2, R, marks, [&](const uint64_t *sku, const uint64_t *skd, const uint64_t *spay, int64_t m, int64_t boff) {
+    if (two) rdm2_pair_kernel<true><<<(unsigned)div_up(m, 256), 256, 0, s>>>(sku, skd, spay, m, boff, cp, Rc);
+    else rdm2_pair_kernel<false><<<(unsigned)div_up(m, 256), 256, 0, s>>>(sku, skd, spay, m, boff, cp, Rc);
+    SQ_LAUNCH_CHECK();
+    return 0;
+  });
 }
 
 static int two_rdm_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int S, const double *wts, int64_t ldw, double *rdm) {
@@ -996,21 +1099,397 @@ static int orbital_derivatives_impl(sqmc_b200_handle *h, int64_t n, const void *
   return 0;
 }
 
-int orbital_derivatives(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw,
-                        const double *state_weights, double *fock, double *hessian, double *energy) {
+// argument checks of the entry points that work on the orbitals of a chem handle
+static int orbital_check_args(sqmc_b200_handle *h, const char *who, int64_t n, int n_states, int64_t ldw) {
   if (h->T.model != MODEL_CHEM) {
-    set_error("orbital_derivatives: only chem handles have orbitals to optimise (heg and hubbardk orbitals are fixed by momentum)");
+    set_error("%s: only chem handles have orbitals to optimise (heg and hubbardk orbitals are fixed by momentum)", who);
     return 2;
   }
-  SQ_CHECK(rdm2_check_args(h, "orbital_derivatives", n, n_states, ldw));
-  if (h->T.nup + h->T.ndn < 2) { set_error("orbital_derivatives: needs at least two electrons"); return 2; }
+  SQ_CHECK(rdm2_check_args(h, who, n, n_states, ldw));
+  if (h->T.nup + h->T.ndn < 2) { set_error("%s: needs at least two electrons", who); return 2; }
+  return 0;
+}
+
+static int state_weights_check(const char *who, int n_states, const double *state_weights) {
   double sum = 0.0;
   for (int k = 0; k < n_states; k++) {
-    if (!(state_weights[k] >= 0.0)) { set_error("orbital_derivatives: state_weights[%d] = %g is negative", k, state_weights[k]); return 2; }
+    if (!(state_weights[k] >= 0.0)) { set_error("%s: state_weights[%d] = %g is negative", who, k, state_weights[k]); return 2; }
     sum += state_weights[k];
   }
-  if (!(fabs(sum - 1.0) <= 1e-12)) { set_error("orbital_derivatives: state_weights sum to %.17g, not 1", sum); return 2; }
+  if (!(fabs(sum - 1.0) <= 1e-12)) { set_error("%s: state_weights sum to %.17g, not 1", who, sum); return 2; }
+  return 0;
+}
+
+int orbital_derivatives(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw,
+                        const double *state_weights, double *fock, double *hessian, double *energy) {
+  SQ_CHECK(orbital_check_args(h, "orbital_derivatives", n, n_states, ldw));
+  SQ_CHECK(state_weights_check("orbital_derivatives", n_states, state_weights));
   return orbital_derivatives_impl(h, n, dets_up, dets_dn, n_states, wts, ldw, state_weights, fock, hessian, energy);
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// sigma-vector y = H x over a determinant list (sqmc_b200_sigma), chem, norb <= 64
+//
+// The two-body contraction of rdm_energy, E(c) = E_core ||c||^2 + 1/2 sum g'_pqrs d_pqrs with the one-body part folded into
+//   g'_pqrs = g_pqrs + (h_pq delta_rs + delta_pq h_rs) / (N - 1)        (sum_r d_pqrr = (N - 1) gamma_pq),
+// is a sum over the representatives of two_rdm, E = E_core ||c||^2 + sum_slot G[slot] rep[slot], G[slot] = dE / drep[slot]
+// (sigma_table_kernel: same spin (g'_pqrs - g'_psrq) x (2 if A != B), alpha beta g'_pqrs x (1 if p = q and r = s, else 2)).
+// rep is quadratic in c: each pair visit of rdm2_for_each_class adds f c_i c_j, each determinant's diagonal slots c_i^2.  So
+// H x = 1/2 grad E(x): a visit adds f G[slot] x_j / 2 to y_i and f G[slot] x_i / 2 to y_j (a single is met once per spectator
+// orbital and each visit adds its own share), the diagonal adds x_i sum G over the determinant's diagonal slots.  Every pair of
+// the list connected by a single or double excitation is visited, whatever its matrix element: no stored pattern is used.
+// With kappa, h and g are replaced by their derivatives along the rotation U(t) = expm(-t kappa) (rotate_fcidump's rule):
+//   h^k = kappa h - h kappa,   g^k_pqrs = sum_m (k_pm g_mqrs + k_qm g_pmrs + k_rm g_pqms + k_sm g_pqrm),
+// and the core term is left out.  g^k is one FP64 product T1(p; x y z) = sum_m k_pm g_mxyz (orb_gemm_kernel, O(norb^5)) and
+// its four index placements.
+//
+// Determinism: y is accumulated per (row of the sorted view, state) as a 128-bit fixed-point integer in units of 2^(e_k - 120),
+// 2^e_k > B_k = max|G| max|x_k| (n_diag + V / 2): n_diag diagonal slots per determinant, and at most V = (N - 1) x
+// min(n2 - 1, singles + doubles of one determinant) visits per row (a single is met N - 1 times, a double once).  B_k bounds
+// every partial sum of a row, so the integers stay below 2^120, and integer addition does not depend on the order of the
+// atomics: repeated calls and row permutations give the same bits.  time_sym lists are expanded as for two_rdm and y is folded
+// back onto the representatives, (y_(u,d) + z y_(d,u)) / sqrt2 and y_(u,u) as it is.
+
+// T1(i; x y z) = C[i + norb (z + norb (y + norb x))] (the product of kappa with g read as B(j, m) = g_{j, m}); g^k and h^k
+__global__ void sigma_kappa_ints_kernel(const double *kap, const double *hd, const double *T1, int norb, double *hk, double *gk) {
+  const int64_t n = norb, nn = n * n, n4 = nn * nn;
+  auto t1 = [&](int64_t i, int64_t x, int64_t y, int64_t z) { return T1[i + n * (z + n * (y + n * x))]; };
+  for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < n4 + nn; t += (int64_t)gridDim.x * blockDim.x) {
+    if (t < n4) {
+      int64_t x = t;
+      const int64_t p = x % n; x /= n;
+      const int64_t q = x % n; x /= n;
+      const int64_t r = x % n;
+      const int64_t s = x / n;
+      gk[t] = (t1(p, q, r, s) + t1(q, p, r, s)) + (t1(r, s, p, q) + t1(s, r, p, q));  // symmetric under p<->q, r<->s, pq<->rs
+    } else {
+      const int64_t u = t - n4, p = u % n, q = u / n;
+      double a = 0.0, b = 0.0;
+      for (int64_t m = 0; m < n; m++) {
+        a += kap[p + n * m] * hd[m + n * q];
+        b += hd[p + n * m] * kap[m + n * q];
+      }
+      hk[u] = a - b;
+    }
+  }
+}
+
+// G[slot] = dE / drep[slot] for every representative slot of R's layout (slots no pair reaches get values nobody reads)
+__global__ void sigma_table_kernel(const double *hd, const double *gd, Rdm2Acc R, double inv_nm1, double *G) {
+  const int64_t n = R.norb, nn = n * n, M = R.M;
+  auto gp = [&](int64_t p, int64_t q, int64_t r, int64_t s) {
+    double a = gd[p + n * (q + n * (r + n * s))];
+    double one = 0.0;
+    if (r == s) one += hd[p + n * q];
+    if (p == q) one += hd[r + n * s];
+    return a + one * inv_nm1;
+  };
+  auto unpair = [](int64_t A, int64_t &p, int64_t &r) {  // A = r (r - 1) / 2 + p, p < r
+    r = (int64_t)((1.0 + sqrt(1.0 + 8.0 * (double)A)) * 0.5);
+    while (r * (r - 1) / 2 > A) r--;
+    while ((r + 1) * r / 2 <= A) r++;
+    p = A - r * (r - 1) / 2;
+  };
+  for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < R.per; t += (int64_t)gridDim.x * blockDim.x) {
+    double v;
+    if (t < R.off_ab) {
+      const int64_t u = t < R.off_bb ? t : t - R.off_bb;
+      const int64_t A = u % M, B = u / M;
+      if (A > B) {
+        v = 0.0;
+      } else {
+        int64_t p, q, r, s;
+        unpair(A, p, r);
+        unpair(B, q, s);
+        v = (gp(p, q, r, s) - gp(p, s, r, q)) * (A != B ? 2.0 : 1.0);
+      }
+    } else {
+      const int64_t u = t - R.off_ab, X = u % nn, Y = u / nn;
+      const int64_t p = X % n, q = X / n, r = Y % n, s = Y / n;
+      v = gp(p, q, r, s) * ((p == q && r == s) ? 1.0 : 2.0);
+    }
+    G[t] = v;
+  }
+}
+
+// *out = max |a| (the bit patterns of non-negative doubles order as the values: an integer max, independent of order)
+__global__ void absmax_kernel(const double *a, int64_t n, unsigned long long *out) {
+  unsigned long long m = 0ull;
+  for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < n; t += (int64_t)gridDim.x * blockDim.x)
+    m = max(m, (unsigned long long)__double_as_longlong(fabs(a[t])));
+  for (int o = 16; o > 0; o >>= 1) m = max(m, __shfl_xor_sync(0xffffffffu, m, o));
+  if ((threadIdx.x & 31) == 0 && m) atomicMax(out, m);
+}
+
+// y of row i starts at x_i times the sum of G over its diagonal slots (summed in bit order), stored, not added
+__global__ void sigma_diag_kernel(const uint64_t *u, const uint64_t *d, int64_t n, const double *x, const double *G, Rdm2Acc R,
+                                  const double *scale, unsigned long long *Y) {
+  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const uint64_t U = u[i], D = d[i];
+  double a = 0.0;
+  for (uint64_t ps = U; ps; ps &= ps - 1) {
+    const int p = __ffsll((long long)ps) - 1;
+    for (uint64_t rs = ps & (ps - 1); rs; rs &= rs - 1) a += G[(int64_t)pair_index(p, __ffsll((long long)rs) - 1) * (1 + R.M)];
+    for (uint64_t rs = D; rs; rs &= rs - 1) {
+      const int r = __ffsll((long long)rs) - 1;
+      a += G[R.off_ab + ab_slot(p, p, r, r, R.norb)];
+    }
+  }
+  for (uint64_t ps = D; ps; ps &= ps - 1) {
+    const int p = __ffsll((long long)ps) - 1;
+    for (uint64_t rs = ps & (ps - 1); rs; rs &= rs - 1) a += G[R.off_bb + (int64_t)pair_index(p, __ffsll((long long)rs) - 1) * (1 + R.M)];
+  }
+  for (int k = 0; k < R.S; k++) {
+    uint64_t lo, hi;
+    fix_to_i128(a * x[i * R.S + k] * scale[k], lo, hi);
+    Y[2 * (i * R.S + k)] = lo;
+    Y[2 * (i * R.S + k) + 1] = hi;
+  }
+}
+
+// one thread per sorted entry i, every later entry j of its bucket: f G[slot] / 2 times x_j into y_i and times x_i into y_j
+__global__ void __launch_bounds__(256) sigma_pair_kernel(const uint64_t *ku, const uint64_t *kd, const uint64_t *pay, int64_t m, int64_t boff,
+                                                         const double *x, const double *G, Rdm2Acc R, const double *scale,
+                                                         unsigned long long *Y) {
+  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (i >= m) return;
+  const uint64_t ki = ku[i], kdi = kd[i], pi = pay[i];
+  const int ai = (int)(pi & 0xff), bi = (int)((pi >> 8) & 0xff);
+  const int64_t ri = (int64_t)(pi >> 16);
+  const double *xi = x + ri * R.S;
+  for (int64_t j = i + 1; j < m && ku[j] == ki && kd[j] == kdi; j++) {
+    const uint64_t pj = pay[j];
+    double f;
+    const int64_t slot = rdm2_pair_slot(ki, kdi, ai, bi, (int)(pj & 0xff), (int)((pj >> 8) & 0xff), boff, R.M, R.norb, R.off_ab, f);
+    const double gs = 0.5 * f * G[slot];
+    if (gs == 0.0) continue;
+    const int64_t rj = (int64_t)(pj >> 16);
+    const double *xj = x + rj * R.S;
+    for (int k = 0; k < R.S; k++) {
+      uint64_t lo, hi;
+      fix_to_i128(gs * xj[k] * scale[k], lo, hi);
+      i128_add(Y + 2 * (ri * R.S + k), lo, hi);
+      fix_to_i128(gs * xi[k] * scale[k], lo, hi);
+      i128_add(Y + 2 * (rj * R.S + k), lo, hi);
+    }
+  }
+}
+
+// y back to doubles, plus the core term, scattered from the sorted view to the expanded order (column-major n2 x S)
+__global__ void sigma_finish_kernel(const unsigned long long *Y, const double *x, const int32_t *idx, int64_t n2, int S, const double *unscale,
+                                    double ecore, double *ye) {
+  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (t >= n2 * S) return;
+  const int64_t v = t / S;
+  const int k = (int)(t % S);
+  const double a = (ldexp((double)(long long)Y[2 * t + 1], 64) + (double)Y[2 * t]) * unscale[k];
+  ye[k * n2 + idx[v]] = a + ecore * x[t];
+}
+
+__global__ void partner_index_kernel(const int32_t *sel, int64_t m, int64_t n, int32_t *partner) {
+  const int64_t j = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (j < m) partner[sel[j]] = (int32_t)(n + j);
+}
+
+// time_sym: y of each representative from its plain determinants, (y_(u,d) + z y_(d,u)) / sqrt2, or y_(u,u)
+__global__ void ts_fold_kernel(const double *ye, int64_t n, int64_t n2, int S, const int32_t *partner, double z, double r, double *y) {
+  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (t >= n * S) return;
+  const int64_t i = t % n, k = t / n;
+  const double a = ye[k * n2 + i];
+  y[t] = partner[i] < 0 ? a : (a + z * ye[k * n2 + partner[i]]) * r;
+}
+
+// dense h and g from the handle's table, or their kappa derivatives (kappa: host, norb^2, kappa_pq at p + norb q)
+static int orbital_integrals(sqmc_b200_handle *h, const double *kappa, DevBuf<double> &hd, DevBuf<double> &gd, cudaStream_t s) {
+  const ModelTables &T = h->T;
+  const int norb = T.norb;
+  const int64_t nn = (int64_t)norb * norb, n4 = nn * nn;
+  SQ_CHECK(hd.alloc(nn));
+  SQ_CHECK(gd.alloc(n4));
+  orbd_integrals_kernel<<<(unsigned)std::min<int64_t>(div_up(n4 + nn, 256), 64 * G.sm_count), 256, 0, s>>>(T.integrals, T.combine_2, norb, hd.p, gd.p);
+  SQ_LAUNCH_CHECK();
+  if (!kappa) return 0;
+  DevBuf<double> kap, T1, hk, gk;
+  SQ_CHECK(kap.alloc(nn));
+  SQ_CUDA(cudaMemcpyAsync(kap.p, kappa, nn * sizeof(double), cudaMemcpyHostToDevice, s));
+  SQ_CHECK(T1.alloc(n4));
+  SQ_CHECK(orb_gemm(GemmSeg{kap.p, gd.p, norb}, GemmSeg{nullptr, nullptr, 0}, norb, (int)(nn * norb), T1.p, s));
+  SQ_CHECK(hk.alloc(nn));
+  SQ_CHECK(gk.alloc(n4));
+  sigma_kappa_ints_kernel<<<(unsigned)std::min<int64_t>(div_up(n4 + nn, 256), 64 * G.sm_count), 256, 0, s>>>(kap.p, hd.p, T1.p, norb, hk.p, gk.p);
+  SQ_LAUNCH_CHECK();
+  hd.release(); gd.release();
+  hd.n = nn; hd.p = hk.take();
+  gd.n = n4; gd.p = gk.take();
+  return 0;
+}
+
+static int sigma_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int S, const double *x, int64_t ldx,
+                      const double *kappa, double *y) {
+  cudaStream_t s = G.stream;
+  const ModelTables &T = h->T;
+  const int norb = T.norb;
+  const bool ts = T.time_sym;
+  HostMarks marks("SQMC_SIGMA_PROFILE", "sigma");  // =1: phase split (synchronising) on stderr
+  DevBuf<uint64_t> up, dn, U, D;
+  DevBuf<double> w, c;
+  DevBuf<int32_t> idx0, sel;
+  int64_t n2 = 0;
+  SQ_CHECK(prepare_dets<1>(h, "sigma", n, dets_up, dets_dn, S, x, ldx, up, dn, w, n2, idx0, U, D, c, &sel));
+  up.release(); dn.release(); w.release();
+  marks.mark("upload, expansion, checks");
+  SQ_CHECK(rdm2_electron_check(T, "sigma", U.p, D.p, n2, s));
+
+  Rdm2Acc R;
+  rdm2_layout(R, norb, S);
+  DevBuf<double> Gt, scale;
+  DevBuf<unsigned long long> gmax;
+  {
+    DevBuf<double> hd, gd;
+    SQ_CHECK(orbital_integrals(h, kappa, hd, gd, s));
+    SQ_CHECK(Gt.alloc(R.per));
+    sigma_table_kernel<<<(unsigned)std::min<int64_t>(div_up(R.per, 256), 64 * G.sm_count), 256, 0, s>>>(hd.p, gd.p, R, 1.0 / (T.nup + T.ndn - 1), Gt.p);
+    SQ_LAUNCH_CHECK();
+  }
+  SQ_CHECK(gmax.alloc(1));
+  SQ_CUDA(cudaMemsetAsync(gmax.p, 0, sizeof(unsigned long long), s));
+  absmax_kernel<<<(unsigned)std::min<int64_t>(div_up(R.per, 256), 8 * G.sm_count), 256, 0, s>>>(Gt.p, R.per, gmax.p);
+  SQ_LAUNCH_CHECK();
+  unsigned long long gbits = 0;
+  SQ_CUDA(cudaMemcpyAsync(&gbits, gmax.p, sizeof(gbits), cudaMemcpyDeviceToHost, s));
+  SQ_CUDA(cudaStreamSynchronize(s));
+  double gm;
+  memcpy(&gm, &gbits, sizeof(gm));
+  marks.mark("integrals, G table");
+
+  // the grid exponent per state (see above); every input of the bound is independent of the row order
+  const double na = T.nup, nb = T.ndn, no = norb;
+  const double ndiag = na * (na - 1) / 2 + nb * (nb - 1) / 2 + na * nb;
+  const double sa = na * (no - na), sb = nb * (no - nb);
+  const double nexc = sa + sb + (na * (na - 1) / 2) * ((no - na) * (no - na - 1) / 2) + (nb * (nb - 1) / 2) * ((no - nb) * (no - nb - 1) / 2) + sa * sb;
+  const double visits = (na + nb - 1) * std::min((double)(n2 - 1), nexc);
+  std::vector<double> hs(2 * S);
+  for (int k = 0; k < S; k++) {
+    double xm = 0.0;
+    for (int64_t i = 0; i < n; i++) xm = std::max(xm, fabs(x[k * ldx + i]));
+    const double B = gm * xm * (ndiag + 0.5 * visits);
+    int e = 0;
+    if (B > 0.0) frexp(B, &e);
+    hs[k] = ldexp(1.0, kFixBits - e);
+    hs[S + k] = ldexp(1.0, e - kFixBits);
+  }
+  SQ_CHECK(scale.alloc(2 * S));
+  SQ_CUDA(cudaMemcpyAsync(scale.p, hs.data(), 2 * S * sizeof(double), cudaMemcpyHostToDevice, s));
+
+  DevBuf<unsigned long long> Y;
+  SQ_CHECK(Y.alloc(2 * n2 * S));
+  sigma_diag_kernel<<<(unsigned)div_up(n2, 256), 256, 0, s>>>(U.p, D.p, n2, c.p, Gt.p, R, scale.p, Y.p);
+  SQ_LAUNCH_CHECK();
+  marks.mark("diagonal");
+  const double *cp = c.p, *gp = Gt.p, *sp = scale.p;
+  unsigned long long *yp = Y.p;
+  SQ_CHECK(rdm2_for_each_class(T, "sigma", U.p, D.p, n2, R, marks, [&](const uint64_t *sku, const uint64_t *skd, const uint64_t *spay, int64_t m, int64_t boff) {
+    sigma_pair_kernel<<<(unsigned)div_up(m, 256), 256, 0, s>>>(sku, skd, spay, m, boff, cp, gp, R, sp, yp);
+    SQ_LAUNCH_CHECK();
+    return 0;
+  }));
+
+  DevBuf<double> ye, yo;
+  SQ_CHECK(ye.alloc(n2 * S));
+  sigma_finish_kernel<<<(unsigned)div_up(n2 * S, 256), 256, 0, s>>>(Y.p, c.p, idx0.p, n2, S, scale.p + S, kappa ? 0.0 : T.enuc, ye.p);
+  SQ_LAUNCH_CHECK();
+  const double *out = ye.p;
+  if (ts) {
+    DevBuf<int32_t> partner;
+    SQ_CHECK(partner.alloc(n));
+    SQ_CUDA(cudaMemsetAsync(partner.p, 0xff, n * sizeof(int32_t), s));  // -1: no partner
+    if (n2 > n) {
+      partner_index_kernel<<<(unsigned)div_up(n2 - n, 256), 256, 0, s>>>(sel.p, n2 - n, n, partner.p);
+      SQ_LAUNCH_CHECK();
+    }
+    SQ_CHECK(yo.alloc(n * S));
+    ts_fold_kernel<<<(unsigned)div_up(n * S, 256), 256, 0, s>>>(ye.p, n, n2, S, partner.p, T.z, T.sqrt2inv, yo.p);
+    SQ_LAUNCH_CHECK();
+    out = yo.p;
+  }
+  SQ_CUDA(cudaMemcpyAsync(y, out, (size_t)n * S * sizeof(double), cudaMemcpyDeviceToHost, s));
+  SQ_CUDA(cudaStreamSynchronize(s));
+  marks.mark("fold + copy out");
+  return 0;
+}
+
+int sigma(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *x, int64_t ldx,
+          const double *kappa, double *y) {
+  SQ_CHECK(orbital_check_args(h, "sigma", n, n_states, ldx));
+  if (kappa) {
+    const int norb = h->T.norb;
+    for (int p = 0; p < norb; p++)
+      for (int q = 0; q <= p; q++)
+        if (kappa[p + norb * q] != -kappa[q + norb * p]) {
+          set_error("sigma: kappa is not antisymmetric (kappa[%d,%d] = %g, kappa[%d,%d] = %g)", p, q, kappa[p + norb * q], q, p, kappa[q + norb * p]);
+          return 2;
+        }
+  }
+  return sigma_impl(h, n, dets_up, dets_dn, n_states, x, ldx, kappa, y);
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// orbital-gradient response (sqmc_b200_orbital_gradient_response): d/dt of the orbital gradient 2 (F - F^T) of
+// orbital_derivatives at the vectors c_k + t dc_k, t = 0.  F is linear in the state-averaged normalised densities, and
+//   d/dt [w_k d(c_k + t dc_k) / ||c_k + t dc_k||^2] = (2 w_k / ||c_k||^2) T(c_k, dc_k')
+// with T the symmetrised transition density and dc_k' = dc_k - (<c_k|dc_k> / ||c_k||^2) c_k (the normalisation term).  So the
+// two-vector mode of rdm2_accumulate gives the representatives of T(c_k, dc_k'), orbd_fill_kernel the spin-summed d with the
+// factors 2 w_k / ||c_k||^2, and one F product (no Y term) the response 2 (F - F^T).
+static int orbital_gradient_response_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int S, const double *wts,
+                                          const double *dwts, int64_t ldw, const double *state_weights, double *response) {
+  cudaStream_t s = G.stream;
+  const ModelTables &T = h->T;
+  const int norb = T.norb;
+  const int64_t nn = (int64_t)norb * norb, n4 = nn * nn;
+  HostMarks marks("SQMC_ORBD_PROFILE", "orbital_gradient_response");  // =1: phase split (synchronising) on stderr
+  std::vector<double> ab((size_t)2 * S * n);  // [c_1 .. c_S | dc_1 .. dc_S], leading dimension n
+  for (int k = 0; k < S; k++) {
+    memcpy(ab.data() + (size_t)k * n, wts + k * ldw, n * sizeof(double));
+    memcpy(ab.data() + (size_t)(S + k) * n, dwts + k * ldw, n * sizeof(double));
+  }
+  std::vector<double> w2(S);
+  for (int k = 0; k < S; k++) w2[k] = 2.0 * state_weights[k];
+  DevBuf<double> norm2, sw, d, D;
+  SQ_CHECK(norm2.alloc(S));
+  SQ_CHECK(sw.alloc(S));
+  SQ_CUDA(cudaMemcpyAsync(sw.p, w2.data(), S * sizeof(double), cudaMemcpyHostToDevice, s));
+  {
+    DevBuf<unsigned long long> acc;
+    DevBuf<double> scale;
+    Rdm2Acc R;
+    SQ_CHECK(rdm2_accumulate(h, "orbital_gradient_response", n, dets_up, dets_dn, S, ab.data(), n, marks, acc, scale, R, norm2.p, true));
+    SQ_CHECK(d.alloc(n4));
+    orbd_fill_kernel<<<(unsigned)std::min<int64_t>(div_up(n4, 256), 64 * G.sm_count), 256, 0, s>>>(R, scale.p + S, sw.p, norm2.p, d.p);
+    SQ_LAUNCH_CHECK();
+  }
+  SQ_CHECK(D.alloc(nn));
+  orbd_trace_kernel<<<(unsigned)div_up(nn, 256), 256, 0, s>>>(d.p, norb, 1.0 / (T.nup + T.ndn - 1), D.p);
+  SQ_LAUNCH_CHECK();
+  DevBuf<double> hd, gd, F;
+  SQ_CHECK(orbital_integrals(h, nullptr, hd, gd, s));
+  SQ_CHECK(F.alloc(nn));
+  SQ_CHECK(orb_gemm(GemmSeg{D.p, hd.p, norb}, GemmSeg{d.p, gd.p, nn * norb}, norb, norb, F.p, s));
+  std::vector<double> Fh(nn);
+  SQ_CUDA(cudaMemcpyAsync(Fh.data(), F.p, nn * sizeof(double), cudaMemcpyDeviceToHost, s));
+  SQ_CUDA(cudaStreamSynchronize(s));
+  marks.mark("d, F, copy out");
+  for (int q = 0; q < norb; q++)
+    for (int p = 0; p < norb; p++) response[p + (int64_t)norb * q] = 2.0 * (Fh[p + norb * q] - Fh[q + norb * p]);
+  return 0;
+}
+
+int orbital_gradient_response(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts,
+                              const double *dwts, int64_t ldw, const double *state_weights, double *response) {
+  SQ_CHECK(orbital_check_args(h, "orbital_gradient_response", n, n_states, ldw));
+  SQ_CHECK(state_weights_check("orbital_gradient_response", n_states, state_weights));
+  return orbital_gradient_response_impl(h, n, dets_up, dets_dn, n_states, wts, dwts, ldw, state_weights, response);
 }
 
 }  // namespace sqmc

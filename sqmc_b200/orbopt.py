@@ -4,13 +4,15 @@ Every macro iteration solves the CI problem in the current orbitals, takes Spars
 state-averaged variational energy, and makes a Newton step in the rotations kappa_pq (p > q, same irrep) on the reduced
 Hessian, level-shifted when its lowest eigenvalue is below a small positive floor and capped in size.  The orbitals are kept
 as the total rotation C relative to the original FCIDUMP, and every iteration writes natorb.rotate_fcidump(original, C), so
-the integral filter of the reader never compounds.  CI-orbital coupling is not included.
+the integral filter of the reader never compounds.
 
-Two modes, both through hci.perform_hci:
+Three modes, all through hci.perform_hci:
   re-select (default)  every iteration runs the input's HCI schedule from the HF determinant in the current orbitals (no PT);
   fixed list           the determinant list of the first run is carried along (remap_determinants), each iteration rebuilds
                        H and runs Davidson from the previous vectors; a step that raises the weighted energy is halved and
                        retried, so the energy does not increase.
+  one step             fixed list, with the Newton step taken in the CI-orbital coupled system (coupled_step): the orbital
+                       step then accounts for the relaxation of the CI vectors, which the two-step Hessian leaves out.
 """
 import os
 import time
@@ -85,6 +87,73 @@ def newton_step(grad, hess, max_step=0.5, floor=1.0e-4):
     return step, shift
 
 
+def kappa_in_library(norb, pairs, step):
+    """the antisymmetric kappa in library numbering from the step over library pairs (p, q)"""
+    K = np.zeros((norb, norb))
+    for (p, q), k in zip(pairs, step):
+        K[p, q], K[q, p] = k, -k
+    return K
+
+
+def coupled_step(H, up, dn, C, energies, sw, grad, hess, pairs, max_step=0.5, floor=1.0e-4, rtol=1.0e-3, max_micro=50):
+    """Newton step of the CI-orbital coupled problem at the orthonormal CI vectors C (n x S, columns the states, energies E_k)
+    over the resident matrix of H (built over up, dn in this order).  Unknowns: x over the rotations `pairs` and Y (n x S),
+    every column orthogonal to all of C (P = 1 - C C^T).  The Hessian-vector product has the blocks
+      oo: hess (the reduced Hessian of orbital_derivatives)      oc: orbital_gradient_response(C, Y, sw) over pairs
+      co: 2 w_k P H^x c_k (H.sigma with kappa)                   cc: 2 w_k P (H - E_k) y_k (the resident H.v)
+    and the gradient is (grad, 2 w_k P (H - E_k) c_k).  The system, shifted by newton_step's level shift of the orbital block,
+    is solved by conjugate gradients preconditioned with diag(hess) and 2 w_k (H_ii - E_k); a direction of non-positive
+    curvature ends the iteration.  The step is scaled so that |x| <= max_step.  -> (x, Y, shift, micro iterations)"""
+    norb = H.system.norb
+    S = C.shape[1]
+    w = np.asarray(sw, dtype=np.float64)
+    E = np.asarray(energies, dtype=np.float64)
+    ip = np.array([p for p, _ in pairs], dtype=np.int64)
+    iq = np.array([q for _, q in pairs], dtype=np.int64)
+    shift = max(0.0, floor - float(np.linalg.eigvalsh(0.5 * (hess + hess.T))[0])) if len(pairs) else 0.0
+    proj = lambda Y: Y - C @ (C.T @ Y)
+
+    def apply(x, Y):
+        HY = H.matvec(Y).reshape(Y.shape)
+        sig = H.sigma(up, dn, C, kappa=kappa_in_library(norb, pairs, x)).reshape(C.shape)
+        rc = proj(2.0 * w * (sig + HY - E * Y)) + shift * Y
+        ro = hess @ x + H.orbital_gradient_response(up, dn, C, Y, state_weights=w)[ip, iq] + shift * x
+        return ro, rc
+
+    go = np.asarray(grad, dtype=np.float64)
+    gc = proj(2.0 * w * (H.matvec(C).reshape(C.shape) - E * C))
+    do = np.maximum(np.diag(hess) + shift, floor)
+    dc = np.maximum(2.0 * w * (H.diagonal(up, dn)[:, None] - E) + shift, floor)
+    x, Y = np.zeros_like(go), np.zeros_like(C)
+    ro, rc = -go, -gc
+    zo, zc = ro / do, proj(rc / dc)
+    po, pc = zo.copy(), zc.copy()
+    rz = float(ro @ zo + np.sum(rc * zc))
+    r0 = np.sqrt(float(ro @ ro + np.sum(rc * rc)))
+    micro = 0
+    while micro < max_micro and r0 > 0.0:
+        ao, ac = apply(po, pc)
+        micro += 1
+        curv = float(po @ ao + np.sum(pc * ac))
+        if curv <= 0.0:
+            if micro == 1:   # no positive curvature along the preconditioned gradient: take that direction
+                x, Y = po, pc
+            break
+        a = rz / curv
+        x, Y = x + a * po, Y + a * pc
+        ro, rc = ro - a * ao, rc - a * ac
+        if np.sqrt(float(ro @ ro + np.sum(rc * rc))) <= rtol * r0:
+            break
+        zo, zc = ro / do, proj(rc / dc)
+        rz_new = float(ro @ zo + np.sum(rc * zc))
+        po, pc = zo + (rz_new / rz) * po, zc + (rz_new / rz) * pc
+        rz = rz_new
+    nrm = float(np.linalg.norm(x))
+    if nrm > max_step:
+        x, Y = x * (max_step / nrm), Y * (max_step / nrm)
+    return x, Y, shift, micro
+
+
 def kappa_in_fcidump_columns(system, pairs, step):
     """the antisymmetric kappa in FCIDUMP columns from the step over library pairs (p, q)"""
     norb = system.norb
@@ -104,10 +173,11 @@ def _write_input(input_path, out_dir):
 
 
 def optimize_orbitals(input_path, out_dir, fixed_list=False, max_macro=10, tol=1.0e-4, max_step=0.5, shift_floor=1.0e-4, max_halvings=8,
-                      state_weights=None, fcidump=None, log=None):
+                      state_weights=None, fcidump=None, log=None, one_step=False):
     """Optimise the orbitals of a chem `hci` input.  Writes out_dir/FCIDUMP (the orbitals of the last macro iteration that ran
-    the CI, columns and irreps as in the original) and a copy of the input as out_dir/<input name>.
-    -> dict(history=[{macro, n_det, energies, energy (weighted), max_grad, step_norm, shift, halvings, seconds}], converged,
+    the CI, columns and irreps as in the original) and a copy of the input as out_dir/<input name>.  one_step implies
+    fixed_list and takes coupled_step's Newton steps; the CI part of the step starts the next Davidson.
+    -> dict(history=[{macro, n_det, energies, energy (weighted), max_grad, step_norm, shift, halvings, micro, seconds}], converged,
     coeffs C (column k = orbital k in the original FCIDUMP orbitals), irreps, system, hamiltonian, up, dn, wts)"""
     from . import ChemSystem, SparseHamiltonian
     say = log or (lambda *_: None)
@@ -137,6 +207,7 @@ def optimize_orbitals(input_path, out_dir, fixed_list=False, max_macro=10, tol=1
         dv = H.davidson_sparse(n_states=ns, initial_vector=w)
         return dict(system=system, H=H, up=up, dn=dn, wts=np.asarray(dv["evecs"]), energy=np.asarray(dv["evals"], dtype=np.float64))
 
+    fixed_list = fixed_list or one_step
     C = np.eye(norb)
     history = []
     converged = False
@@ -148,6 +219,8 @@ def optimize_orbitals(input_path, out_dir, fixed_list=False, max_macro=10, tol=1
             system, H = setup(C)
             res = hci.perform_hci(H, system, cfg["eps_var"], cfg["eps_var_sched"], n_states=ns, eps_pt=None)
             state = dict(system=system, H=H, up=res["up"], dn=res["dn"], wts=res["wts"], energy=np.asarray(res["energy"], dtype=np.float64))
+            if one_step:   # the resident matrix in the order of the carried list, for the H.v of the coupled step
+                H.generate_sparse_ham_upper_triangular(state["up"], state["dn"])
         system, H = state["system"], state["H"]
         der = H.orbital_derivatives(state["up"], state["dn"], state["wts"], state_weights=sw)
         pairs = rotation_parameters(system)
@@ -156,7 +229,7 @@ def optimize_orbitals(input_path, out_dir, fixed_list=False, max_macro=10, tol=1
         grad = der["gradient"][idx_p, idx_q]
         max_g = float(np.max(np.abs(grad))) if len(grad) else 0.0
         entry = dict(macro=macro, n_det=int(len(state["up"])), energies=[float(e) for e in state["energy"]], energy=float(sw @ state["energy"]),
-                     rdm_energy=der["energy"], max_grad=max_g, n_params=len(pairs), step_norm=0.0, shift=0.0, halvings=0)
+                     rdm_energy=der["energy"], max_grad=max_g, n_params=len(pairs), step_norm=0.0, shift=0.0, halvings=0, micro=0)
         if max_g < tol or macro == max_macro - 1:
             converged = max_g < tol
             entry["seconds"] = time.perf_counter() - t0
@@ -164,15 +237,25 @@ def optimize_orbitals(input_path, out_dir, fixed_list=False, max_macro=10, tol=1
             say("orbopt %d: E=%.10f max|g|=%.3e n_det=%d" % (macro, entry["energy"], max_g, entry["n_det"]))
             break
         hess = der["hessian"][idx_p, idx_q][:, idx_p, idx_q]
-        step, shift = newton_step(grad, hess, max_step=max_step, floor=shift_floor)
+        ci_step = None
+        if one_step:
+            wv = np.asarray(state["wts"], dtype=np.float64).reshape(len(state["up"]), -1)
+            step, ci_step, shift, micro = coupled_step(H, state["up"], state["dn"], wv, state["energy"], sw, grad, hess, pairs,
+                                                       max_step=max_step, floor=shift_floor)
+            entry["micro"] = micro
+        else:
+            step, shift = newton_step(grad, hess, max_step=max_step, floor=shift_floor)
         if fixed_list:
             e_prev = entry["energy"]
             while True:
                 U = expm(-kappa_in_fcidump_columns(system, pairs, step))
-                trial = solve_fixed(C @ U, state)
+                start = state if ci_step is None else dict(state, wts=(wv + ci_step).reshape(np.shape(state["wts"])))
+                trial = solve_fixed(C @ U, start)
                 if float(sw @ trial["energy"]) <= e_prev or halvings >= max_halvings:
                     break
                 step = 0.5 * step
+                if ci_step is not None:
+                    ci_step = 0.5 * ci_step
                 halvings += 1
             if float(sw @ trial["energy"]) > e_prev:   # no step lowered the energy: stay, and stop
                 setup(C)
@@ -186,7 +269,7 @@ def optimize_orbitals(input_path, out_dir, fixed_list=False, max_macro=10, tol=1
             C = C @ expm(-kappa_in_fcidump_columns(system, pairs, step))
         entry.update(step_norm=float(np.linalg.norm(step)), shift=shift, halvings=halvings, seconds=time.perf_counter() - t0)
         history.append(entry)
-        say("orbopt %d: E=%.10f max|g|=%.3e |step|=%.3e shift=%.2e halvings=%d n_det=%d"
-            % (macro, entry["energy"], max_g, entry["step_norm"], shift, halvings, entry["n_det"]))
+        say("orbopt %d: E=%.10f max|g|=%.3e |step|=%.3e shift=%.2e halvings=%d micro=%d n_det=%d"
+            % (macro, entry["energy"], max_g, entry["step_norm"], shift, halvings, entry["micro"], entry["n_det"]))
     return dict(history=history, converged=converged, coeffs=C, irreps=np.array(orbsym, dtype=np.int32), system=state["system"],
                 hamiltonian=state["H"], up=state["up"], dn=state["dn"], wts=state["wts"], fcidump=out_fcidump)
