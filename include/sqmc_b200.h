@@ -177,6 +177,24 @@ int sqmc_b200_orbital_gradient_response(sqmc_b200_handle *h, int64_t n, const vo
                                         const double *wts, const double *dwts, int64_t ldw, const double *state_weights,
                                         double *response);
 
+/* ---- ladder images (single-particle Green's function) --------------------------------------------------------------
+ * Images a_{p sigma}|Psi> (create = 0) or a+_{p sigma}|Psi> (create != 0) of state `state` (0-based column of wts, n_states
+ * columns of leading dimension ldw) for every p of orbs[0 .. n_orbs) (library orbital numbering), sigma = spin (0 up, 1 dn).
+ * Phase convention: alpha string first, each string with ascending creators (that of chem_single, permutation_factor and
+ * sqmc_b200_one_rdm): a_{p alpha} carries (-1)^(alpha electrons below p), a_{p beta} (-1)^(N_alpha + beta electrons below p).
+ * time_sym handles: the representatives are expanded first (c/sqrt2 on (u,d), z c/sqrt2 on (d,u)); the images are plain
+ * determinants of the N-1 / N+1 electron space.  *n_out receives the number of determinants of the union of the images;
+ * sqmc_b200_ladder_result then copies that list (16 bytes per determinant, sorted by (up, dn) as unsigned 128-bit labels, no
+ * duplicates) and the n_out x n_orbs coefficient matrix (column j = the image of orbs[j], leading dimension ldc >= n_out).
+ * Every coefficient is written once, so the result is bit-identical across calls and row permutations.  The model tables
+ * are not read: one- and two-word strings of any model work.
+ * Errors: n <= 0, n_states < 1, ldw < n, state outside [0, n_states), spin not 0 / 1, an orbital outside [0, norb) or listed
+ * twice, annihilation from an empty spin string or creation into a full one, the duplicate / time_sym partner checks of
+ * sqmc_b200_one_rdm, nranks > 1. */
+int sqmc_b200_ladder(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw,
+                     int state, int spin, int create, int n_orbs, const int32_t *orbs, int64_t *n_out);
+int sqmc_b200_ladder_result(sqmc_b200_handle *h, void *up_out, void *dn_out, double *coeffs, int64_t ldc);
+
 /* ---- sparse H build --------------------------------------------------------
  * Replaces generate_sparse_ham_chem_upper_triangular (chemistry.f90:7639),
  * its _mpi twin (:8012), generate_sparse_ham_heg_upper_triangular
@@ -283,6 +301,20 @@ int sqmc_b200_exchange_mode(sqmc_b200_handle *h);
  * ritz_log (may be NULL): the values printed as "Iteration, Eigenvalue=" (:1852). */
 int sqmc_b200_lanczos(sqmc_b200_handle *h, const double *v0, double *evec, double *eig3, double tol, int max_iter,
                       int *n_iter_out, double *ritz_log, int ritz_log_cap, int *n_ritz_logged);
+
+/* ---- tridiagonal Lanczos (single-particle Green's function) ---------------------------------------------------------
+ * One Lanczos run on the resident matrix per start vector r (v0: nvec columns of leading dimension ldv >= n, caller row
+ * order): q_0 = v0_r / ||v0_r||, w = H q_j - alpha_j q_j - beta_{j-1} q_{j-1}, then one classical Gram-Schmidt pass of w
+ * against q_0 .. q_j (full reorthogonalisation), beta_j = ||w||, q_{j+1} = w / beta_j.  A run stops after max_steps steps (at
+ * most n) or when beta_j < tol * max|alpha| (the Krylov space is invariant).
+ * alpha, beta: nvec x max_steps (run r at r * max_steps); entries past the run's steps are 0.  beta[j] couples q_j and q_{j+1};
+ * the last one is the norm of the final residual.  overlaps: nvec x max_steps x nvec, <v0_k | q_j> of run r at
+ * (r * max_steps + j) * nvec + k (v0_k as given, not normalised).  steps_out: nvec steps taken.
+ * Start vectors go through the two-vector H.v in pairs; a run's alpha / beta are bit-identical whether it runs alone or in a
+ * pair, and across calls.  Errors: no matrix, nvec < 1, ldv < n, max_steps < 1, tol < 0, a zero start vector, a basis that
+ * does not fit in device memory, nranks > 1. */
+int sqmc_b200_lanczos_tridiagonal(sqmc_b200_handle *h, int nvec, const double *v0, int64_t ldv, int max_steps, double tol, double *alpha,
+                                  double *beta, double *overlaps, int *steps_out);
 
 /* ---- device-resident entry points (used by bench.py for the HBM-resident leg)
  * x_dev/y_dev are device pointers in the library's INTERNAL row order (length n for x,

@@ -23,7 +23,7 @@ SYMBOLS = [
     "sqmc_b200_set_ownership", "sqmc_b200_matvec_local", "sqmc_b200_projector_local", "sqmc_b200_davidson_local",
     "sqmc_b200_last_build_incremental", "sqmc_b200_alloc_stall_ms", "sqmc_b200_register_host", "sqmc_b200_unregister_host", "sqmc_b200_exchange_mode",
     "sqmc_b200_one_rdm", "sqmc_b200_two_rdm", "sqmc_b200_orbital_derivatives", "sqmc_b200_sigma",
-    "sqmc_b200_orbital_gradient_response",
+    "sqmc_b200_orbital_gradient_response", "sqmc_b200_ladder", "sqmc_b200_ladder_result", "sqmc_b200_lanczos_tridiagonal",
 ]
 
 
@@ -68,6 +68,9 @@ def load():
     L.sqmc_b200_orbital_derivatives.argtypes = [vp, i64, vp, vp, i32, vp, i64, vp, vp, vp, vp]
     L.sqmc_b200_sigma.argtypes = [vp, i64, vp, vp, i32, vp, i64, vp, vp]
     L.sqmc_b200_orbital_gradient_response.argtypes = [vp, i64, vp, vp, i32, vp, vp, i64, vp, vp]
+    L.sqmc_b200_ladder.argtypes = [vp, i64, vp, vp, i32, vp, i64, i32, i32, i32, i32, vp, vp]
+    L.sqmc_b200_ladder_result.argtypes = [vp, vp, vp, vp, i64]
+    L.sqmc_b200_lanczos_tridiagonal.argtypes = [vp, i32, vp, i64, i32, dbl, vp, vp, vp, vp]
     L.sqmc_b200_pt2.argtypes = [vp, i64, vp, vp, vp, dbl, dbl, vp, vp]
     L.sqmc_b200_pt2_sample.argtypes = [vp, i64, vp, vp, i64, vp, vp, vp, vp, i32, dbl, dbl, dbl, vp, vp]
     L.sqmc_b200_pt2_alias.argtypes = [vp, i64, vp, vp, vp, dbl, dbl, dbl, i32, dbl, vp, i32, vp, vp, vp, vp, vp]

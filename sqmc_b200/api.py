@@ -412,6 +412,47 @@ class SparseHamiltonian:
                                                           _p(out)))
         return np.ascontiguousarray(out.T)   # (p,q) at p + norb*q
 
+    def ladder(self, dets_up, dets_dn, wts, orbitals, spin, create, state=0):
+        """Images a_{p spin}|Psi> (create False) or a+_{p spin}|Psi> (create True) of the wavefunction wts[:, state] (wts (n,) or
+        (n, n_states); on time_sym systems over the representatives, which are expanded first) for every p of orbitals (library
+        numbering), spin 0 / "a" = up, 1 / "b" = dn.  Phases: alpha string first, ascending creators (those of one_rdm).
+        -> (up', dn', phi): the union of the images as plain N-1 / N+1 electron determinants ((m, 2) uint64, sorted by (up, dn)
+        label, no duplicates) and phi (m, len(orbitals)), column j = the image of orbitals[j] in that list."""
+        up = np.ascontiguousarray(dets_up, dtype=np.uint64).reshape(-1, 2)
+        dn = np.ascontiguousarray(dets_dn, dtype=np.uint64).reshape(-1, 2)
+        w = np.asarray(wts, dtype=np.float64)
+        w = np.asfortranarray(w.reshape(-1, 1) if w.ndim == 1 else w)
+        if len(dn) != len(up) or w.shape[0] != len(up):
+            raise ValueError("ladder: dets_up, dets_dn and wts must have the same number of rows")
+        orbs = np.ascontiguousarray(orbitals, dtype=np.int32).reshape(-1)
+        sp = {"a": 0, "b": 1}.get(spin, spin)
+        nn = C.c_int64()
+        check(self._L.sqmc_b200_ladder(self._h, len(up), _p(up), _p(dn), w.shape[1], _p(w), max(w.shape[0], 1), int(state), int(sp),
+                                       int(bool(create)), len(orbs), _p(orbs), C.byref(nn)))
+        m = nn.value
+        nu = np.zeros((max(m, 1), 2), dtype=np.uint64)
+        nd = np.zeros((max(m, 1), 2), dtype=np.uint64)
+        phi = np.zeros((max(m, 1), len(orbs)), order="F")
+        check(self._L.sqmc_b200_ladder_result(self._h, _p(nu), _p(nd), _p(phi), max(m, 1)))
+        return nu[:m].copy(), nd[:m].copy(), np.ascontiguousarray(phi[:m])
+
+    def lanczos_tridiagonal(self, V0, max_steps, tol=1e-12):
+        """Lanczos with full reorthogonalisation on the resident matrix from each column of V0 ((n,) or (n, nvec), caller row
+        order).  -> dict(alpha (nvec, max_steps), beta (nvec, max_steps): beta[r, j] couples q_j and q_{j+1}, overlaps
+        (nvec, max_steps, nvec): overlaps[r, j, k] = <V0[:, k] | q_j of run r>, steps (nvec,)); entries past a run's steps are 0.
+        A run stops after max_steps steps or when beta_j < tol max|alpha| (its Krylov space is then invariant)."""
+        v = np.asarray(V0, dtype=np.float64)
+        v = np.asfortranarray(v.reshape(-1, 1) if v.ndim == 1 else v)
+        if v.shape[0] != self.n:
+            raise ValueError("lanczos_tridiagonal: V0 has %d rows, the matrix %d" % (v.shape[0], self.n))
+        nv, ms = v.shape[1], int(max_steps)
+        a = np.zeros((nv, max(ms, 1)))
+        b = np.zeros((nv, max(ms, 1)))
+        ov = np.zeros((nv, max(ms, 1), nv))
+        st = np.zeros(nv, dtype=np.int32)
+        check(self._L.sqmc_b200_lanczos_tridiagonal(self._h, nv, _p(v), max(v.shape[0], 1), ms, float(tol), _p(a), _p(b), _p(ov), _p(st)))
+        return dict(alpha=a, beta=b, overlaps=ov, steps=st.astype(np.int64))
+
     def second_order_pt(self, dets_up, dets_dn, wts, var_energy, eps_pt):
         """Deterministic second-order PT with the HCI screened sum (second_order_pt, hci.f90:1100-1182) -> (delta_e_2pt, ndets_connected)."""
         up = np.ascontiguousarray(dets_up, dtype=np.uint64).reshape(-1, 2)

@@ -475,6 +475,18 @@ int sqmc_b200_sigma(sqmc_b200_handle *h, int64_t n, const void *dets_up, const v
   return sigma(h, n, dets_up, dets_dn, n_states, x, ldx, kappa, y);
 }
 
+int sqmc_b200_ladder(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw,
+                     int state, int spin, int create, int n_orbs, const int32_t *orbs, int64_t *n_out) {
+  SQ_CHECK(require_init());
+  if (!h || !dets_up || !dets_dn || !wts || !orbs || !n_out) { set_error("ladder: null argument"); return 2; }
+  return ladder(h, n, dets_up, dets_dn, n_states, wts, ldw, state, spin, create, n_orbs, orbs, n_out);
+}
+
+int sqmc_b200_ladder_result(sqmc_b200_handle *h, void *up_out, void *dn_out, double *coeffs, int64_t ldc) {
+  if (!h || !up_out || !dn_out || !coeffs) { set_error("ladder_result: null argument"); return 2; }
+  return ladder_result(h, up_out, dn_out, coeffs, ldc);
+}
+
 int sqmc_b200_orbital_gradient_response(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts,
                                         const double *dwts, int64_t ldw, const double *state_weights, double *response) {
   SQ_CHECK(require_init());
@@ -530,6 +542,13 @@ int sqmc_b200_lanczos(sqmc_b200_handle *h, const double *v0, double *evec, doubl
   if (!h) { set_error("lanczos: null handle"); return 2; }
   if (max_iter < 1) { set_error("lanczos: max_iter must be positive"); return 2; }
   return lanczos(h, v0, evec, eig3, tol, max_iter, n_iter_out, ritz_log, ritz_log_cap, n_ritz_logged);
+}
+
+int sqmc_b200_lanczos_tridiagonal(sqmc_b200_handle *h, int nvec, const double *v0, int64_t ldv, int max_steps, double tol, double *alpha,
+                                  double *beta, double *overlaps, int *steps_out) {
+  SQ_CHECK(require_init());
+  if (!h || !v0 || !alpha || !beta || !overlaps || !steps_out) { set_error("lanczos_tridiagonal: null argument"); return 2; }
+  return lanczos_tridiagonal(h, nvec, v0, ldv, max_steps, tol, alpha, beta, overlaps, steps_out);
 }
 
 int sqmc_b200_set_row_bundle(sqmc_b200_handle *h, int rows_per_bundle) {

@@ -748,4 +748,169 @@ int lanczos(sqmc_b200_handle *h, const double *v0, double *evec, double *eig3, d
   return 0;
 }
 
+// ------------------------------------------------------------------ tridiagonal Lanczos (Green's functions)
+// For every start vector v0_r: q_0 = v0_r / ||v0_r||, and for j = 0, 1, ...
+//   w = H q_j,  alpha_j = q_j . w,  w -= alpha_j q_j + beta_{j-1} q_{j-1},  w -= Q_j (Q_j^T w)  (one classical Gram-Schmidt pass
+//   against q_0 .. q_j: full reorthogonalisation),  beta_j = ||w||,  q_{j+1} = w / beta_j,
+// until j + 1 = max_steps or beta_j < tol max|alpha| (beta_j = 0 included): the Krylov space is then invariant.
+// Runs go in pairs through the two-vector H.v (one pass over the matrix); every other operation of a run reads only its own
+// vectors, in the fixed order of the two-stage dot products, so a run's alpha / beta do not depend on its partner.  The
+// scalars of the three-term step and of the projection stay on the device; alpha_j and beta_j^2 are fetched once per step
+// for the stopping test.  SQMC_DAV_PROFILE=1 prints the H.v / orthogonalisation split to stderr.
+
+// The two update kernels below subtract in place in one pass over w.  axpy_neg_dev_kernel would take one launch and one read
+// and write of w per basis column (j + 1 passes at step j), and combine_kernel writes a fresh output rather than updating w;
+// the three-term kernel reads beta^2, the value the dot product leaves on the device, so beta never goes through the host.
+// w -= alpha q + sqrt(beta2) q_prev (q_prev null: first step)
+__global__ void lanczos_three_term_kernel(double *w, const double *q, const double *q_prev, const double *alpha, const double *beta2, int64_t n) {
+  const int64_t j = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (j >= n) return;
+  double v = w[j] - (*alpha) * q[j];
+  if (q_prev) v -= sqrt(*beta2) * q_prev[j];
+  w[j] = v;
+}
+// w -= sum_k Q[k*ld + j] c[k], k ascending
+__global__ void project_out_columns_kernel(double *w, const double *__restrict__ Q, int64_t ld, int k, const double *__restrict__ c, int64_t n) {
+  const int64_t j = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (j >= n) return;
+  double acc = 0.0;
+  for (int i = 0; i < k; i++) acc += Q[(int64_t)i * ld + j] * c[i];
+  w[j] -= acc;
+}
+
+int lanczos_tridiagonal(sqmc_b200_handle *h, int nvec, const double *v0, int64_t ldv, int max_steps, double tol, double *alpha, double *beta,
+                        double *overlaps, int *steps_out) {
+  if (G.nranks > 1) { set_error("lanczos_tridiagonal: runs on a single process only (nranks = %d)", G.nranks); return 2; }
+  if (!h->d_rowptr) { set_error("lanczos_tridiagonal: no matrix on this handle"); return 2; }
+  const int64_t n = h->n;
+  if (nvec < 1) { set_error("lanczos_tridiagonal: nvec must be >= 1"); return 2; }
+  if (ldv < n) { set_error("lanczos_tridiagonal: ldv (%lld) must be >= n (%lld)", (long long)ldv, (long long)n); return 2; }
+  if (max_steps < 1) { set_error("lanczos_tridiagonal: max_steps must be >= 1"); return 2; }
+  if (!(tol >= 0.0)) { set_error("lanczos_tridiagonal: tol must be >= 0"); return 2; }
+  const int m = (int)std::min<int64_t>(max_steps, n);  // a Krylov space has at most n dimensions
+  Dav D;
+  D.h = h;
+  D.s = G.stream;
+  D.n = n;
+  D.nloc = n;
+  D.ld = (std::max<int64_t>(n, 1) + 63) / 64 * 64;  // columns start on 512-byte boundaries (texture-path gathers)
+  const int64_t ld = D.ld;
+  cudaStream_t s = D.s;
+  const int npair = std::min(nvec, 2);
+  // every device buffer of the call: V0 (nvec columns), (m + 1) Lanczos columns and 3m + 8 scalars per run of a pair, the
+  // overlaps, the dot partials, and the two interleaved-vector buffers spmv_pair allocates on its first use
+  const bool pair_buffers = nvec >= 2 && h->bundle_R && !h->d_y2;
+  const size_t need = sizeof(double) * ((size_t)ld * ((size_t)nvec + (size_t)npair * (m + 1)) + (size_t)npair * (3 * m + 8) +
+                                        (size_t)m * nvec + (size_t)kDotBlocks * (std::max(m, nvec) + 2) +
+                                        (pair_buffers ? (size_t)4 * std::max<int64_t>(n, 1) : 0));
+  {
+    size_t fr = 0, tot = 0;
+    SQ_CUDA(cudaMemGetInfo(&fr, &tot));
+    size_t cached = 0;
+    cudaMemPool_t pool;
+    if (cudaDeviceGetDefaultMemPool(&pool, G.device) == cudaSuccess) {
+      uint64_t res = 0, used = 0;
+      if (cudaMemPoolGetAttribute(pool, cudaMemPoolAttrReservedMemCurrent, &res) == cudaSuccess &&
+          cudaMemPoolGetAttribute(pool, cudaMemPoolAttrUsedMemCurrent, &used) == cudaSuccess && res > used)
+        cached = (size_t)(res - used);
+    }
+    if (need > fr + cached) {
+      set_error("lanczos_tridiagonal: the Krylov basis needs %.2f GB (%d start vectors + %d runs x %d vectors of %lld doubles, with work buffers) but "
+                "%.2f GB of device memory is free; lower max_steps",
+                need / 1e9, nvec, npair, m + 1, (long long)n, (fr + cached) / 1e9);
+      return 2;
+    }
+  }
+  double *V0 = nullptr, *Q[2] = {nullptr, nullptr}, *sc[2] = {nullptr, nullptr}, *ov = nullptr;
+  struct Free {
+    std::vector<double *> p;
+    ~Free() {
+      for (double *q : p)
+        if (q) devbuf_free(q);
+    }
+  } fr;
+  SQ_CHECK(devbuf_alloc((void **)&V0, (size_t)ld * nvec * sizeof(double)));
+  fr.p.push_back(V0);
+  for (int r = 0; r < npair; r++) {
+    SQ_CHECK(devbuf_alloc((void **)&Q[r], (size_t)ld * (m + 1) * sizeof(double)));
+    fr.p.push_back(Q[r]);
+    SQ_CHECK(devbuf_alloc((void **)&sc[r], (size_t)(3 * m + 8) * sizeof(double)));  // [alpha_j, beta_j^2] pairs | projection coefficients
+    fr.p.push_back(sc[r]);
+  }
+  SQ_CHECK(devbuf_alloc((void **)&ov, (size_t)m * nvec * sizeof(double)));
+  fr.p.push_back(ov);
+  SQ_CHECK(devbuf_alloc((void **)&D.partial, (size_t)kDotBlocks * (std::max(m, nvec) + 2) * sizeof(double)));
+  SQ_CHECK(pinned_scratch(&D.h_scal, (size_t)((int64_t)m * nvec + 8) * sizeof(double)));
+  SQ_CUDA(cudaMemsetAsync(V0, 0, (size_t)ld * nvec * sizeof(double), s));
+  std::vector<double> norm2(nvec);
+  for (int r = 0; r < nvec; r++) {
+    SQ_CHECK(load_block(h, v0 + (int64_t)r * ldv, false, V0 + (int64_t)r * ld, s));
+    SQ_CHECK(D.dots(V0 + (int64_t)r * ld, 1, V0 + (int64_t)r * ld, sc[0]));
+    SQ_CHECK(D.fetch(sc[0], 1, &norm2[r]));
+    if (!(norm2[r] > 0.0)) { set_error("lanczos_tridiagonal: start vector %d has zero norm", r); return 2; }
+  }
+  for (int r = 0; r < nvec; r++)
+    for (int j = 0; j < max_steps; j++) {
+      alpha[(int64_t)r * max_steps + j] = 0.0;
+      beta[(int64_t)r * max_steps + j] = 0.0;
+    }
+  PhaseTimer PT(s);
+  for (int r0 = 0; r0 < nvec; r0 += 2) {
+    const int nr = std::min(2, nvec - r0);
+    int steps[2] = {0, 0};
+    bool active[2] = {false, false};
+    double amax[2] = {0.0, 0.0};
+    auto q = [&](int r, int j) { return Q[r] + (int64_t)j * ld; };
+    for (int r = 0; r < nr; r++) {
+      SQ_CUDA(cudaMemcpyAsync(q(r, 0), V0 + (int64_t)(r0 + r) * ld, n * sizeof(double), cudaMemcpyDeviceToDevice, s));
+      SQ_CHECK(D.dots(q(r, 0), 1, q(r, 0), sc[r]));
+      SQ_CHECK(D.normalize(q(r, 0), sc[r]));
+      active[r] = true;
+    }
+    for (int j = 0; j < m && (active[0] || active[1]); j++) {
+      PT.start();
+      if (active[0] && active[1]) {
+        SQ_CHECK(spmv_pair(h, q(0, j), q(1, j), q(0, j + 1), q(1, j + 1), s));
+      } else {
+        const int r = active[0] ? 0 : 1;
+        SQ_CHECK(spmv_block(h, q(r, j), q(r, j + 1), s));
+      }
+      PT.stop(0);
+      PT.start();
+      for (int r = 0; r < nr; r++) {
+        if (!active[r]) continue;
+        double *w = q(r, j + 1), *a = sc[r] + 2 * j, *b2 = a + 1, *c = sc[r] + 2 * m + 4;
+        SQ_CHECK(D.dots(q(r, j), 1, w, a));
+        lanczos_three_term_kernel<<<D.blocks(n), 256, 0, s>>>(w, q(r, j), j > 0 ? q(r, j - 1) : nullptr, a, j > 0 ? a - 1 : nullptr, n);
+        SQ_LAUNCH_CHECK();
+        SQ_CHECK(D.dots(Q[r], j + 1, w, c));
+        project_out_columns_kernel<<<D.blocks(n), 256, 0, s>>>(w, Q[r], ld, j + 1, c, n);
+        SQ_LAUNCH_CHECK();
+        SQ_CHECK(D.dots(w, 1, w, b2));
+        double ab[2];
+        SQ_CHECK(D.fetch(a, 2, ab));
+        const int64_t o = (int64_t)(r0 + r) * max_steps + j;
+        alpha[o] = ab[0];
+        beta[o] = sqrt(ab[1]);
+        amax[r] = std::max(amax[r], fabs(ab[0]));
+        steps[r] = j + 1;
+        if (beta[o] < tol * amax[r] || beta[o] == 0.0 || j + 1 == m) active[r] = false;
+        else SQ_CHECK(D.normalize(w, b2));
+      }
+      PT.stop(1);
+    }
+    // overlaps <v0_k | q_j> of every start vector with this pair's Lanczos vectors
+    for (int r = 0; r < nr; r++) {
+      for (int j = 0; j < steps[r]; j++) SQ_CHECK(D.dots(V0, nvec, q(r, j), ov + (int64_t)j * nvec));
+      SQ_CHECK(D.fetch(ov, steps[r] * nvec, overlaps + (int64_t)(r0 + r) * max_steps * nvec));
+      for (int64_t k = (int64_t)steps[r] * nvec; k < (int64_t)max_steps * nvec; k++) overlaps[(int64_t)(r0 + r) * max_steps * nvec + k] = 0.0;
+      steps_out[r0 + r] = steps[r];
+    }
+  }
+  if (PT.on)
+    fprintf(stderr, "[sqmc_b200 lanczos_tridiagonal] n=%lld runs=%d  H.v %.3f ms | orthogonalisation %.3f ms\n", (long long)n, nvec, PT.acc[0] * 1e3,
+            PT.acc[1] * 1e3);
+  return 0;
+}
+
 }  // namespace sqmc

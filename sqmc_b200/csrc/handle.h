@@ -190,6 +190,10 @@ struct sqmc_b200_handle {
   // ---- heat-bath selection (select.cu) ----
   int32_t *d_orbsym = nullptr;        // [norb] orbital irreps (chem), set by sqmc_b200_system_orbital_symmetries
   std::vector<uint64_t> sel_new_up, sel_new_dn;  // result of the last hci_select (host, 16 B per det)
+  // ---- ladder images (rdm.cu): result of the last sqmc_b200_ladder (host; 16 B per det, coefficients n x lad_norbs column-major)
+  std::vector<uint64_t> lad_up, lad_dn;
+  std::vector<double> lad_coef;
+  int lad_norbs = 0;
   // heat-bath tables of the chem double excitations (norb <= 64): per hole pair (p,q) -- row p*norb+q -- the particle
   // pairs (r,s) packed r | s<<8, sorted by decreasing |H|; [0] same spin (p<q, r<s), [1] opposite spin (p,r up; q,s dn)
   double *d_hb_val[2] = {nullptr, nullptr};
@@ -276,6 +280,8 @@ int davidson_single(sqmc_b200_handle *h, const double *v0, double *evec, double 
                     int ritz_log_cap, int *n_ritz_logged);
 int lanczos(sqmc_b200_handle *h, const double *v0, double *evec, double *eig3, double tol, int max_iter, int *n_iter_out, double *ritz_log,
             int ritz_log_cap, int *n_ritz_logged);
+int lanczos_tridiagonal(sqmc_b200_handle *h, int nvec, const double *v0, int64_t ldv, int max_steps, double tol, double *alpha, double *beta,
+                        double *overlaps, int *steps_out);
 // rdm.cu
 int one_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw, double *rdm);
 int two_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw, double *rdm2);
@@ -285,4 +291,7 @@ int sigma(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_
           const double *kappa, double *y);
 int orbital_gradient_response(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts,
                               const double *dwts, int64_t ldw, const double *state_weights, double *response);
+int ladder(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw, int state, int spin,
+           int create, int n_orbs, const int32_t *orbs, int64_t *n_out);
+int ladder_result(sqmc_b200_handle *h, void *up_out, void *dn_out, double *coeffs, int64_t ldc);
 }  // namespace sqmc

@@ -1,4 +1,5 @@
-// rdm.cu -- one- and two-particle density matrices of variational wavefunctions (sqmc_b200_one_rdm, sqmc_b200_two_rdm).
+// rdm.cu -- one- and two-particle density matrices of variational wavefunctions (sqmc_b200_one_rdm, sqmc_b200_two_rdm), the
+// orbital-optimisation quantities built on them, and the ladder images a_p|Psi>, a+_p|Psi> of the Green's function (sqmc_b200_ladder).
 //
 //   rdm[s][sigma](p,q) = <Psi_s| a+_{p sigma} a_{q sigma} |Psi_s>,   Psi_s = sum_i wts(i,s) |D_i>
 //
@@ -1490,6 +1491,219 @@ int orbital_gradient_response(sqmc_b200_handle *h, int64_t n, const void *dets_u
   SQ_CHECK(orbital_check_args(h, "orbital_gradient_response", n, n_states, ldw));
   SQ_CHECK(state_weights_check("orbital_gradient_response", n_states, state_weights));
   return orbital_gradient_response_impl(h, n, dets_up, dets_dn, n_states, wts, dwts, ldw, state_weights, response);
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// ladder images (sqmc_b200_ladder / sqmc_b200_ladder_result): a_{p sigma}|Psi> or a+_{p sigma}|Psi> for every p of a list
+//
+// Determinant phase convention: the alpha string first, each string with ascending creators (chem_single,
+// permutation_factor, one_rdm).  a_{p alpha} and a+_{p alpha} carry (-1)^(alpha electrons below p); the beta operators carry
+// (-1)^(N_alpha + beta electrons below p).
+//
+// Every determinant of the sorted view 0 of prepare_dets (time_sym lists expanded) emits one candidate per orbital into slot
+// i * P + j.  For a fixed orbital the map D -> a_p D is injective, so a column never receives two values; the same image
+// reached from several orbitals is one row of the union.  The valid candidates are compacted in slot order, sorted by
+// (up, dn) with the stable radix sort of sort_pairs_index, and the first entry of each run of equal determinants opens a
+// row.  Each coefficient is then written to (row, column) exactly once: no sums, so the result does not depend on the
+// caller's row order or on scheduling.
+template <int NW>
+__global__ void ladder_candidates_kernel(const uint64_t *up, const uint64_t *dn, const double *c, int64_t n, const int32_t *orbs, int P, int spin,
+                                         int create, uint64_t *iu, uint64_t *id, double *iv, int32_t *ok) {
+  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (t >= n * P) return;
+  const int64_t i = t / P;
+  const int p = orbs[t - i * P];
+  const Bits<NW> U = b_load<NW>(up, i), D = b_load<NW>(dn, i);
+  Bits<NW> x = spin ? D : U;
+  const bool occ = b_test(x, p);
+  ok[t] = occ != (create != 0);
+  const int par = b_popc(b_and(x, b_maskr<NW>(p))) + (spin ? b_popc(U) : 0);
+  if (create) b_set(x, p);
+  else b_clear(x, p);
+  b_store(iu, t, spin ? U : x);
+  b_store(id, t, spin ? x : D);
+  iv[t] = (par & 1) ? -c[i] : c[i];
+}
+
+// first entry of each run of equal (up, dn) in a sorted list
+template <int NW>
+__global__ void run_head_kernel(const uint64_t *u, const uint64_t *d, int64_t m, int32_t *head) {
+  const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (k >= m) return;
+  head[k] = (k == 0 || !b_eq(b_load<NW>(u, k), b_load<NW>(u, k - 1)) || !b_eq(b_load<NW>(d, k), b_load<NW>(d, k - 1))) ? 1 : 0;
+}
+
+// coef[row(k) + nout * col(k)] = value of sorted candidate k; row(k) = inclusive head count - 1
+__global__ void ladder_scatter_kernel(const int32_t *sel, const int32_t *order, const int32_t *row_incl, const double *iv, int64_t m, int P, int64_t nout,
+                                      double *coef) {
+  const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (k >= m) return;
+  const int32_t slot = sel[order[k]];
+  coef[(int64_t)(row_incl[k] - 1) + nout * (slot % P)] = iv[slot];
+}
+
+// strings of NW words -> the 16-byte host layout (two words per determinant)
+template <int NW>
+__global__ void widen_strings_kernel(const uint64_t *src, int64_t n, uint64_t *dst) {
+  const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  dst[2 * k] = src[k * NW];
+  dst[2 * k + 1] = NW == 2 ? src[k * NW + 1] : 0ull;
+}
+
+// indices k < n with flag[k] != 0, in ascending order -> sel (device), count (host)
+static int select_flagged(const int32_t *flag, int64_t n, DevBuf<int32_t> &sel, int64_t &count, cudaStream_t s) {
+  SQ_CHECK(sel.alloc(std::max<int64_t>(n, 1)));
+  DevBuf<int> nsel;
+  SQ_CHECK(nsel.alloc(1));
+  thrust::counting_iterator<int32_t> rows(0);
+  size_t tb = 0;
+  cub::DeviceSelect::Flagged(nullptr, tb, rows, flag, sel.p, nsel.p, (int)n, s);
+  DevBuf<char> tmp;
+  SQ_CHECK(tmp.alloc((int64_t)tb + 16));
+  SQ_CUDA(cub::DeviceSelect::Flagged(tmp.p, tb, rows, flag, sel.p, nsel.p, (int)n, s));
+  g_launch_count += 1;
+  int m = 0;
+  SQ_CUDA(cudaMemcpyAsync(&m, nsel.p, sizeof(int), cudaMemcpyDeviceToHost, s));
+  SQ_CUDA(cudaStreamSynchronize(s));
+  count = m;
+  return 0;
+}
+
+template <int NW>
+static int ladder_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, const double *w_state, int64_t ldw, int spin, int create,
+                       int P, const int32_t *orbs, int64_t *n_out) {
+  cudaStream_t s = G.stream;
+  const int norb = h->T.norb;
+  DevBuf<uint64_t> up, dn, ma0, mi0;
+  DevBuf<double> w, c0;
+  DevBuf<int32_t> idx0;
+  int64_t n2 = 0;
+  SQ_CHECK(prepare_dets<NW>(h, "ladder", n, dets_up, dets_dn, 1, w_state, ldw, up, dn, w, n2, idx0, ma0, mi0, c0));
+  up.release(); dn.release(); w.release(); idx0.release();
+  const int64_t nc = n2 * P;
+  if (nc > INT32_MAX) { set_error("ladder: %lld determinants x %d orbitals exceed the 32-bit candidate index", (long long)n2, P); return 2; }
+  DevBuf<int32_t> d_orbs, ok, sel;
+  DevBuf<uint64_t> iu, id;
+  DevBuf<double> iv;
+  SQ_CHECK(d_orbs.alloc(P));
+  SQ_CUDA(cudaMemcpyAsync(d_orbs.p, orbs, P * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+  SQ_CHECK(iu.alloc(nc * NW));
+  SQ_CHECK(id.alloc(nc * NW));
+  SQ_CHECK(iv.alloc(nc));
+  SQ_CHECK(ok.alloc(nc));
+  ladder_candidates_kernel<NW><<<(unsigned)div_up(nc, 256), 256, 0, s>>>(ma0.p, mi0.p, c0.p, n2, d_orbs.p, P, spin, create, iu.p, id.p, iv.p, ok.p);
+  SQ_LAUNCH_CHECK();
+  ma0.release(); mi0.release(); c0.release();
+  int64_t m = 0;
+  SQ_CHECK(select_flagged(ok.p, nc, sel, m, s));
+  ok.release();
+  h->lad_up.clear();
+  h->lad_dn.clear();
+  h->lad_coef.clear();
+  h->lad_norbs = P;
+  *n_out = 0;
+  if (m == 0) return 0;
+  // valid candidates in slot order, then sorted by (up, dn)
+  DevBuf<uint64_t> cu, cd, su, sd;
+  DevBuf<int32_t> order;
+  SQ_CHECK(cu.alloc(m * NW));
+  SQ_CHECK(cd.alloc(m * NW));
+  SQ_CHECK(gather_strings(NW, iu.p, sel.p, cu.p, m, s));
+  SQ_CHECK(gather_strings(NW, id.p, sel.p, cd.p, m, s));
+  iu.release(); id.release();
+  SQ_CHECK(order.alloc(m));
+  SQ_CHECK(sort_pairs_index(NW, norb, cu.p, cd.p, order.p, m, s));
+  SQ_CHECK(su.alloc(m * NW));
+  SQ_CHECK(sd.alloc(m * NW));
+  SQ_CHECK(gather_strings(NW, cu.p, order.p, su.p, m, s));
+  SQ_CHECK(gather_strings(NW, cd.p, order.p, sd.p, m, s));
+  cu.release(); cd.release();
+  DevBuf<int32_t> head, row;
+  SQ_CHECK(head.alloc(m));
+  SQ_CHECK(row.alloc(m));
+  run_head_kernel<NW><<<(unsigned)div_up(m, 256), 256, 0, s>>>(su.p, sd.p, m, head.p);
+  SQ_LAUNCH_CHECK();
+  {
+    size_t tb = 0;
+    cub::DeviceScan::InclusiveSum(nullptr, tb, head.p, row.p, (int)m, s);
+    DevBuf<char> tmp;
+    SQ_CHECK(tmp.alloc((int64_t)tb + 16));
+    SQ_CUDA(cub::DeviceScan::InclusiveSum(tmp.p, tb, head.p, row.p, (int)m, s));
+    g_launch_count += 1;
+  }
+  int32_t nout32 = 0;
+  SQ_CUDA(cudaMemcpyAsync(&nout32, row.p + (m - 1), sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+  SQ_CUDA(cudaStreamSynchronize(s));
+  const int64_t nout = nout32;
+  DevBuf<double> coef;
+  SQ_CHECK(coef.alloc(nout * P));
+  SQ_CUDA(cudaMemsetAsync(coef.p, 0, nout * P * sizeof(double), s));
+  ladder_scatter_kernel<<<(unsigned)div_up(m, 256), 256, 0, s>>>(sel.p, order.p, row.p, iv.p, m, P, nout, coef.p);
+  SQ_LAUNCH_CHECK();
+  // the union: the head of every run, widened to the 16-byte layout
+  DevBuf<int32_t> heads;
+  int64_t nh = 0;
+  SQ_CHECK(select_flagged(head.p, m, heads, nh, s));
+  DevBuf<uint64_t> ou, od, wide;
+  SQ_CHECK(ou.alloc(nout * NW));
+  SQ_CHECK(od.alloc(nout * NW));
+  SQ_CHECK(gather_strings(NW, su.p, heads.p, ou.p, nout, s));
+  SQ_CHECK(gather_strings(NW, sd.p, heads.p, od.p, nout, s));
+  SQ_CHECK(wide.alloc(2 * nout));
+  h->lad_up.resize(2 * nout);
+  h->lad_dn.resize(2 * nout);
+  h->lad_coef.resize(nout * P);
+  widen_strings_kernel<NW><<<(unsigned)div_up(nout, 256), 256, 0, s>>>(ou.p, nout, wide.p);
+  SQ_LAUNCH_CHECK();
+  SQ_CUDA(cudaMemcpyAsync(h->lad_up.data(), wide.p, 2 * nout * sizeof(uint64_t), cudaMemcpyDeviceToHost, s));
+  SQ_CUDA(cudaStreamSynchronize(s));
+  widen_strings_kernel<NW><<<(unsigned)div_up(nout, 256), 256, 0, s>>>(od.p, nout, wide.p);
+  SQ_LAUNCH_CHECK();
+  SQ_CUDA(cudaMemcpyAsync(h->lad_dn.data(), wide.p, 2 * nout * sizeof(uint64_t), cudaMemcpyDeviceToHost, s));
+  SQ_CUDA(cudaMemcpyAsync(h->lad_coef.data(), coef.p, nout * P * sizeof(double), cudaMemcpyDeviceToHost, s));
+  SQ_CUDA(cudaStreamSynchronize(s));
+  *n_out = nout;
+  return 0;
+}
+
+int ladder(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw, int state, int spin,
+           int create, int n_orbs, const int32_t *orbs, int64_t *n_out) {
+  h->lad_up.clear();
+  h->lad_dn.clear();
+  h->lad_coef.clear();
+  h->lad_norbs = 0;
+  if (G.nranks > 1) { set_error("ladder: runs on a single process only (nranks = %d)", G.nranks); return 2; }
+  if (n <= 0) { set_error("ladder: n must be positive"); return 2; }
+  if (n > INT32_MAX) { set_error("ladder: n exceeds the 32-bit row index"); return 2; }
+  if (n_states < 1) { set_error("ladder: n_states must be >= 1"); return 2; }
+  if (ldw < n) { set_error("ladder: ldw (%lld) must be >= n (%lld)", (long long)ldw, (long long)n); return 2; }
+  if (state < 0 || state >= n_states) { set_error("ladder: state %d is not in [0, %d)", state, n_states); return 2; }
+  if (spin != 0 && spin != 1) { set_error("ladder: spin must be 0 (up) or 1 (dn), got %d", spin); return 2; }
+  if (n_orbs < 1) { set_error("ladder: n_orbs must be >= 1"); return 2; }
+  const int norb = h->T.norb;
+  std::vector<char> seen(norb, 0);
+  for (int j = 0; j < n_orbs; j++) {
+    if (orbs[j] < 0 || orbs[j] >= norb) { set_error("ladder: orbital %d is not in [0, %d)", orbs[j], norb); return 2; }
+    if (seen[orbs[j]]) { set_error("ladder: orbital %d is listed twice", orbs[j]); return 2; }
+    seen[orbs[j]] = 1;
+  }
+  const int nspin = spin ? h->T.ndn : h->T.nup;
+  if (!create && nspin == 0) { set_error("ladder: cannot annihilate from an empty %s string", spin ? "dn" : "up"); return 2; }
+  if (create && nspin == norb) { set_error("ladder: cannot create into a full %s string", spin ? "dn" : "up"); return 2; }
+  const double *w_state = wts + (int64_t)state * ldw;
+  return h->NW == 1 ? ladder_impl<1>(h, n, dets_up, dets_dn, w_state, ldw, spin, create, n_orbs, orbs, n_out)
+                    : ladder_impl<2>(h, n, dets_up, dets_dn, w_state, ldw, spin, create, n_orbs, orbs, n_out);
+}
+
+int ladder_result(sqmc_b200_handle *h, void *up_out, void *dn_out, double *coeffs, int64_t ldc) {
+  const int64_t nout = (int64_t)h->lad_up.size() / 2, P = h->lad_norbs;
+  if (ldc < nout) { set_error("ladder_result: ldc (%lld) must be >= the number of images (%lld)", (long long)ldc, (long long)nout); return 2; }
+  if (nout == 0) return 0;
+  memcpy(up_out, h->lad_up.data(), h->lad_up.size() * sizeof(uint64_t));
+  memcpy(dn_out, h->lad_dn.data(), h->lad_dn.size() * sizeof(uint64_t));
+  for (int64_t j = 0; j < P; j++) memcpy(coeffs + j * ldc, h->lad_coef.data() + j * nout, nout * sizeof(double));
+  return 0;
 }
 
 }  // namespace sqmc

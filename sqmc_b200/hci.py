@@ -9,8 +9,8 @@ Loop rules restated from the reference (hci.f90:359-517; do_walk.f90:418-533):
     or after 50 iterations (:89);
   * Davidson starts from the previous vectors padded with zeros, from unit vectors in iteration 1 (:453-485);
   * PT per state: second_order_pt with eps_pt on the final wavefunction (do_pt, :4220-4243).
-Out of scope here: active spaces, Green's functions, stochastic PT (n_mc > 0, eps_pt_big).  Natural orbitals of the final
-wavefunction: natorb.py and scripts/natorb.py.
+Out of scope here: active spaces, stochastic PT (n_mc > 0, eps_pt_big).  Natural orbitals of the final wavefunction:
+natorb.py and scripts/natorb.py; its single-particle Green's function: greens.py and scripts/greens.py.
 """
 import re
 
