@@ -137,6 +137,26 @@ int sqmc_b200_one_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const
 int sqmc_b200_two_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states,
                       const double *wts, int64_t ldw, double *rdm2);
 
+/* ---- transition density matrices -----------------------------------------------------------------------------------
+ * One- and two-particle transition density matrices between pairs of vectors over one determinant list:
+ *   tdm[k][sigma](p,q)        = <bra_k| a+_{p sigma} a_{q sigma} |ket_k>
+ *   tdm2[k][b](p,q,r,s')      = <bra_k| a+_{p sigma} a+_{r tau} a_{s' tau} a_{q sigma} |ket_k>,   b = 0 (aa), 1 (ab), 2 (bb)
+ * bra, ket: n x n_pairs each, column-major with leading dimension ldw >= n; pair k is (column k of bra, column k of ket).  The
+ * vectors are arbitrary (not normalised, not made orthogonal); pass state I as bra and state J as ket for <I| . |J>.
+ * The output layouts are those of sqmc_b200_one_rdm / sqmc_b200_two_rdm with "state" read as "pair"; so are the orbital
+ * numbering, the phase convention (alpha string first), time_sym handling (both vectors over the representatives, expanded
+ * with the same factors), the duplicate and partner checks, the errors (n_pairs in place of n_states), the models covered and
+ * "no communication on a multi-rank handle".  The 2-TDM needs norb <= 64, the 1-TDM has no such limit.
+ * Bit-for-bit properties: T(ket, bra) is the Hermitian transpose of T(bra, ket) ((p,q) -> (q,p) for the 1-TDM,
+ * (p,q,r,s') -> (q,p,s',r) for the 2-TDM); T(c, c) equals sqmc_b200_one_rdm / sqmc_b200_two_rdm of c; the result is identical
+ * across calls and across permutations of the rows.  In the same-spin blocks Gamma_{pq,rs} = Gamma_{rs,pq} = -Gamma_{ps,rq} and
+ * Gamma = 0 for p = r or q = s still hold exactly; Gamma_{pq,rs} = Gamma_{qp,sr} does not hold for a transition density.
+ * With them, <bra|H|ket> = E_core <bra|ket> + sum h tdm + 1/2 sum (pq|rs) tdm2 and <bra|ket> = trace(tdm) / N. */
+int sqmc_b200_transition_one_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_pairs,
+                                 const double *bra, const double *ket, int64_t ldw, double *tdm);
+int sqmc_b200_transition_two_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_pairs,
+                                 const double *bra, const double *ket, int64_t ldw, double *tdm2);
+
 /* ---- orbital gradient and Hessian (orbital optimisation) ------------------------------------------------------------
  * Derivatives at kappa = 0 of the state-averaged variational energy E(kappa) = E_core + sum h'D + 1/2 sum g'd under a real orbital
  * rotation kappa = sum_{p>q} k_pq (E_pq - E_qp) (Helgaker, Jorgensen, Olsen, 10.8.1), chem handles only, norb <= 64:

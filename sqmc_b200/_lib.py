@@ -24,6 +24,7 @@ SYMBOLS = [
     "sqmc_b200_last_build_incremental", "sqmc_b200_alloc_stall_ms", "sqmc_b200_register_host", "sqmc_b200_unregister_host", "sqmc_b200_exchange_mode",
     "sqmc_b200_one_rdm", "sqmc_b200_two_rdm", "sqmc_b200_orbital_derivatives", "sqmc_b200_sigma",
     "sqmc_b200_orbital_gradient_response", "sqmc_b200_ladder", "sqmc_b200_ladder_result", "sqmc_b200_lanczos_tridiagonal",
+    "sqmc_b200_transition_one_rdm", "sqmc_b200_transition_two_rdm",
 ]
 
 
@@ -65,6 +66,8 @@ def load():
     L.sqmc_b200_set_row_bundle.argtypes = [vp, i32]
     L.sqmc_b200_one_rdm.argtypes = [vp, i64, vp, vp, i32, vp, i64, vp]
     L.sqmc_b200_two_rdm.argtypes = [vp, i64, vp, vp, i32, vp, i64, vp]
+    L.sqmc_b200_transition_one_rdm.argtypes = [vp, i64, vp, vp, i32, vp, vp, i64, vp]
+    L.sqmc_b200_transition_two_rdm.argtypes = [vp, i64, vp, vp, i32, vp, vp, i64, vp]
     L.sqmc_b200_orbital_derivatives.argtypes = [vp, i64, vp, vp, i32, vp, i64, vp, vp, vp, vp]
     L.sqmc_b200_sigma.argtypes = [vp, i64, vp, vp, i32, vp, i64, vp, vp]
     L.sqmc_b200_orbital_gradient_response.argtypes = [vp, i64, vp, vp, i32, vp, vp, i64, vp, vp]

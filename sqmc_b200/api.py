@@ -336,6 +336,46 @@ class SparseHamiltonian:
         out = np.ascontiguousarray(out.transpose(0, 1, 5, 4, 3, 2))
         return out[0] if one else out
 
+    def _transition_args(self, who, dets_up, dets_dn, bra, ket):
+        up = np.ascontiguousarray(dets_up, dtype=np.uint64).reshape(-1, 2)
+        dn = np.ascontiguousarray(dets_dn, dtype=np.uint64).reshape(-1, 2)
+        a = np.asarray(bra, dtype=np.float64)
+        b = np.asarray(ket, dtype=np.float64)
+        if a.shape != b.shape or a.ndim not in (1, 2):
+            raise ValueError("%s: bra and ket must both be (n,) or (n, n_pairs) of the same shape, not %s and %s" % (who, a.shape, b.shape))
+        one = a.ndim == 1
+        a = np.asfortranarray(a.reshape(-1, 1) if one else a)
+        b = np.asfortranarray(b.reshape(-1, 1) if one else b)
+        if len(dn) != len(up) or a.shape[0] != len(up):
+            raise ValueError("%s: dets_up, dets_dn, bra and ket must have the same number of rows" % who)
+        return up, dn, a, b, one
+
+    def transition_one_rdm(self, dets_up, dets_dn, bra, ket):
+        """One-particle transition density matrices <bra_k| a+_{p sigma} a_{q sigma} |ket_k> over the determinant list, bra and ket
+        (n,) or (n, n_pairs) of the same shape (column k of each forms pair k; any vectors, no normalisation or orthogonalisation).
+        Orbital numbering, time_sym handling and errors are those of one_rdm; transition_one_rdm(c, c) is one_rdm(c) bit for bit
+        and transition_one_rdm(b, a) is the (p, q) transpose of transition_one_rdm(a, b).
+        -> float64 array [k, sigma, p, q] of shape (n_pairs, 2, norb, norb); (2, norb, norb) for 1-D bra and ket."""
+        up, dn, a, b, one = self._transition_args("transition_one_rdm", dets_up, dets_dn, bra, ket)
+        norb, npair = self.system.norb, a.shape[1]
+        out = np.zeros((npair, 2, norb, norb))
+        check(self._L.sqmc_b200_transition_one_rdm(self._h, len(up), _p(up), _p(dn), npair, _p(a), _p(b), max(a.shape[0], 1), _p(out)))
+        out = np.ascontiguousarray(out.transpose(0, 1, 3, 2))   # (p,q) at p + norb*q, as in one_rdm
+        return out[0] if one else out
+
+    def transition_two_rdm(self, dets_up, dets_dn, bra, ket):
+        """Two-particle transition density matrices <bra_k| a+_{p s} a+_{r t} a_{s t} a_{q s} |ket_k> (chemists' order, blocks aa, ab,
+        bb as in two_rdm) for the pairs of transition_one_rdm; norb <= 64.  transition_two_rdm(c, c) is two_rdm(c) bit for bit and
+        transition_two_rdm(b, a)[.., p, q, r, s] is transition_two_rdm(a, b)[.., q, p, s, r].  rdm.rdm_energy and rdm.spin_squared
+        of the pair's matrices give <bra|H|ket> and <bra|S^2|ket>.
+        -> float64 array [k, b, p, q, r, s] of shape (n_pairs, 3, norb, norb, norb, norb); (3, norb, ...) for 1-D bra and ket."""
+        up, dn, a, b, one = self._transition_args("transition_two_rdm", dets_up, dets_dn, bra, ket)
+        norb, npair = self.system.norb, a.shape[1]
+        out = np.zeros((npair, 3) + (norb,) * 4) if norb <= 64 else np.zeros(1)   # the library rejects norb > 64
+        check(self._L.sqmc_b200_transition_two_rdm(self._h, len(up), _p(up), _p(dn), npair, _p(a), _p(b), max(a.shape[0], 1), _p(out)))
+        out = np.ascontiguousarray(out.transpose(0, 1, 5, 4, 3, 2))
+        return out[0] if one else out
+
     def orbital_derivatives(self, dets_up, dets_dn, wts, state_weights=None):
         """Orbital gradient and Hessian at kappa = 0 of the state-averaged variational energy
         E(kappa) = E_core + sum h'D + 1/2 sum g'd, h' = U^T h U and (pq|rs)' rotated alike (natorb.rotate_fcidump with C = U),

@@ -458,6 +458,20 @@ int sqmc_b200_two_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const
   return two_rdm(h, n, dets_up, dets_dn, n_states, wts, ldw, rdm2);
 }
 
+int sqmc_b200_transition_one_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_pairs, const double *bra,
+                                 const double *ket, int64_t ldw, double *tdm) {
+  SQ_CHECK(require_init());
+  if (!h || !dets_up || !dets_dn || !bra || !ket || !tdm) { set_error("transition_one_rdm: null argument"); return 2; }
+  return transition_one_rdm(h, n, dets_up, dets_dn, n_pairs, bra, ket, ldw, tdm);
+}
+
+int sqmc_b200_transition_two_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_pairs, const double *bra,
+                                 const double *ket, int64_t ldw, double *tdm2) {
+  SQ_CHECK(require_init());
+  if (!h || !dets_up || !dets_dn || !bra || !ket || !tdm2) { set_error("transition_two_rdm: null argument"); return 2; }
+  return transition_two_rdm(h, n, dets_up, dets_dn, n_pairs, bra, ket, ldw, tdm2);
+}
+
 int sqmc_b200_orbital_derivatives(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts,
                                   int64_t ldw, const double *state_weights, double *fock, double *hessian, double *energy) {
   SQ_CHECK(require_init());

@@ -285,6 +285,10 @@ int lanczos_tridiagonal(sqmc_b200_handle *h, int nvec, const double *v0, int64_t
 // rdm.cu
 int one_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw, double *rdm);
 int two_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw, double *rdm2);
+int transition_one_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_pairs, const double *bra, const double *ket,
+                       int64_t ldw, double *tdm);
+int transition_two_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_pairs, const double *bra, const double *ket,
+                       int64_t ldw, double *tdm2);
 int orbital_derivatives(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw,
                         const double *state_weights, double *fock, double *hessian, double *energy);
 int sigma(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *x, int64_t ldx,

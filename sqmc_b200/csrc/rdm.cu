@@ -19,6 +19,12 @@
 //
 // Time-reversal symmetrised lists are first expanded to plain determinants on the device: a representative (u,d), u != d,
 // becomes c/sqrt2 on (u,d) and z c/sqrt2 on (d,u); (u,u) keeps c (the norm factors of chem_hamiltonian_time_sym).
+//
+// Transition mode (sqmc_b200_transition_one_rdm, TR = true): every row holds 2S coefficients, bra a_k at k and ket b_k at
+// S + k, and gamma^{ab}_pq = <a| a+_p a_q |b> is accumulated as the full norb x norb matrix.  The pair D_j = sg a+_p a_q D_i
+// (p > q) adds (sg a_i) b_j to (q,p) and (sg a_j) b_i to (p,q), the diagonal a_i b_i.  Both slots of a pair belong to one
+// lane, so the warp-private accumulation and the reduction tree are those of one_rdm; for a = b every product has the bits
+// of its one_rdm counterpart (IEEE products commute), so the result is one_rdm's bit for bit.
 #include <thrust/iterator/counting_iterator.h>
 
 #include <cub/cub.cuh>
@@ -102,7 +108,8 @@ struct RdmView {
 // slot of (p,q), p >= q, in a packed lower triangle
 __device__ __forceinline__ int tri_slot(int p, int q) { return p * (p + 1) / 2 + q; }
 
-template <int NW>
+// tri: accumulator slots per state, the packed triangle (TR = false) or norb^2 (TR = true, (p,q) at p + norb q)
+template <int NW, bool TR>
 __global__ void one_rdm_kernel(RdmView v0, RdmView v1, int64_t n, int norb, int S, int tri, int64_t chunk, int nwarps, int shared_acc) {
   extern __shared__ double sacc[];
   // field by field: selecting the whole struct by a run-time index would copy it to local memory
@@ -127,11 +134,16 @@ __global__ void one_rdm_kernel(RdmView v0, RdmView v1, int64_t n, int norb, int 
       g1 = run_end<NW>(major, i, n, ma);
     }
     const Bits<NW> mi = b_load<NW>(minor, i);
-    const double *ci = coef + i * S;
+    const int cs = TR ? 2 * S : S;
+    const double *ci = coef + i * cs;
     for (int p = lane; p < norb; p += 32) {
       if (b_test(mi, p)) {
-        const int t = tri_slot(p, p);
-        for (int s = 0; s < S; s++) acc[s * tri + t] += ci[s] * ci[s];
+        if constexpr (TR) {
+          for (int s = 0; s < S; s++) acc[s * tri + p + norb * p] += ci[s] * ci[S + s];
+        } else {
+          const int t = tri_slot(p, p);
+          for (int s = 0; s < S; s++) acc[s * tri + t] += ci[s] * ci[s];
+        }
       }
     }
     const Bits<NW> emp = b_andnot(all, mi);
@@ -151,9 +163,16 @@ __global__ void one_rdm_kernel(RdmView v0, RdmView v1, int64_t n, int norb, int 
       }
       if (lo >= g1 || !b_eq(b_load<NW>(minor, lo), mj)) continue;
       const double sg = (double)permutation_factor(mi, mj);
-      const double *cj = coef + lo * S;
-      const int t = tri_slot(p, q);
-      for (int s = 0; s < S; s++) acc[s * tri + t] += (sg * ci[s]) * cj[s];
+      const double *cj = coef + lo * cs;
+      if constexpr (TR) {
+        for (int s = 0; s < S; s++) {
+          acc[s * tri + q + norb * p] += (sg * ci[s]) * cj[S + s];
+          acc[s * tri + p + norb * q] += (sg * cj[s]) * ci[S + s];
+        }
+      } else {
+        const int t = tri_slot(p, q);
+        for (int s = 0; s < S; s++) acc[s * tri + t] += (sg * ci[s]) * cj[s];
+      }
     }
     __syncwarp();
   }
@@ -163,9 +182,10 @@ __global__ void one_rdm_kernel(RdmView v0, RdmView v1, int64_t n, int norb, int 
   }
 }
 
-// one block per (slot, view): thread k sums warps k, k + 256, ... in order, then a fixed tree; writes (p,q) and (q,p)
+// one block per (slot, view): thread k sums warps k, k + 256, ... in order, then a fixed tree; writes (p,q) and (q,p) of the
+// packed triangle, or (full: tri = norb^2 slots) the one element (p,q) the slot holds
 __global__ void __launch_bounds__(kRdmThreads) one_rdm_reduce_kernel(const double *part0, const double *part1, int nwarps, int S, int tri, int norb,
-                                                                       double *out) {
+                                                                       int full, double *out) {
   __shared__ double red[kRdmThreads];
   const int64_t slot = blockIdx.x, per = (int64_t)S * tri;
   const double *part = blockIdx.y ? part1 : part0;
@@ -179,11 +199,15 @@ __global__ void __launch_bounds__(kRdmThreads) one_rdm_reduce_kernel(const doubl
   }
   if (threadIdx.x != 0) return;
   const int s = (int)(slot / tri), t = (int)(slot % tri);
+  const int sigma = blockIdx.y ? 0 : 1;  // view 0 is (up, dn) order: its minor string is beta
+  double *m = out + ((int64_t)s * 2 + sigma) * norb * norb;
+  if (full) {
+    m[t] = red[0];
+    return;
+  }
   int p = 0;
   while ((p + 1) * (p + 2) / 2 <= t) p++;
   const int q = t - p * (p + 1) / 2;
-  const int sigma = blockIdx.y ? 0 : 1;  // view 0 is (up, dn) order: its minor string is beta
-  double *m = out + ((int64_t)s * 2 + sigma) * norb * norb;
   m[p + (int64_t)norb * q] = red[0];
   m[q + (int64_t)norb * p] = red[0];
 }
@@ -319,10 +343,13 @@ static int prepare_dets(sqmc_b200_handle *h, const char *who, int64_t n, const v
   return 0;
 }
 
-template <int NW>
-static int one_rdm_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int S, const double *wts, int64_t ldw, double *rdm) {
+// TR: wts holds 2S columns, the bras a_k = column k and the kets b_k = column S + k (one_rdm_kernel's transition mode)
+template <int NW, bool TR>
+static int one_rdm_impl(sqmc_b200_handle *h, const char *who, int64_t n, const void *dets_up, const void *dets_dn, int S, const double *wts,
+                        int64_t ldw, double *rdm) {
   cudaStream_t s = G.stream;
   const int norb = h->T.norb;
+  const int cs = TR ? 2 * S : S;
   // view 0: (up, dn) order, beta singles; view 1: (dn, up) order, alpha singles
   DevBuf<uint64_t> up, dn;
   DevBuf<double> w;
@@ -330,11 +357,11 @@ static int one_rdm_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, con
   DevBuf<int32_t> idx0, idx1;
   DevBuf<uint64_t> ma0, mi0, ma1, mi1;
   DevBuf<double> c0, c1;
-  SQ_CHECK(prepare_dets<NW>(h, "one_rdm", n, dets_up, dets_dn, S, wts, ldw, up, dn, w, n2, idx0, ma0, mi0, c0));
-  SQ_CHECK(make_view<NW>(norb, dn.p, up.p, w.p, n2, S, idx1, ma1, mi1, c1, s));
+  SQ_CHECK(prepare_dets<NW>(h, who, n, dets_up, dets_dn, cs, wts, ldw, up, dn, w, n2, idx0, ma0, mi0, c0));
+  SQ_CHECK(make_view<NW>(norb, dn.p, up.p, w.p, n2, cs, idx1, ma1, mi1, c1, s));
   up.release(); dn.release(); w.release(); idx0.release(); idx1.release();
 
-  const int tri = norb * (norb + 1) / 2;
+  const int tri = TR ? norb * norb : norb * (norb + 1) / 2;
   const int64_t per = (int64_t)S * tri;
   const int nwarps = (int)std::min<int64_t>(kRdmMaxWarps, div_up(n2, 32));
   const int64_t chunk = div_up(n2, nwarps);
@@ -345,26 +372,50 @@ static int one_rdm_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, con
   SQ_CHECK(part0.alloc(nwarps * per));
   SQ_CHECK(part1.alloc(nwarps * per));
   SQ_CHECK(out.alloc((int64_t)S * 2 * norb * norb));
-  auto kern = one_rdm_kernel<NW>;
+  auto kern = one_rdm_kernel<NW, TR>;
   const size_t dyn = shared_acc ? shmem : 0;
   SQ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
   RdmView v0{ma0.p, mi0.p, c0.p, part0.p}, v1{ma1.p, mi1.p, c1.p, part1.p};
   kern<<<dim3((unsigned)div_up(nwarps, wpb), 2), kRdmThreads, dyn, s>>>(v0, v1, n2, norb, S, tri, chunk, nwarps, shared_acc);
   SQ_LAUNCH_CHECK();
-  one_rdm_reduce_kernel<<<dim3((unsigned)per, 2), kRdmThreads, 0, s>>>(part0.p, part1.p, nwarps, S, tri, norb, out.p);
+  one_rdm_reduce_kernel<<<dim3((unsigned)per, 2), kRdmThreads, 0, s>>>(part0.p, part1.p, nwarps, S, tri, norb, TR ? 1 : 0, out.p);
   SQ_LAUNCH_CHECK();
   SQ_CUDA(cudaMemcpyAsync(rdm, out.p, (size_t)S * 2 * norb * norb * sizeof(double), cudaMemcpyDeviceToHost, s));
   SQ_CUDA(cudaStreamSynchronize(s));
   return 0;
 }
 
+// argument checks both one-particle entry points share; count: "n_states" or "n_pairs"
+static int rdm1_check_args(const char *who, const char *count, int64_t n, int S, int64_t ldw) {
+  if (n <= 0) { set_error("%s: n must be positive", who); return 2; }
+  if (S < 1) { set_error("%s: %s must be >= 1", who, count); return 2; }
+  if (ldw < n) { set_error("%s: ldw (%lld) must be >= n (%lld)", who, (long long)ldw, (long long)n); return 2; }
+  if (n > INT32_MAX) { set_error("%s: n exceeds the 32-bit row index", who); return 2; }
+  return 0;
+}
+
 int one_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw, double *rdm) {
-  if (n <= 0) { set_error("one_rdm: n must be positive"); return 2; }
-  if (n_states < 1) { set_error("one_rdm: n_states must be >= 1"); return 2; }
-  if (ldw < n) { set_error("one_rdm: ldw (%lld) must be >= n (%lld)", (long long)ldw, (long long)n); return 2; }
-  if (n > INT32_MAX) { set_error("one_rdm: n exceeds the 32-bit row index"); return 2; }
-  return h->NW == 1 ? one_rdm_impl<1>(h, n, dets_up, dets_dn, n_states, wts, ldw, rdm)
-                    : one_rdm_impl<2>(h, n, dets_up, dets_dn, n_states, wts, ldw, rdm);
+  SQ_CHECK(rdm1_check_args("one_rdm", "n_states", n, n_states, ldw));
+  return h->NW == 1 ? one_rdm_impl<1, false>(h, "one_rdm", n, dets_up, dets_dn, n_states, wts, ldw, rdm)
+                    : one_rdm_impl<2, false>(h, "one_rdm", n, dets_up, dets_dn, n_states, wts, ldw, rdm);
+}
+
+// [a_1 .. a_S | b_1 .. b_S], leading dimension n: the 2S-column layout of the transition modes
+static std::vector<double> stack_columns(int64_t n, int S, const double *a, const double *b, int64_t ldw) {
+  std::vector<double> ab((size_t)2 * S * n);
+  for (int k = 0; k < S; k++) {
+    memcpy(ab.data() + (size_t)k * n, a + k * ldw, n * sizeof(double));
+    memcpy(ab.data() + (size_t)(S + k) * n, b + k * ldw, n * sizeof(double));
+  }
+  return ab;
+}
+
+int transition_one_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_pairs, const double *bra, const double *ket,
+                       int64_t ldw, double *tdm) {
+  SQ_CHECK(rdm1_check_args("transition_one_rdm", "n_pairs", n, n_pairs, ldw));
+  const std::vector<double> ab = stack_columns(n, n_pairs, bra, ket, ldw);
+  return h->NW == 1 ? one_rdm_impl<1, true>(h, "transition_one_rdm", n, dets_up, dets_dn, n_pairs, ab.data(), n, tdm)
+                    : one_rdm_impl<2, true>(h, "transition_one_rdm", n, dets_up, dets_dn, n_pairs, ab.data(), n, tdm);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -392,6 +443,14 @@ int one_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *det
 // with 2^e_k >= sum_i c_ik^2 (by Cauchy-Schwarz no element exceeds that).  A term sign * c_i * c_j is rounded once to that grid
 // and added with a 64-bit atomic on the low word plus the carry and sign extension on the high word.  Integer addition does not
 // depend on order, so repeated calls and permuted rows give the same bits.
+//
+// Transition mode (sqmc_b200_transition_two_rdm): Gamma^{ab} = <a| ... |b> is not Hermitian, so Gamma_{pq,rs} = Gamma_{qp,sr}
+// no longer holds and the two orientations of a representative are kept apart.  Each slot has two accumulators: F =
+// <a| E_c |b> and B = <a| E_c^+ |b>, E_c the canonical orientation ss_slot / ab_slot pick (flip: they took the Hermitian image
+// of the element asked for).  A pair (i, j) with f = <i| E |j> adds f a_i b_j to the orientation of E and f a_j b_i to the
+// other one.  Diagonal terms a_i b_i fall only on self-adjoint slots (A = B, or p = q and r = s), where F = B; they go to F
+// once and the fill reads F there.  The grid is set from ||a|| ||b||.  For a = b every term has the bits of its two_rdm
+// counterpart, sqrt(fl(na na)) = na, and F = B = two_rdm's representative; T(b, a) holds in F what T(a, b) holds in B.
 static const int kFixBits = 120;
 
 __device__ __forceinline__ int par_between(uint64_t x, int a, int b) {  // parity of the electrons of x strictly between a and b
@@ -422,28 +481,43 @@ __device__ __forceinline__ void i128_add(unsigned long long *slot, uint64_t lo, 
 }
 
 __device__ __forceinline__ int pair_index(int p, int r) { return r * (r - 1) / 2 + p; }  // p < r
-// representative of the same-spin element (p,q,r,s), p != r, q != s, inside an M x M block; sg: element = sg * representative
-__device__ __forceinline__ int64_t ss_slot(int p, int q, int r, int s, int M, int &sg) {
+// representative of the same-spin element (p,q,r,s), p != r, q != s, inside an M x M block; sg: element = sg * representative;
+// flip: the representative is the Hermitian image of the element (creator pair A > annihilator pair B)
+__device__ __forceinline__ int64_t ss_slot(int p, int q, int r, int s, int M, int &sg, bool &flip) {
   sg = 1;
   if (p > r) { const int t = p; p = r; r = t; sg = -sg; }
   if (q > s) { const int t = q; q = s; s = t; sg = -sg; }
   const int64_t A = pair_index(p, r), B = pair_index(q, s);
-  return A <= B ? A + M * B : B + M * A;
+  flip = A > B;
+  return flip ? B + M * A : A + M * B;
 }
-__device__ __forceinline__ int64_t ab_slot(int p, int q, int r, int s, int norb) {
+__device__ __forceinline__ int64_t ss_slot(int p, int q, int r, int s, int M, int &sg) {
+  bool flip;
+  return ss_slot(p, q, r, s, M, sg, flip);
+}
+__device__ __forceinline__ int64_t ab_slot(int p, int q, int r, int s, int norb, bool &flip) {
   int64_t X = p + (int64_t)norb * q, Y = r + (int64_t)norb * s;
   const int64_t X2 = q + (int64_t)norb * p, Y2 = s + (int64_t)norb * r;
-  if (X2 < X || (X2 == X && Y2 < Y)) { X = X2; Y = Y2; }
+  flip = X2 < X || (X2 == X && Y2 < Y);
+  if (flip) { X = X2; Y = Y2; }
   return X + (int64_t)norb * norb * Y;
+}
+__device__ __forceinline__ int64_t ab_slot(int p, int q, int r, int s, int norb) {
+  bool flip;
+  return ab_slot(p, q, r, s, norb, flip);
 }
 
 struct Rdm2Acc {
   unsigned long long *a;  // [S][per] slots of two words
+  unsigned long long *b;  // transition mode: [S][per] accumulators of the Hermitian-image orientation B (a holds F); else null
   const double *scale;    // [S] 2^(120 - e_k)
   int64_t per, off_bb, off_ab;
   int M, norb, S;
-  int cs;                 // coefficients per row: S, or 2S in the two-vector mode (a_k at k, b_k at S + k)
+  int cs;                 // coefficients per row: S, or 2S in the two-vector modes (a_k at k, b_k at S + k)
 };
+
+// rdm2_accumulate modes: one state, the symmetrised two-vector density (orbital-gradient response), the transition density
+enum Rdm2Mode { RDM2_ONE = 0, RDM2_SYM = 1, RDM2_TRANS = 2 };
 
 __global__ void electron_count_kernel(const uint64_t *u, const uint64_t *d, int64_t n, int nup, int ndn, int *bad) {
   const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
@@ -486,9 +560,10 @@ __global__ void rdm2_keys_ab_kernel(const uint64_t *u, const uint64_t *d, int64_
 }
 
 // The representative slot of the pair (i, j) of one bucket (entries ki / kdi / ai / bi of i and aj / bj of j) and the sign f
-// of <i| operator |j> on it; boff: block offset of a same-spin class, -1: alpha beta
+// of <i| operator |j> on it; boff: block offset of a same-spin class, -1: alpha beta; flip: the slot's canonical orientation
+// is the Hermitian image of the <i| . |j> one, f = <j| E_c |i>
 __device__ __forceinline__ int64_t rdm2_pair_slot(uint64_t ki, uint64_t kdi, int ai, int bi, int aj, int bj, int64_t boff, int M, int norb,
-                                                  int64_t off_ab, double &f) {
+                                                  int64_t off_ab, double &f, bool &flip) {
   int neg, sg = 1;
   int64_t slot;
   if (boff >= 0) {
@@ -503,24 +578,25 @@ __device__ __forceinline__ int64_t rdm2_pair_slot(uint64_t ki, uint64_t kdi, int
       neg = par_between(ki | 1ull << r0, xi, xj);
       p = xi; q = xj; r = r0; s = r0;
     }
-    slot = boff + ss_slot(p, q, r, s, M, sg);
+    slot = boff + ss_slot(p, q, r, s, M, sg, flip);
   } else if (ai != aj && bi != bj) {
     neg = par_between(ki, ai, aj) ^ par_between(kdi, bi, bj);
-    slot = off_ab + ab_slot(ai, aj, bi, bj, norb);
+    slot = off_ab + ab_slot(ai, aj, bi, bj, norb, flip);
   } else if (ai != aj) {
     neg = par_between(ki, ai, aj);
-    slot = off_ab + ab_slot(ai, aj, bi, bi, norb);
+    slot = off_ab + ab_slot(ai, aj, bi, bi, norb, flip);
   } else {
     neg = par_between(kdi, bi, bj);
-    slot = off_ab + ab_slot(ai, ai, bi, bj, norb);
+    slot = off_ab + ab_slot(ai, ai, bi, bj, norb, flip);
   }
   f = (neg ? -1.0 : 1.0) * sg;
   return slot;
 }
 
 // one thread per sorted entry i: every later entry j of the same bucket; boff: block offset of a same-spin class, -1: alpha beta.
-// TWO = false: the term f c_i c_j of each state; TWO = true: the symmetrised transition term f (a_i b_j + b_i a_j) / 2.
-template <bool TWO>
+// RDM2_ONE: the term f c_i c_j of each state; RDM2_SYM: the symmetrised transition term f (a_i b_j + b_i a_j) / 2; RDM2_TRANS:
+// f a_i b_j to the orientation of <i| . |j> and f a_j b_i to the other one (F in R.a, B in R.b).
+template <int MODE>
 __global__ void __launch_bounds__(256) rdm2_pair_kernel(const uint64_t *ku, const uint64_t *kd, const uint64_t *pay, int64_t m, int64_t boff,
                                                         const double *coef, Rdm2Acc R) {
   const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
@@ -531,13 +607,22 @@ __global__ void __launch_bounds__(256) rdm2_pair_kernel(const uint64_t *ku, cons
   for (int64_t j = i + 1; j < m && ku[j] == ki && kd[j] == kdi; j++) {
     const uint64_t pj = pay[j];
     double f;
-    const int64_t slot = rdm2_pair_slot(ki, kdi, ai, bi, (int)(pj & 0xff), (int)((pj >> 8) & 0xff), boff, R.M, R.norb, R.off_ab, f);
+    bool flip;
+    const int64_t slot = rdm2_pair_slot(ki, kdi, ai, bi, (int)(pj & 0xff), (int)((pj >> 8) & 0xff), boff, R.M, R.norb, R.off_ab, f, flip);
     const double *cj = coef + (int64_t)(pj >> 16) * R.cs;
     for (int k = 0; k < R.S; k++) {
       uint64_t lo, hi;
-      if constexpr (TWO) fix_to_i128(f * (0.5 * (ci[k] * cj[R.S + k] + ci[R.S + k] * cj[k])) * R.scale[k], lo, hi);
-      else fix_to_i128(f * (ci[k] * cj[k]) * R.scale[k], lo, hi);
-      i128_add(R.a + 2 * (k * R.per + slot), lo, hi);
+      if constexpr (MODE == RDM2_TRANS) {
+        const double fw = f * (ci[k] * cj[R.S + k]), bw = f * (cj[k] * ci[R.S + k]);
+        fix_to_i128((flip ? bw : fw) * R.scale[k], lo, hi);
+        i128_add(R.a + 2 * (k * R.per + slot), lo, hi);
+        fix_to_i128((flip ? fw : bw) * R.scale[k], lo, hi);
+        i128_add(R.b + 2 * (k * R.per + slot), lo, hi);
+      } else {
+        if constexpr (MODE == RDM2_SYM) fix_to_i128(f * (0.5 * (ci[k] * cj[R.S + k] + ci[R.S + k] * cj[k])) * R.scale[k], lo, hi);
+        else fix_to_i128(f * (ci[k] * cj[k]) * R.scale[k], lo, hi);
+        i128_add(R.a + 2 * (k * R.per + slot), lo, hi);
+      }
     }
   }
 }
@@ -585,7 +670,8 @@ __global__ void __launch_bounds__(256) rdm2_diag_kernel(const uint64_t *u, const
   }
 }
 
-// every element of the output (column-major p, q, r, s, block, state) from its representative
+// every element of the output (column-major p, q, r, s, block, state) from its representative; transition mode (R.b set):
+// from F or B by the element's orientation (self-adjoint slots never flip and read F)
 __global__ void rdm2_fill_kernel(Rdm2Acc R, const double *unscale, double *out) {
   const int norb = R.norb;
   const int64_t n4 = (int64_t)norb * norb * norb * norb, total = n4 * 3 * R.S;
@@ -598,16 +684,17 @@ __global__ void rdm2_fill_kernel(Rdm2Acc R, const double *unscale, double *out) 
     const int b = (int)(x % 3);
     const int k = (int)(x / 3);
     int sg = 1;
+    bool flip;
     int64_t slot;
     if (b == 1) {
-      slot = R.off_ab + ab_slot(p, q, r, s, norb);
+      slot = R.off_ab + ab_slot(p, q, r, s, norb, flip);
     } else if (p == r || q == s) {
       out[t] = 0.0;
       continue;
     } else {
-      slot = (b ? R.off_bb : 0) + ss_slot(p, q, r, s, R.M, sg);
+      slot = (b ? R.off_bb : 0) + ss_slot(p, q, r, s, R.M, sg, flip);
     }
-    const unsigned long long *v = R.a + 2 * (k * R.per + slot);
+    const unsigned long long *v = (flip && R.b ? R.b : R.a) + 2 * (k * R.per + slot);
     const double a = (ldexp((double)(long long)v[1], 64) + (double)v[0]) * unscale[k];
     out[t] = sg < 0 ? -a : a;
   }
@@ -724,6 +811,7 @@ static int rdm2_for_each_class(const ModelTables &T, const char *who, const uint
 static void rdm2_layout(Rdm2Acc &R, int norb, int S) {
   const int M = norb * (norb - 1) / 2;
   R.M = M; R.norb = norb; R.S = S; R.cs = S;
+  R.b = nullptr;
   R.off_bb = (int64_t)M * M;
   R.off_ab = 2 * R.off_bb;
   R.per = R.off_ab + (int64_t)norb * norb * norb * norb;
@@ -732,12 +820,15 @@ static void rdm2_layout(Rdm2Acc &R, int norb, int S) {
 // The accumulation both two-particle entry points share: upload, time_sym expansion, checks, the diagonal and the three key
 // classes with their pairs.  On return acc / scale hold the representatives of R (scale[S + k]: the factor back to doubles);
 // norm2 (device, S doubles, may be null) receives ||Psi_k||^2 summed in a fixed order.
-// two = true: wts holds 2S columns, a_k = column k and b_k = column S + k; b_k is first made orthogonal to a_k on the device, and
-// the representatives are those of the symmetrised transition density (<a_k| E |b_k> + <b_k| E |a_k>) / 2, on a grid from
+// mode RDM2_SYM: wts holds 2S columns, a_k = column k and b_k = column S + k; b_k is first made orthogonal to a_k on the device,
+// and the representatives are those of the symmetrised transition density (<a_k| E |b_k> + <b_k| E |a_k>) / 2, on a grid from
 // ||a_k|| ||b_k|| (Cauchy-Schwarz again); norm2 receives ||a_k||^2.
+// mode RDM2_TRANS: the same 2S columns, no projection; R.a / R.b hold F = <a_k| E_c |b_k> and B = <a_k| E_c^+ |b_k> on the grid
+// from ||a_k|| ||b_k||; norm2 must be null.
 static int rdm2_accumulate(sqmc_b200_handle *h, const char *who, int64_t n, const void *dets_up, const void *dets_dn, int S, const double *wts,
                            int64_t ldw, HostMarks &marks, DevBuf<unsigned long long> &acc, DevBuf<double> &scale, Rdm2Acc &R, double *norm2,
-                           bool two = false) {
+                           int mode = RDM2_ONE) {
+  const bool two = mode != RDM2_ONE;
   cudaStream_t s = G.stream;
   const ModelTables &T = h->T;
   const int norb = T.norb;
@@ -749,7 +840,7 @@ static int rdm2_accumulate(sqmc_b200_handle *h, const char *who, int64_t n, cons
   up.release(); dn.release(); w.release(); idx0.release();
   marks.mark("upload, expansion, checks");
   SQ_CHECK(rdm2_electron_check(T, who, U.p, D.p, n2, s));
-  if (two) {
+  if (mode == RDM2_SYM) {
     DevBuf<double> dots;
     SQ_CHECK(dots.alloc(2 * S));
     dots_kernel<<<S, 256, 0, s>>>(c.p, n2, S, dots.p);
@@ -781,11 +872,13 @@ static int rdm2_accumulate(sqmc_b200_handle *h, const char *who, int64_t n, cons
   }
   rdm2_layout(R, norb, S);
   if (two) R.cs = 2 * S;
-  SQ_CHECK(acc.alloc(2 * S * R.per));
+  const int nacc = mode == RDM2_TRANS ? 2 : 1;  // F, and B in the transition mode
+  SQ_CHECK(acc.alloc(2 * nacc * S * R.per));
   SQ_CHECK(scale.alloc(2 * S));
   SQ_CUDA(cudaMemsetAsync(acc.p, 0, (size_t)acc.n * sizeof(unsigned long long), s));
   SQ_CUDA(cudaMemcpyAsync(scale.p, hs.data(), 2 * S * sizeof(double), cudaMemcpyHostToDevice, s));
   R.a = acc.p;
+  R.b = mode == RDM2_TRANS ? acc.p + 2 * S * R.per : nullptr;
   R.scale = scale.p;
 
   const size_t dsh = (size_t)6 * norb * norb * sizeof(unsigned long long);
@@ -798,21 +891,24 @@ static int rdm2_accumulate(sqmc_b200_handle *h, const char *who, int64_t n, cons
   const Rdm2Acc Rc = R;
   const double *cp = c.p;
   return rdm2_for_each_class(T, who, U.p, D.p, n2, R, marks, [&](const uint64_t *sku, const uint64_t *skd, const uint64_t *spay, int64_t m, int64_t boff) {
-    if (two) rdm2_pair_kernel<true><<<(unsigned)div_up(m, 256), 256, 0, s>>>(sku, skd, spay, m, boff, cp, Rc);
-    else rdm2_pair_kernel<false><<<(unsigned)div_up(m, 256), 256, 0, s>>>(sku, skd, spay, m, boff, cp, Rc);
+    if (mode == RDM2_TRANS) rdm2_pair_kernel<RDM2_TRANS><<<(unsigned)div_up(m, 256), 256, 0, s>>>(sku, skd, spay, m, boff, cp, Rc);
+    else if (two) rdm2_pair_kernel<RDM2_SYM><<<(unsigned)div_up(m, 256), 256, 0, s>>>(sku, skd, spay, m, boff, cp, Rc);
+    else rdm2_pair_kernel<RDM2_ONE><<<(unsigned)div_up(m, 256), 256, 0, s>>>(sku, skd, spay, m, boff, cp, Rc);
     SQ_LAUNCH_CHECK();
     return 0;
   });
 }
 
-static int two_rdm_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int S, const double *wts, int64_t ldw, double *rdm) {
+// mode RDM2_ONE (two_rdm) or RDM2_TRANS (transition_two_rdm: wts holds the 2S columns [bras | kets])
+static int two_rdm_impl(sqmc_b200_handle *h, const char *who, int64_t n, const void *dets_up, const void *dets_dn, int S, const double *wts,
+                        int64_t ldw, double *rdm, int mode) {
   cudaStream_t s = G.stream;
   const int norb = h->T.norb;
-  HostMarks marks("SQMC_RDM2_PROFILE", "two_rdm");  // =1: phase split (synchronising) on stderr
+  HostMarks marks("SQMC_RDM2_PROFILE", who);  // =1: phase split (synchronising) on stderr
   DevBuf<unsigned long long> acc;
   DevBuf<double> scale;
   Rdm2Acc R;
-  SQ_CHECK(rdm2_accumulate(h, "two_rdm", n, dets_up, dets_dn, S, wts, ldw, marks, acc, scale, R, nullptr));
+  SQ_CHECK(rdm2_accumulate(h, who, n, dets_up, dets_dn, S, wts, ldw, marks, acc, scale, R, nullptr, mode));
   const int64_t n4 = (int64_t)norb * norb * norb * norb;
   DevBuf<double> out;
   SQ_CHECK(out.alloc(3 * S * n4));
@@ -824,10 +920,10 @@ static int two_rdm_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, con
   return 0;
 }
 
-// argument checks both two-particle entry points share
-static int rdm2_check_args(sqmc_b200_handle *h, const char *who, int64_t n, int n_states, int64_t ldw) {
+// argument checks the two-particle entry points share; count: the name of n_states in the caller's interface
+static int rdm2_check_args(sqmc_b200_handle *h, const char *who, int64_t n, int n_states, int64_t ldw, const char *count = "n_states") {
   if (n <= 0) { set_error("%s: n must be positive", who); return 2; }
-  if (n_states < 1) { set_error("%s: n_states must be >= 1", who); return 2; }
+  if (n_states < 1) { set_error("%s: %s must be >= 1", who, count); return 2; }
   if (ldw < n) { set_error("%s: ldw (%lld) must be >= n (%lld)", who, (long long)ldw, (long long)n); return 2; }
   if (n > INT32_MAX) { set_error("%s: n exceeds the 32-bit row index", who); return 2; }
   if (h->T.norb > 64) {
@@ -840,7 +936,14 @@ static int rdm2_check_args(sqmc_b200_handle *h, const char *who, int64_t n, int 
 
 int two_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_states, const double *wts, int64_t ldw, double *rdm) {
   SQ_CHECK(rdm2_check_args(h, "two_rdm", n, n_states, ldw));
-  return two_rdm_impl(h, n, dets_up, dets_dn, n_states, wts, ldw, rdm);
+  return two_rdm_impl(h, "two_rdm", n, dets_up, dets_dn, n_states, wts, ldw, rdm, RDM2_ONE);
+}
+
+int transition_two_rdm(sqmc_b200_handle *h, int64_t n, const void *dets_up, const void *dets_dn, int n_pairs, const double *bra, const double *ket,
+                       int64_t ldw, double *tdm2) {
+  SQ_CHECK(rdm2_check_args(h, "transition_two_rdm", n, n_pairs, ldw, "n_pairs"));
+  const std::vector<double> ab = stack_columns(n, n_pairs, bra, ket, ldw);
+  return two_rdm_impl(h, "transition_two_rdm", n, dets_up, dets_dn, n_pairs, ab.data(), n, tdm2, RDM2_TRANS);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -1262,7 +1365,8 @@ __global__ void __launch_bounds__(256) sigma_pair_kernel(const uint64_t *ku, con
   for (int64_t j = i + 1; j < m && ku[j] == ki && kd[j] == kdi; j++) {
     const uint64_t pj = pay[j];
     double f;
-    const int64_t slot = rdm2_pair_slot(ki, kdi, ai, bi, (int)(pj & 0xff), (int)((pj >> 8) & 0xff), boff, R.M, R.norb, R.off_ab, f);
+    bool flip;
+    const int64_t slot = rdm2_pair_slot(ki, kdi, ai, bi, (int)(pj & 0xff), (int)((pj >> 8) & 0xff), boff, R.M, R.norb, R.off_ab, f, flip);
     const double gs = 0.5 * f * G[slot];
     if (gs == 0.0) continue;
     const int64_t rj = (int64_t)(pj >> 16);
@@ -1450,11 +1554,7 @@ static int orbital_gradient_response_impl(sqmc_b200_handle *h, int64_t n, const 
   const int norb = T.norb;
   const int64_t nn = (int64_t)norb * norb, n4 = nn * nn;
   HostMarks marks("SQMC_ORBD_PROFILE", "orbital_gradient_response");  // =1: phase split (synchronising) on stderr
-  std::vector<double> ab((size_t)2 * S * n);  // [c_1 .. c_S | dc_1 .. dc_S], leading dimension n
-  for (int k = 0; k < S; k++) {
-    memcpy(ab.data() + (size_t)k * n, wts + k * ldw, n * sizeof(double));
-    memcpy(ab.data() + (size_t)(S + k) * n, dwts + k * ldw, n * sizeof(double));
-  }
+  const std::vector<double> ab = stack_columns(n, S, wts, dwts, ldw);  // [c_1 .. c_S | dc_1 .. dc_S]
   std::vector<double> w2(S);
   for (int k = 0; k < S; k++) w2[k] = 2.0 * state_weights[k];
   DevBuf<double> norm2, sw, d, D;
@@ -1465,7 +1565,7 @@ static int orbital_gradient_response_impl(sqmc_b200_handle *h, int64_t n, const 
     DevBuf<unsigned long long> acc;
     DevBuf<double> scale;
     Rdm2Acc R;
-    SQ_CHECK(rdm2_accumulate(h, "orbital_gradient_response", n, dets_up, dets_dn, S, ab.data(), n, marks, acc, scale, R, norm2.p, true));
+    SQ_CHECK(rdm2_accumulate(h, "orbital_gradient_response", n, dets_up, dets_dn, S, ab.data(), n, marks, acc, scale, R, norm2.p, RDM2_SYM));
     SQ_CHECK(d.alloc(n4));
     orbd_fill_kernel<<<(unsigned)std::min<int64_t>(div_up(n4, 256), 64 * G.sm_count), 256, 0, s>>>(R, scale.p + S, sw.p, norm2.p, d.p);
     SQ_LAUNCH_CHECK();

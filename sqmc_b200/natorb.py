@@ -49,6 +49,41 @@ def natural_orbitals(system, rdm, state_weights=None):
     return dict(occupations=np.array(occ)[order], coeffs=np.array(cols).T[:, order].copy(), irreps=np.array(irr, dtype=np.int32)[order])
 
 
+def natural_transition_orbitals(system, tdm1, spin_sign=+1):
+    """Natural transition orbitals of one pair <bra| . |ket> from transition_one_rdm's output (2, norb, norb).
+
+    The SVD gamma = sum_k sigma_k |particle_k><hole_k| of gamma = gamma^alpha + spin_sign gamma^beta: spin_sign = +1 for a
+    singlet-coupled transition, -1 for a triplet-coupled one within M_s = 0.  gamma_pq = <bra| a+_p a_q |ket>, so the holes
+    (right vectors) are the ket-side orbitals that are emptied and the particles (left vectors) the bra-side orbitals that are
+    filled.  chem: gamma is mapped to FCIDUMP numbering through system.orb_order first (as natural_orbitals does); heg /
+    hubbardk: the library's orbitals.  Each hole's largest component is made positive and its particle flipped with it, so
+    gamma = particles @ diag(singular_values) @ holes.T still holds.
+    -> dict(singular_values (descending), weights sigma^2 / sum sigma^2, participation_ratio (sum sigma^2)^2 / sum sigma^4,
+    holes, particles (norb, norb): column k = orbital k)."""
+    if spin_sign not in (1, -1):
+        raise ValueError("natural_transition_orbitals: spin_sign must be +1 or -1")
+    g = np.asarray(tdm1, dtype=np.float64)
+    if g.ndim != 3 or g.shape[0] != 2 or g.shape[1] != g.shape[2]:
+        raise ValueError("natural_transition_orbitals: tdm1 must be one pair's (2, norb, norb), not %s" % (g.shape,))
+    gamma = g[0] + spin_sign * g[1]
+    if isinstance(system, systems.ChemSystem):
+        o = np.asarray(system.orb_order[:gamma.shape[0]]) - 1     # library orbital p is FCIDUMP orbital o[p]
+        gf = np.zeros_like(gamma)
+        gf[np.ix_(o, o)] = gamma
+        gamma = gf
+    u, sv, vt = np.linalg.svd(gamma)
+    holes, particles = vt.T.copy(), u.copy()
+    for k in range(len(sv)):
+        if holes[np.argmax(np.abs(holes[:, k])), k] < 0:
+            holes[:, k] = -holes[:, k]
+            particles[:, k] = -particles[:, k]
+    s2 = sv * sv
+    tot = float(np.sum(s2))
+    weights = s2 / tot if tot > 0 else np.zeros_like(s2)
+    pr = tot * tot / float(np.sum(s2 * s2)) if tot > 0 else 0.0
+    return dict(singular_values=sv, weights=weights, participation_ratio=pr, holes=holes, particles=particles)
+
+
 def dense_integrals(path):
     """FCIDUMP -> (header, h (norb, norb), eri (norb,)*4 with the 8-fold symmetry filled in, core energy)."""
     header, body = systems._read_fcidump(path)

@@ -1,7 +1,9 @@
 """Host quantities from the density matrices of SparseHamiltonian.one_rdm / two_rdm: <S^2> and the energy identity.
 
 Both read the matrices in the library's numbering (the bits of the determinant words) and apply no normalisation: a
-wavefunction of norm ||Psi||^2 gives ||Psi||^2 times the expectation value.
+wavefunction of norm ||Psi||^2 gives ||Psi||^2 times the expectation value.  Both are linear in the matrices, so fed the
+transition density matrices of SparseHamiltonian.transition_one_rdm / transition_two_rdm of a pair (a, b), with norm2 read as
+the overlap <a|b>, they give the transition elements <a|S^2|b> and <a|H|b>.
 """
 import numpy as np
 
@@ -9,7 +11,8 @@ import numpy as np
 def spin_squared(rdm2, nup, ndn, norm2=1.0):
     """<Psi|S^2|Psi> = [S_z(S_z+1) + N_beta] ||Psi||^2 - sum_pq Gamma^{ab}_{pq,qp}, S_z = (N_alpha - N_beta)/2.
 
-    rdm2: [b, p, q, r, s] of one state, or [k, b, p, q, r, s] (then norm2 may be one value per state)."""
+    rdm2: [b, p, q, r, s] of one state, or [k, b, p, q, r, s] (then norm2 may be one value per state).
+    With a transition two_rdm of (a, b) and norm2 = <a|b> (the trace of its gamma over N) this is <a|S^2|b>."""
     g = np.asarray(rdm2)
     sz = 0.5 * (nup - ndn)
     return (sz * (sz + 1.0) + ndn) * np.asarray(norm2, dtype=np.float64) - np.einsum("...pqqp->...", g[..., 1, :, :, :, :])
@@ -37,7 +40,8 @@ def integrals_library_order(chem_system):
 def rdm_energy(chem_system, rdm1, rdm2):
     """enuc ||Psi||^2 + sum_pq h_pq gamma_pq + 1/2 sum (pq|rs) Gamma_pq,rs of one state, spins summed (the alpha-beta block
     counts twice: beta-alpha is the same block).  rdm1: [sigma, p, q] from one_rdm; rdm2: [b, p, q, r, s] from two_rdm.
-    ||Psi||^2 is the trace of gamma over the electron count."""
+    ||Psi||^2 is the trace of gamma over the electron count.  Fed transition_one_rdm / transition_two_rdm of one pair (a, b),
+    the same formula gives <a|H|b> (the trace then gives <a|b>), since H is Hermitian and the sums are linear."""
     h, eri, enuc = integrals_library_order(chem_system)
     g1 = np.asarray(rdm1)
     g2 = np.asarray(rdm2)
