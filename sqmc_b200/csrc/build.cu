@@ -1683,6 +1683,7 @@ static int build_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, const
     cudaEventRecord(e1, s);
     SQ_CUDA(cudaMemsetAsync(row_nnz.p, 0, (nr + 1) * sizeof(int32_t), s));
     int c2bytes = (T.model == MODEL_CHEM) ? (T.norb + 1) * (T.norb + 1) * 4 : 0;
+    SQ_MODEL_DISPATCH(T, SQ_CUDA((allow_dynamic_smem(eval_kernel<NW, kModel, kTS>, c2bytes))));
     SQ_MODEL_DISPATCH(T, (eval_kernel<NW, kModel, kTS><<<nblocks(nr * 32), 256, c2bytes, s>>>(T, h->d_up, h->d_dn, h->d_perm, h->d_diag, h->row0, r, r_end, cptr.p,
                                                                                               cand_count.p + r, cand_tmp.p, vals_tmp.p, row_nnz.p, ts ? nullptr : alen.p, d_olen)));
     SQ_LAUNCH_CHECK();

@@ -450,6 +450,17 @@ __device__ __forceinline__ double model_hamiltonian(const ModelTables &T, const 
   }
 }
 
+// host: a kernel may take 48 KiB of static plus dynamic shared memory unless it opts into more, so its default dynamic
+// budget is 48 KiB minus its own static shared memory.  Chem kernels stage combine_2, (norb + 1)^2 * 4 bytes: 64 KiB at
+// 127 orbitals, and already above the default budget of eval_kernel / select_kernel (3 KiB static) from 107 orbitals on.
+template <typename Kernel>
+inline cudaError_t allow_dynamic_smem(Kernel kernel, int bytes) {
+  cudaFuncAttributes a;
+  cudaError_t e = cudaFuncGetAttributes(&a, kernel);
+  if (e != cudaSuccess || bytes <= a.maxDynamicSharedSizeBytes) return e;
+  return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+}
+
 // host: run `call` with the compile-time constants kModel / kTS of the system described by T
 #define SQ_MODEL_DISPATCH(T, call)                                                          \
   do {                                                                                      \

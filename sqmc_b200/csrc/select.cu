@@ -534,6 +534,7 @@ static int select_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, cons
   SQ_CHECK(counts.alloc(nd + 1));
   SQ_CUDA(cudaMemsetAsync(counts.p, 0, (nd + 1) * sizeof(int32_t), s));
   if (nd > 0) {
+    SQ_MODEL_DISPATCH(T, SQ_CUDA((allow_dynamic_smem(select_kernel<NW, false, 0, kModel, kTS>, c2bytes))));
     SQ_MODEL_DISPATCH(T, (select_kernel<NW, false, 0, kModel, kTS><<<(unsigned)div_up(nd * 32, 128), 128, c2bytes, s>>>(S, 0, nd, counts.p, nullptr, nullptr, nullptr, nullptr)));
     SQ_LAUNCH_CHECK();
   }
@@ -562,6 +563,7 @@ static int select_impl(sqmc_b200_handle *h, int64_t n, const void *dets_up, cons
     std::vector<int64_t> hp(prefix.begin() + i0, prefix.begin() + i1 + 1);
     for (auto &v : hp) v -= prefix[i0];
     SQ_CUDA(cudaMemcpyAsync(optr.p, hp.data(), hp.size() * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+    SQ_MODEL_DISPATCH(T, SQ_CUDA((allow_dynamic_smem(select_kernel<NW, true, 0, kModel, kTS>, c2bytes))));
     SQ_MODEL_DISPATCH(T, (select_kernel<NW, true, 0, kModel, kTS><<<(unsigned)div_up((i1 - i0) * 32, 128), 128, c2bytes, s>>>(S, i0, i1, nullptr, optr.p, ca.p, cb.p, nullptr)));
     SQ_LAUNCH_CHECK();
     SQ_CUDA(cudaStreamSynchronize(s));
@@ -748,6 +750,7 @@ static int pt2_core(sqmc_b200_handle *h, int64_t n_var, const uint64_t *sup, con
   SQ_CHECK(counts.alloc(n + 1));
   SQ_CUDA(cudaMemsetAsync(counts.p, 0, (n + 1) * sizeof(int32_t), s));
   if (n > 0) {
+    SQ_MODEL_DISPATCH(T, SQ_CUDA((allow_dynamic_smem(select_kernel<NW, false, 0, kModel, kTS>, c2bytes))));
     SQ_MODEL_DISPATCH(T, (select_kernel<NW, false, 0, kModel, kTS><<<(unsigned)div_up(n * 32, 128), 128, c2bytes, s>>>(S, 0, n, counts.p, nullptr, nullptr, nullptr, nullptr)));
     SQ_LAUNCH_CHECK();
   }
@@ -781,8 +784,10 @@ static int pt2_core(sqmc_b200_handle *h, int64_t n_var, const uint64_t *sup, con
     SQ_CUDA(cudaMemcpyAsync(optr.p, hp.data(), hp.size() * sizeof(int64_t), cudaMemcpyHostToDevice, s));
     const unsigned g = (unsigned)div_up((i1 - i0) * 32, 128);
     if (nch == 1) {
+      SQ_MODEL_DISPATCH(T, SQ_CUDA((allow_dynamic_smem(select_kernel<NW, true, 1, kModel, kTS>, c2bytes))));
       SQ_MODEL_DISPATCH(T, (select_kernel<NW, true, 1, kModel, kTS><<<g, 128, c2bytes, s>>>(S, i0, i1, nullptr, optr.p, ca.p, cb.p, cv.p)));
     } else {
+      SQ_MODEL_DISPATCH(T, SQ_CUDA((allow_dynamic_smem(select_kernel<NW, true, 4, kModel, kTS>, c2bytes))));
       SQ_MODEL_DISPATCH(T, (select_kernel<NW, true, 4, kModel, kTS><<<g, 128, c2bytes, s>>>(S, i0, i1, nullptr, optr.p, ca.p, cb.p, cv.p)));
     }
     SQ_LAUNCH_CHECK();

@@ -133,15 +133,16 @@ def hci_space(H, system, n_dets, eps_schedule=(1e-3, 3e-4, 1e-4, 3e-5, 1e-5, 5e-
 def hubbard_momentum_sector(hub, n_dets=None, ktot=(0, 0)):
     """Determinants of one total-momentum sector of the k-space Hubbard model, ranked by
     ascending diagonal energy then label, truncated to n_dets, stored sorted by label
-    (the order generate_sparse_ham_hubbardk_upper_triangular's binary search needs, hubbard.f90:9646)."""
+    (the order generate_sparse_ham_hubbardk_upper_triangular's binary search needs, hubbard.f90:9646).
+    Strings are (n, 2) uint64 words, so lattices of more than 64 sites (up to 127) are enumerated too."""
     ns = hub.norb
-    su = np.array(_strings(ns, hub.nup), dtype=np.uint64)
-    sd = np.array(_strings(ns, hub.ndn), dtype=np.uint64)
+    su = _words(_strings(ns, hub.nup))
+    sd = _words(_strings(ns, hub.ndn))
     kx = hub.k_vectors[:, 0].astype(np.int64)
     ky = hub.k_vectors[:, 1].astype(np.int64)
 
     def props(strs):
-        occ = ((strs[:, None] >> np.arange(ns, dtype=np.uint64)[None, :]) & np.uint64(1)).astype(np.int64)
+        occ = np.stack([(strs[:, o >> 6] >> np.uint64(o & 63)) & np.uint64(1) for o in range(ns)], axis=1).astype(np.int64)
         return (occ @ kx) % (2 * hub.l_x), (occ @ ky) % (2 * hub.l_y), occ.astype(np.float64) @ hub.k_energies
 
     ux, uy, ue = props(su)
@@ -154,18 +155,21 @@ def hubbard_momentum_sector(hub, n_dets=None, ktot=(0, 0)):
             if len(iu) == 0 or len(id_) == 0:
                 continue
             E = ue[iu][:, None] + de[id_][None, :]
-            ups.append(np.broadcast_to(su[iu][:, None], E.shape).ravel())
-            dns.append(np.broadcast_to(sd[id_][None, :], E.shape).ravel())
+            ups.append(np.broadcast_to(iu[:, None], E.shape).ravel())
+            dns.append(np.broadcast_to(id_[None, :], E.shape).ravel())
             ens.append(E.ravel())
-    up = np.concatenate(ups); dn = np.concatenate(dns); en = np.concatenate(ens)
+    up = su[np.concatenate(ups)]; dn = sd[np.concatenate(dns)]; en = np.concatenate(ens)
     total = len(en)
     if n_dets is not None and n_dets < total:
-        order = np.lexsort((dn, up, np.round(en, 12)))[:n_dets]
+        order = np.lexsort((dn[:, 0], dn[:, 1], up[:, 0], up[:, 1], np.round(en, 12)))[:n_dets]
         up, dn = up[order], dn[order]
-    order = np.lexsort((dn, up))
-    up, dn = up[order], dn[order]
-    z = np.zeros(len(up), dtype=np.uint64)
-    return np.ascontiguousarray(np.stack([up, z], axis=1)), np.ascontiguousarray(np.stack([dn, z], axis=1)), total
+    order = np.lexsort((dn[:, 0], dn[:, 1], up[:, 0], up[:, 1]))   # 128-bit label: high word first
+    return np.ascontiguousarray(up[order]), np.ascontiguousarray(dn[order]), total
+
+
+def _words(strs):
+    """python ints below 2^128 -> (n, 2) uint64, low word first"""
+    return np.array([(s & 0xFFFFFFFFFFFFFFFF, s >> 64) for s in strs], dtype=np.uint64).reshape(-1, 2)
 
 
 def splitmix_vector(n, seed=12345):

@@ -25,7 +25,7 @@ class ChemSystem:
 
     def __init__(self, fcidump, nelec=None, nup=None, orbital_symmetries=None, time_sym=False, z=1, hf_up=None, hf_dn=None):
         header, body = _read_fcidump(fcidump)
-        self.norb = norb = int(header["NORB"])
+        self.norb = norb = _check_norb(int(header["NORB"]))
         self.nelec = int(header["NELEC"]) if nelec is None else nelec
         ms2 = int(header.get("MS2", 0))
         self.nup = (self.nelec + ms2) // 2 if nup is None else nup
@@ -139,6 +139,13 @@ class ChemSystem:
         return h, J, K
 
 
+def _check_norb(norb):
+    """a determinant string is two 64-bit words holding a value below 2^127 (types.f90:44): 1..127 orbitals"""
+    if not 1 <= norb <= 127:
+        raise ValueError("norb=%d outside 1..127: determinant strings hold at most 127 orbitals" % norb)
+    return norb
+
+
 def _read_fcidump(path):
     with open(path) as f:
         lines = f.read().splitlines()
@@ -215,7 +222,7 @@ class HegSystem:
             if math.sqrt(s2(v)) > 2 * math.pi / self.length_cell * cutoff_radius + EPS:
                 break
             norb += 1
-        self.norb = norb
+        self.norb = _check_norb(norb)
         self.k_vectors = np.array(kv[:norb], dtype=np.float64)  # (norb, n_dim) C-order == (n_dim, norb) column-major
         self.hf_up = (1 << nup) - 1
         self.hf_dn = (1 << self.ndn) - 1
@@ -227,7 +234,7 @@ class HubbardKSystem:
     def __init__(self, l_x, l_y, t, U, nup, ndn):
         self.l_x, self.l_y, self.t, self.U, self.nup, self.ndn = l_x, l_y, t, U, nup, ndn
         ns = l_x * l_y
-        self.norb = ns
+        self.norb = _check_norb(ns)
         kv = np.zeros((ns, 2), dtype=np.int64)
         for i in range(1, l_x + 1):
             for j in range(1, l_y + 1):

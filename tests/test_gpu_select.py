@@ -45,8 +45,9 @@ def test_select_step_heg(oracle, heg_space):
     assert np.array_equal(got_up, ref_up) and np.array_equal(got_dn, ref_dn) and np.array_equal(got_mh, ref_mh)
 
 
-def _hci_on_gpu(H, hf_up, hf_dn, sched, n_states=1, max_iters=50):
-    """perform_hci (hci.f90:359-517) with selection, build and Davidson all on the GPU."""
+def _hci_on_gpu(H, hf_up, hf_dn, sched, n_states=1, max_iters=50, trace=None):
+    """perform_hci (hci.f90:359-517) with selection, build and Davidson all on the GPU; trace, a list, receives the
+    (new up, new dn, updated min_H) of every selection step."""
     import sqmc_b200 as sq
     up = sq.dets_to_u64([hf_up])
     dn = sq.dets_to_u64([hf_dn])
@@ -60,6 +61,8 @@ def _hci_on_gpu(H, hf_up, hf_dn, sched, n_states=1, max_iters=50):
         n_old = len(up)
         coeffs = np.abs(wts).max(axis=1) if it > 1 else wts[:, 0].copy()
         nu, nd, min_h = H.get_next_det_list(up, dn, coeffs, min_h, eps)
+        if trace is not None:
+            trace.append((nu, nd, min_h.copy()))
         n_new = n_old + len(nu)
         min_h = np.concatenate([min_h, np.full(len(nu), 9e99)])
         if n_new == n_old:
